@@ -2,7 +2,7 @@
 """bench.py -- GAE + PPO-loss transitions/s on the B200 hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2_atari_large] [--scaling weak|strong]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one synthetic batch (SURVEY.md §8d): GAE once, then
 (epochs x minibatches) fused loss forward+backward covering every transition once per epoch.
@@ -23,6 +23,8 @@ compressed frame leaf into pinned memory (`wire_decode_native`, host GB/s).
 `--impl reference` times the reference's OWN functions (`MultiAgentPPO._compute_adv_and_value_target`, `_compute_loss` +
 backward, loaded unmodified through oracle/ref_loader.py from oracle/_ref) on the host cores, same config / metric / unit,
 per stage; where a GPU is visible it adds the same functions on cuda (the ATen-eager path SRL users have today).
+`--dump-outputs DIR` writes what the timed step computed in its last timed step as DIR/<name>.npy (see dump_step_outputs);
+the inputs depend only on the arguments, so two builds of the library can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,6 +41,8 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# bench.py writes nothing into the tree it runs from: no __pycache__/*.pyc next to the modules it imports either
+sys.dont_write_bytecode = True
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -49,6 +53,7 @@ METRIC = "gae_ppo_loss_transitions_per_sec"
 UNIT = "transitions/s"
 GAE_BYTES = 19  # SURVEY.md §8(d): 11 B read + 8 B written per scanned row-lane
 LOSS_BYTES = {True: 41, False: 37}  # per transition per pass, with / without value clipping
+DUMP_BYTES = 64_000_000 - 4096  # --dump-outputs: array data of all files together (the .npy headers fit in the rest)
 
 
 def peaks():
@@ -526,6 +531,36 @@ def parity_check(hp, cfg, pol_np, sample_np, rank, world, dist, dev):
     return out
 
 
+def dump_step_outputs(out_dir, hp, shard):
+    """--dump-outputs: what one step hands its caller -- adv and ret [L, N] float32, the loss / statistics rows
+    [E*M, 16] float64 and the gradients w.r.t. new_logp, v_pred and entropy [E, M, T, n] float32 -- as
+    out_dir/<name>.npy.  Where they hold more than DUMP_BYTES, the loss table stays whole and every other array keeps the
+    same fraction k / n of its n elements, flattened: the array is cut into k stretches of n // k or n // k + 1 elements
+    that cover all of it, and one element of each is kept, at an offset drawn from a fixed seed, so the same arguments give
+    the same sample.  `shard` says whose step it is (with several GPUs: rank 0's slice of the workload)."""
+    arrays = dict(adv=hp.adv, ret=hp.ret, loss_out=hp.out, g_logp=hp.grads_all[:, :, 0], g_value=hp.grads_all[:, :, 1],
+                  g_entropy=hp.grads_all[:, :, 2])
+    nbytes = lambda t: t.numel() * t.element_size()
+    frac = min(1.0, (DUMP_BYTES - nbytes(hp.out)) / sum(nbytes(t) for k, t in arrays.items() if k != "loss_out"))
+    os.makedirs(out_dir, exist_ok=True)
+    info = {}
+    for seed, (name, t) in enumerate(arrays.items()):
+        x = t.contiguous().view(-1)
+        n = x.numel()
+        k = n if frac == 1.0 or name == "loss_out" else max(1, int(n * frac))
+        if k < n:  # k strata [lo, hi) that tile the whole array; one element of each
+            lo = np.arange(k, dtype=np.int64) * n // k
+            hi = np.arange(1, k + 1, dtype=np.int64) * n // k
+            idx = lo + np.random.default_rng(seed).integers(0, hi - lo)
+            x = x.index_select(0, torch.from_numpy(idx).to(x.device))
+        else:
+            x = x.view(t.shape)
+        np.save(os.path.join(out_dir, f"{name}.npy"), x.cpu().numpy())
+        info[name] = dict(shape=list(t.shape), dtype=str(t.dtype).replace("torch.", ""),
+                          stored="all" if k == n else f"{k} of {n} elements")
+    return dict(dir=os.path.abspath(out_dir), shard=shard, arrays=info)
+
+
 def run_ours(args, cfg_full, rank, world, local_rank):
     import torch.distributed as dist
     from srl_b200 import ops
@@ -638,6 +673,11 @@ def run_ours(args, cfg_full, rank, world, local_rank):
     ms = timed_steps(args.steps, step)
     barrier()
     windows.append((w0, time.perf_counter()))
+    # before anything else runs on the step's buffers
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = dump_step_outputs(args.dump_outputs, hp, "the whole workload on one GPU" if world == 1 else
+                                   f"rank 0 of {world}: {workload_name(cfg)} ({args.scaling} scaling), inputs seeded for rank 0")
     ms_per_step = max_over_ranks(sum(ms)) / args.steps
     total_transitions = cfg.transitions * world
     value = total_transitions / (ms_per_step * 1e-3)
@@ -838,6 +878,8 @@ def run_ours(args, cfg_full, rank, world, local_rank):
                       value_l2_warm=total_transitions / (statistics.mean(ms_warm) * 1e-3)),
             step_trainer_order=trainer_order, trainer_step=trainer_line, extra=extra,
             cpu_baseline=cpu)
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         print(json.dumps(line), flush=True)
     align = None
     del hp, g_loss, g_gae  # CUDA graphs and peer mailboxes go before the process group does
@@ -941,7 +983,8 @@ def extras_run(cfg, dev, peak, timed_steps):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 2000; 50 with --impl reference, whose CPU step of cfg2 takes ~0.1 s)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="cfg2_atari_large", choices=sorted(synth.CONFIGS))
@@ -966,14 +1009,21 @@ def main():
                     help="A/B: minibatch statistics from the srl_group_stats table instead of inside the loss kernel")
     ap.add_argument("--no-pack", action="store_true", help="A/B: gather the five sample leaves instead of K2's pack")
     ap.add_argument("--no-batch", action="store_true", help="A/B: one loss launch per minibatch (parallel graph branches)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed step's outputs of its last step to DIR/<name>.npy (at most 64 MB in all); "
+                         "with several GPUs, rank 0's step on its slice of the workload")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 50 if args.impl == "reference" else 2000
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     cfg = synth.CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
-        if args.steps > 50:
-            args.steps = 50  # a CPU step of cfg2 is ~0.1 s; keep the whole arm within minutes
         run_reference_arm(args, cfg, rank, world)
         return
     if world != args.gpus and world == 1 and args.gpus > 1:

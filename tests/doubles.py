@@ -1,7 +1,8 @@
 """Test doubles for the trainer boundary, in the spirit of SRL's api/testing (NullTrainer, RandomPolicy):
 a tiny actor-critic policy with the surface `MultiAgentPPO` calls on a policy (SURVEY.md §8b), and mirrors of
 RunningMeanStd / PopArtValueHead (legacy/algorithm/modules/utils.py:70-151, popart.py:8-59) with the same
-attribute names, so the trainer's PopArt bridge is exercised without an SRL checkout."""
+attribute names, so the trainer's PopArt bridge is exercised without an SRL checkout; and a record family of its own
+(NamedArray, SampleBatch, recursive_apply) standing in for SRL's."""
 from __future__ import annotations
 
 import dataclasses
@@ -11,6 +12,49 @@ from typing import Optional
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
+
+
+class NamedArray:
+    """A record family of its own, standing in for SRL's base.namedarray.NamedArray where no SRL checkout is staged: keyword
+    construction, keys(), item access by name or by index / slice over every leaf, attribute access and assignment -- what
+    the trainer and an SRL policy use of it -- and
+    nothing shared with srl_b200.namedarray (duck-typed like SRL's class, not a subclass of the mirror)."""
+
+    def __init__(self, **fields):
+        object.__setattr__(self, "_fields", dict(fields))
+
+    def keys(self):
+        return self._fields.keys()
+
+    def __getitem__(self, key):
+        """A field by name; any other key (an index, a slice) indexes every leaf and gives a record of the same type."""
+        if isinstance(key, str):
+            return self._fields[key]
+        new = object.__new__(type(self))
+        object.__setattr__(new, "_fields", {k: None if v is None else v[key] for k, v in self._fields.items()})
+        return new
+
+    def __getattr__(self, name):
+        fields = object.__getattribute__(self, "_fields")
+        if name in fields:
+            return fields[name]
+        raise AttributeError(name)
+
+    def __setattr__(self, name, value):
+        self._fields[name] = value
+
+
+class SampleBatch(NamedArray):
+    """api/trainer.py's SampleBatch in the stand-in family."""
+
+
+def recursive_apply(x, fn):
+    """base/namedarray.py's recursive_apply in the stand-in family: subclasses come back as plain NamedArray records."""
+    if x is None:
+        return None
+    if isinstance(x, NamedArray):
+        return NamedArray(**{k: recursive_apply(x[k], fn) for k in x.keys()})
+    return fn(x)
 
 
 @dataclasses.dataclass

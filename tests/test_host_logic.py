@@ -100,18 +100,35 @@ def test_popart_mirror_matches_oracle():
     assert torch.equal(head.normalize(y), ref.normalize(y)) and torch.equal(head.denormalize(y), ref.denormalize(y))
 
 
-def test_plugin_registers_into_srl_registry_when_srl_is_importable():
-    """INTEGRATION.md: `import srl_b200.srl_plugin` inside an SRL checkout adds 'mappo_b200' next to 'mappo'."""
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("/root/reference not present on this box")
-    R = ref_loader.load()
+def test_plugin_registers_into_srl_registry_when_srl_is_importable(monkeypatch):
+    """INTEGRATION.md: `import srl_b200.srl_plugin` inside an SRL checkout adds 'mappo_b200' next to 'mappo'.  Where the
+    reference files are not staged, SRL's `api.trainer` is a stand-in: its two registries and their register functions
+    (api/trainer.py:84-99,231-235, mirrored by srl_b200/api.py), with 'mappo' in it as SRL's own import leaves it."""
     import importlib
+    import sys
+    import types
+
+    from oracle import ref_loader
+    if ref_loader.available():
+        srl_trainer = ref_loader.load().trainer
+    else:
+        srl_trainer = types.ModuleType("api.trainer")
+        srl_trainer.ALL_TRAINER_CLASSES = {"mappo": object}
+        srl_trainer.ALL_TRAJ_POSTPROCESSOR_CLASSES = {}
+        srl_trainer.register = srl_trainer.ALL_TRAINER_CLASSES.__setitem__
+        srl_trainer.register_traj_postprocessor = srl_trainer.ALL_TRAJ_POSTPROCESSOR_CLASSES.__setitem__
+        srl_api = types.ModuleType("api")
+        srl_api.trainer = srl_trainer
+        monkeypatch.setitem(sys.modules, "api", srl_api)
+        monkeypatch.setitem(sys.modules, "api.trainer", srl_trainer)
 
     import srl_b200.srl_plugin as plugin
     importlib.reload(plugin)
     assert plugin.REGISTERED_IN_SRL
-    assert {"mappo", "mappo_b200"} <= set(R.trainer.ALL_TRAINER_CLASSES)
+    assert {"mappo", "mappo_b200"} <= set(srl_trainer.ALL_TRAINER_CLASSES)
+    assert srl_trainer.ALL_TRAINER_CLASSES["mappo_b200"] is plugin.MultiAgentPPOB200
+    if not ref_loader.available():
+        assert srl_trainer.ALL_TRAJ_POSTPROCESSOR_CLASSES == {"gae_b200": plugin.TrajGAEB200}
 
 
 # ---- chunk reshape descriptors (ops.to_chunk / back_to_trajectory build these for srl_batch_gather) ----------------
