@@ -106,6 +106,20 @@ inline cudaError_t launch_pdl_scan(void (*kern)(KArgs...), dim3 grid, dim3 block
   return e;
 }
 
+// Lets kernel KERN use up to `bytes` of dynamic shared memory on the current device.  The driver is asked once per device
+// (one flag table per kernel, not per signature), so later launches -- stream capture included -- cost nothing.
+template <auto KERN>
+inline int opt_in_smem(size_t bytes) {
+  static bool opted_in[64] = {};
+  int dev = 0;
+  SRL_CUDA(cudaGetDevice(&dev));
+  if (dev < 64 && !opted_in[dev]) {
+    SRL_CUDA(cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(bytes)));
+    opted_in[dev] = true;
+  }
+  return SRL_OK;
+}
+
 // ---- debug timeline (profiles/microbench/timeline.py; library built with -DSRL_TIMELINE, never the product build) ------
 // One record per (kernel, CTA, slot): %globaltimer (ns, common to all SMs) and the SM's clock64.  The buffer pointer is a
 // per-translation-unit device symbol set through the TU's own exported setter; a null pointer switches the stamps off.

@@ -6,13 +6,13 @@
 //    (gae.py:36,64-65,88-89).  One thread owns one (lane, critic) column for the whole trajectory; adjacent threads own
 //    adjacent columns, so every row access of a warp is one coalesced segment.  Rows are taken newest first in chunks of
 //    CH: all loads of a chunk are issued before the first dependent float64 operation, so a thread exposes one DRAM
-//    round trip per CH rows.  Same float64 rounding sequence as K2 (explicit __dmul_rn / __dadd_rn, compiled with
-//    -fmad=false) -> bit-identical to the reference.
+//    round trip per CH rows.  The per-cell arithmetic is K2's (gae_common.cuh) -> bit-identical to the reference.
 //
 // 2. srl_traj_gae -- TrajGAE.process (gae.py:100-139): GAE along whole episodes, one after another in memory
 //    ([total_steps, W] with an offset table), in the arrays' own dtype (numpy semantics: float32 arrays stay float32,
 //    the python scalars gamma and gamma * lmbda are rounded to that dtype first).  One thread per (trajectory, element).
 #include "common.cuh"
+#include "gae_common.cuh"
 
 namespace srl {
 namespace {
@@ -48,7 +48,7 @@ __global__ void __launch_bounds__(kTraceThreads) gae_trace_kernel(const TracePar
   // v'[L-1]: the bootstrap value of the newest row
   float vnext = __ldg(p.value + static_cast<long long>(L - 1) * NC + col);
   if (p.done != nullptr)
-    vnext = __fmul_rn(vnext, 1.f - static_cast<float>(__ldg(p.done + static_cast<long long>(L - 1) * N + lane) != 0));
+    vnext = gae_vprime(vnext, __ldg(p.done + static_cast<long long>(L - 1) * N + lane) != 0, false, 0.0, 1.0);
   if (p.pad_last_row) {  // mappo.py:254-256
     p.adv[static_cast<long long>(L - 1) * NC + col] = 0.f;
     if (p.ret != nullptr) p.ret[static_cast<long long>(L - 1) * NC + col] = 0.f;
@@ -80,27 +80,18 @@ __global__ void __launch_bounds__(kTraceThreads) gae_trace_kernel(const TracePar
     for (int u = 0; u < CH; ++u) {
       const int row = t - u;
       if (row >= 0) {
-        const float v0 = p.done != nullptr ? __fmul_rn(vv[u], 1.f - static_cast<float>(dn[u] != 0)) : vv[u];
-        const double alive = rs[u] ? 0.0 : 1.0;   // 1 - on_reset[t+1]
-        const double not_tr = tr[u] ? 0.0 : 1.0;  // 1 - truncated[t+1]
+        const float v0 = p.done != nullptr ? gae_vprime(vv[u], dn[u] != 0, false, 0.0, 1.0) : vv[u];
+        const bool reset1 = rs[u] != 0, trunc1 = tr[u] != 0;
         const double gam = HAS_G ? static_cast<double>(gm[u]) : p.gamma;
-        // gae.py:63  reward + gamma * value[1:] * (1 - on_reset[1:]) - value[:-1]
-        double d = __dmul_rn(__dmul_rn(gam, static_cast<double>(vnext)), alive);
-        d = __dadd_rn(static_cast<double>(rw[u]), d);
-        d = __dsub_rn(d, static_cast<double>(v0));
-        // gae.py:87  gamma * lmbda * (1 - on_reset[1:]) * (1 - truncated[1:])
+        double d = gae_delta(&rw[u], v0, vnext, reset1, gam);
         const double gl = (HAS_G || HAS_L) ? __dmul_rn(gam, HAS_L ? static_cast<double>(lm[u]) : p.lmbda) : gl_const;
-        double m = __dmul_rn(__dmul_rn(gl, alive), not_tr);
-        if (HAS_R) {
-          const double rd = static_cast<double>(ir[u]);
-          d = __dmul_rn(d, fmin(rd, p.rho));  // gae.py:64-65
-          m = __dmul_rn(m, fmin(rd, p.c));    // gae.py:88-89
-        }
-        g = __dadd_rn(d, __dmul_rn(m, g));  // gae.py:92
+        double m = gae_carry_product(gl, reset1, trunc1);  // any per-element gamma / lmbda: the product, not a select
+        if (HAS_R) gae_vtrace_scale(d, m, static_cast<double>(ir[u]), p.rho, p.c);
+        g = gae_step(d, m, g);
         const float a = static_cast<float>(g);  // gae.py:97
         const long long e = static_cast<long long>(row) * NC + col;
         stg_stream(p.adv + e, a);
-        if (p.ret != nullptr) stg_stream(p.ret + e, __fadd_rn(a, v0));  // mappo.py:143
+        if (p.ret != nullptr) stg_stream(p.ret + e, gae_value_target(a, v0));
         vnext = v0;
       }
     }

@@ -98,15 +98,12 @@ __global__ void __launch_bounds__(kThreads, 4) gae_scan_kernel(const GaeParams p
     for (int u = 0; u < kUnroll; ++u) {
       const int t = t0 + u * RPP;
       if (t < L) {
-        float vv = v[u];
+        const float vv = v[u];
         if (PACK) {
           svr[t * LW + lane] = vv;
           sol[t * LW + lane] = ol[u];
         }
-        if (popart)  // RunningMeanStd.denormalize: (x.double() * std + mean).float()   utils.py:146-151
-          vv = static_cast<float>(__dadd_rn(__dmul_rn(static_cast<double>(vv), pa_std), pa_mean));
-        vv = __fmul_rn(vv, 1.f - static_cast<float>(dn[u] != 0));  // value * (1 - done), fp32   mappo.py:120-124
-        sv[t * LW + lane] = vv;
+        sv[t * LW + lane] = gae_vprime(vv, dn[u] != 0, popart, pa_mean, pa_std);
         sf[t * LW + lane] = static_cast<uint8_t>((dn[u] != 0 ? 1u : 0u) | (tr[u] != 0 ? 2u : 0u) | (rs[u] != 0 ? 4u : 0u));
         sdm[t * LW + lane].x = static_cast<double>(rw[u]);
         if (VTRACE) sa[t * LW + lane] = expf(nl[u] - ol[u]);  // importance ratio, fp32   mappo.py:129-132
@@ -119,30 +116,20 @@ __global__ void __launch_bounds__(kThreads, 4) gae_scan_kernel(const GaeParams p
   // ---- A2: delta_t and m_t for t in [0, L-1), shared memory only -----------------------------------
   for (int t = trow; t < L - 1; t += RPP) {
     const uint32_t f1 = sf[(t + 1) * LW + lane];
-    const double alive = (f1 & 4u) ? 0.0 : 1.0;   // 1 - on_reset[t+1]
-    const double not_tr = (f1 & 2u) ? 0.0 : 1.0;  // 1 - truncated[t+1]
+    const bool reset1 = (f1 & 4u) != 0, trunc1 = (f1 & 2u) != 0;
     const double v1 = static_cast<double>(sv[(t + 1) * LW + lane]);
     const double v0 = static_cast<double>(sv[t * LW + lane]);
-    // gae.py:63  reward + gamma * value[1:] * (1 - on_reset[1:]) - value[:-1]
-    double d = __dmul_rn(__dmul_rn(p.gamma, v1), alive);
-    d = __dadd_rn(sdm[t * LW + lane].x, d);
-    d = __dsub_rn(d, v0);
-    // gae.py:87  gamma * lmbda * (1 - on_reset[1:]) * (1 - truncated[1:])
-    double m = __dmul_rn(__dmul_rn(p.gamma_lmbda, alive), not_tr);
-    if (VTRACE) {
-      const double rd = static_cast<double>(sa[t * LW + lane]);
-      d = __dmul_rn(d, fmin(rd, p.rho));  // gae.py:64-65
-      m = __dmul_rn(m, fmin(rd, p.c));    // gae.py:88-89
-    }
+    double d = gae_delta(&sdm[t * LW + lane].x, v0, v1, reset1, p.gamma);
+    double m = gae_carry_product(p.gamma_lmbda, reset1, trunc1);
+    if (VTRACE) gae_vtrace_scale(d, m, static_cast<double>(sa[t * LW + lane]), p.rho, p.c);
     sdm[t * LW + lane] = make_double2(d, m);
   }
   __syncthreads();
   SRL_STAMP(2);
 
   // ---- B: the sequential scan, one (partial) warp -----------------------------------------------------
-  // A_t = delta_t + m_t * A_{t+1}: separate fp64 multiply and add, as the reference's two torch ops
-  // (gae.py:92).  Software-pipelined: the (delta, m) pairs of the next 4 steps are already in registers
-  // while the dependent DMUL/DADD chain of the current 4 runs, so shared-memory latency is off the chain.
+  // A_t = delta_t + m_t * A_{t+1} (gae_step).  Software-pipelined: the (delta, m) pairs of the next 4 steps are already
+  // in registers while the dependent DMUL/DADD chain of the current 4 runs, so shared-memory latency is off the chain.
   if (tid < LW) {
     constexpr int CH = 4;
     double g = 0.0;
@@ -163,7 +150,7 @@ __global__ void __launch_bounds__(kThreads, 4) gae_scan_kernel(const GaeParams p
       // (profiles/microbench/f2f.cu) behind every 16-cycle DMUL+DADD link; phase C converts in parallel instead
 #pragma unroll
       for (int u = 0; u < CH; ++u) {
-        g = __dadd_rn(q[u].x, __dmul_rn(q[u].y, g));
+        g = gae_step(q[u].x, q[u].y, g);
         sdm[(t - u) * LW + lane].x = g;
       }
       if (more) {
@@ -173,7 +160,7 @@ __global__ void __launch_bounds__(kThreads, 4) gae_scan_kernel(const GaeParams p
     }
     for (; t >= 0; --t) {
       const double2 dm = sdm[t * LW + lane];
-      g = __dadd_rn(dm.x, __dmul_rn(dm.y, g));
+      g = gae_step(dm.x, dm.y, g);
       sdm[t * LW + lane].x = g;
     }
   }
@@ -186,7 +173,7 @@ __global__ void __launch_bounds__(kThreads, 4) gae_scan_kernel(const GaeParams p
     float a = 0.f, r = 0.f;
     if (t < L - 1) {
       a = static_cast<float>(sdm[t * LW + lane].x);  // adv.float(), gae.py:97
-      r = __fadd_rn(a, sv[t * LW + lane]);  // value_target = adv + v'[:-1], fp32   mappo.py:143
+      r = gae_value_target(a, sv[t * LW + lane]);
       if (t >= p.row_lo && t < p.row_hi) {
         const uint32_t f0 = sf[t * LW + lane], f1 = sf[(t + 1) * LW + lane];
         const double mk = (f1 & 4u) ? 0.0 : 1.0;  // loss mask = 1 - on_reset[t+1]   mappo.py:260-261
@@ -208,7 +195,7 @@ __global__ void __launch_bounds__(kThreads, 4) gae_scan_kernel(const GaeParams p
       if (PACK) {  // sample side of the loss as one 16-byte item (see include/srl_b200.h)
         const bool keep = t < L - 1 && (sf[(t + 1) * LW + lane] & 4u) == 0u;
         __stcg(reinterpret_cast<float4*>(p.pack) + pack_index(t, N, col),
-               make_float4(sol[t * LW + lane], svr[t * LW + lane], r, keep ? a : __int_as_float(0x7fc00000)));
+               pack_item(sol[t * LW + lane], svr[t * LW + lane], r, a, keep));
       }
     }
   }
@@ -224,18 +211,7 @@ __global__ void __launch_bounds__(kThreads, 4) gae_scan_kernel(const GaeParams p
     red[(trow * 7 + 5) * LW + lane] = s5;
     red[(trow * 7 + 6) * LW + lane] = s6;
     __syncthreads();
-    // 8 * LW outputs; fixed summation order over the RPP row groups
-    for (int o = tid; o < SRL_LANE_PART * LW; o += kThreads) {
-      const int k = o / LW, ln = o % LW;
-      const int c2 = blockIdx.x * LW + ln;
-      if (c2 < N) {
-        double s = 0.0;
-        if (k < 7)
-          for (int rr = 0; rr < RPP; ++rr) s += red[(rr * 7 + k) * LW + ln];
-        p.lane_part[static_cast<size_t>(k) * N + c2] = s;
-        if (p.lane_aos != nullptr && k < 4) p.lane_aos[static_cast<size_t>(c2) * 4 + k] = k < 3 ? s : 0.0;
-      }
-    }
+    fold_lane_sums<LW, RPP, kThreads>(p, red, [](int, int, double) {});
   }
   if (tid == 0) pdl_wait();  // scan complete => permutation kernel complete (see gae_scan_ws.cu)
 #ifdef SRL_DEBUG_PHASES
@@ -249,14 +225,9 @@ __global__ void __launch_bounds__(kThreads, 4) gae_scan_kernel(const GaeParams p
 template <int LW, bool VTRACE, bool PACK, int UN>
 int launch_un(const GaeParams& p, cudaStream_t st) {
   const size_t smem = gae_smem_bytes(p.L, LW, PACK);
-  auto kern = gae_scan_kernel<LW, VTRACE, PACK, UN>;
-  static bool opted_in[64] = {};  // once per device and instantiation (keeps launches capturable and cheap)
-  int dev = 0;
-  SRL_CUDA(cudaGetDevice(&dev));
-  if (dev < 64 && !opted_in[dev]) {
-    SRL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kSmemBudget)));
-    opted_in[dev] = true;
-  }
+  constexpr auto kern = gae_scan_kernel<LW, VTRACE, PACK, UN>;
+  const int rc = opt_in_smem<kern>(kSmemBudget);
+  if (rc != SRL_OK) return rc;
   const int grid = (p.N + LW - 1) / LW;
   SRL_CUDA(launch_pdl_scan(kern, dim3(grid), dim3(kThreads), smem, st, p));
   return SRL_OK;
@@ -396,31 +367,15 @@ int gae_scan_impl(const float* reward, const float* value, const uint8_t* done, 
   p.perm.part = nullptr;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
 
-  // Three kernels, picked by how many 32-lane groups the batch has (SRL_GAE_PATH=tile|tma|ws, read once, overrides:
-  // a tuning knob for profiles/, not an API):
+  // Three kernels, picked by how many 32-lane groups the batch has:
   //   >= 2 groups per SM : one warp per lane group, TMA ring (gae_scan_tma.cu): fewest instructions per row
   //   fewer              : warp-specialised CTA per lane group (gae_scan_ws.cu): the chain runs in its own warp and 16
   //                        worker warps keep a lone CTA's latency per chunk short (measured at mid sizes -- cfg3, cfg4 --
   //                        it only ties or loses: there the machine is issue-bound and it executes more instructions)
   //   ragged / unaligned / V-trace on few lanes: the shared-memory tile kernel below
-  static const int path_env = [] {
-    const char* e = getenv("SRL_GAE_PATH");
-    if (e == nullptr) return 0;
-    return e[0] == 't' && e[1] == 'i' ? 1 : (e[0] == 't' ? 2 : (e[0] == 'w' ? 3 : 0));
-  }();
-  static const int min_groups_env = [] {
-    const char* e = getenv("SRL_GAE_TMA_MIN_GROUPS");
-    return e ? atoi(e) : -1;
-  }();
   const int groups = (N + 31) / 32;
-  const int min_groups = min_groups_env >= 0 ? min_groups_env : 2 * sm_count();
-  bool use_tma = gae_tma_eligible(p) && groups >= min_groups;
-  bool use_ws = !use_tma && groups >= 8 && gae_ws_eligible(p);  // a handful of lanes: the tile kernel's many short CTAs win
-  if (path_env == 1) use_tma = use_ws = false;
-  if (path_env == 2) use_tma = gae_tma_eligible(p), use_ws = false;
-  if (path_env == 3) use_ws = gae_ws_eligible(p), use_tma = use_tma && !use_ws;
-  if (use_tma) return launch_gae_tma(p, st);
-  if (use_ws) {
+  if (groups >= 2 * sm_count() && gae_tma_eligible(p)) return launch_gae_tma(p, st);
+  if (groups >= 8 && gae_ws_eligible(p)) {  // a handful of lanes: the tile kernel's many short CTAs win
     if (job != nullptr) {  // the warp-specialised kernel's workers compute the permutation while they wait for data
       p.perm = *job;
       *fused = 1;

@@ -14,16 +14,14 @@
 // with no per-row range tests, masks are selects instead of fp64 multiplies, the mask / done / truncated counts
 // are integers, and squares accumulate with one DFMA.
 //
-// Arithmetic on adv / ret is identical, operation for operation, to the tile kernel (same explicit roundings),
-// so both paths are bit-identical to the reference's float64 scan.
-#include <cuda.h>
-#include <stdlib.h>
-
-#include "common.cuh"
+// The per-cell arithmetic is gae_common.cuh's, shared with the other scan kernels.
 #include "gae_common.cuh"
+#include "tma_util.cuh"
 
 namespace srl {
 namespace {
+
+using namespace srl::tma;
 
 #ifndef SRL_TMA_ROWS
 #define SRL_TMA_ROWS 8
@@ -59,35 +57,6 @@ struct StageLayout {
   static constexpr int stride = (bytes + 127) / 128 * 128;
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_LOOP:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra WAIT_DONE;\n"
-      "bra WAIT_LOOP;\n"
-      "WAIT_DONE:\n"
-      "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(
-          smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(smem_u32(bar))
-      : "memory");
-}
-
 template <bool VTRACE, bool OLDLP, int LPW>
 __device__ __forceinline__ void issue_stage(const GaeTmaParams& q, unsigned char* slot, uint64_t* bar, int col0, int row0) {
   using SL = StageLayout<VTRACE, OLDLP, LPW>;
@@ -106,10 +75,6 @@ struct Carry {
   double vd_next = 0.0;  // float64 image of v'[t+1]
   double g = 0.0;        // A[t+1]
   bool reset_next = false, trunc_next = false;
-};
-struct LaneStats {
-  double s1 = 0, s2 = 0, s3 = 0, s4 = 0;
-  int cnt = 0, dn = 0, tr = 0;
 };
 
 // One stage of kRows rows.  EDGE = false: every row t of the stage satisfies row_lo <= t < row_hi (<= L-1), so all
@@ -136,13 +101,11 @@ __device__ __forceinline__ void run_stage(const GaeParams& p, const unsigned cha
   bool dnf[kRows], trf[kRows], rsf[kRows];
 #pragma unroll
   for (int r = 0; r < kRows; ++r) {
-    float x = sv[r * LPW + lane];
+    const float x = sv[r * LPW + lane];
     dnf[r] = sdn[r * LPW + lane] != 0;
     trf[r] = str_[r * LPW + lane] != 0;
     rsf[r] = srs[r * LPW + lane] != 0;
-    if (popart)  // RunningMeanStd.denormalize: (x.double() * std + mean).float()   utils.py:146-151
-      x = static_cast<float>(__dadd_rn(__dmul_rn(static_cast<double>(x), pa_std), pa_mean));
-    v[r] = __fmul_rn(x, dnf[r] ? 0.f : 1.f);  // value * (1 - done), fp32   mappo.py:120-124
+    v[r] = gae_vprime(x, dnf[r], popart, pa_mean, pa_std);
     vd[r] = static_cast<double>(v[r]);
   }
 #pragma unroll
@@ -150,18 +113,13 @@ __device__ __forceinline__ void run_stage(const GaeParams& p, const unsigned cha
     const double vn = (r == kRows - 1) ? cy.vd_next : vd[r + 1];
     const bool rn = (r == kRows - 1) ? cy.reset_next : rsf[r + 1];
     const bool tn = (r == kRows - 1) ? cy.trunc_next : trf[r + 1];
-    // gae.py:63  reward + gamma * value[1:] * (1 - on_reset[1:]) - value[:-1]
-    double d = __dmul_rn(__dmul_rn(gamma, vn), rn ? 0.0 : 1.0);
-    d = __dadd_rn(static_cast<double>(sr[r * LPW + lane]), d);
-    d = __dsub_rn(d, vd[r]);
-    // gae.py:87  gamma * lmbda * (1 - on_reset[1:]) * (1 - truncated[1:]): exactly 0 or gamma*lmbda
-    double m = (rn || tn) ? 0.0 : gl;
+    double d = gae_delta(&sr[r * LPW + lane], vd[r], vn, rn, gamma);
+    double m = gae_carry(!rn && !tn, gl);
     if (VTRACE) {
       const float* snl = reinterpret_cast<const float*>(slot + SL::vt_new);
       const float* sol = reinterpret_cast<const float*>(slot + SL::old_logp);
       const double rd = static_cast<double>(expf(snl[r * LPW + lane] - sol[r * LPW + lane]));  // mappo.py:129-132
-      d = __dmul_rn(d, fmin(rd, p.rho));  // gae.py:64-65
-      m = __dmul_rn(m, fmin(rd, p.c));    // gae.py:88-89
+      gae_vtrace_scale(d, m, rd, p.rho, p.c);
     }
     if (EDGE) {
       const bool scanned = tbase + r < L - 1;  // rows L-1 (padding row) and beyond carry no advantage
@@ -171,12 +129,12 @@ __device__ __forceinline__ void run_stage(const GaeParams& p, const unsigned cha
     dl[r] = d;
     mm[r] = m;
   }
-  // ---- pass 2: the only sequential part, A_t = delta_t + m_t * A_{t+1} (two roundings, gae.py:92) -------------
+  // ---- pass 2: the only sequential part, A_t = delta_t + m_t * A_{t+1} ----------------------------------------------
   float a[kRows];
   double g = cy.g;
 #pragma unroll
   for (int r = kRows - 1; r >= 0; --r) {
-    g = __dadd_rn(dl[r], __dmul_rn(mm[r], g));
+    g = gae_step(dl[r], mm[r], g);
     a[r] = static_cast<float>(g);  // adv.float(), gae.py:97
   }
   cy.g = g;
@@ -186,7 +144,7 @@ __device__ __forceinline__ void run_stage(const GaeParams& p, const unsigned cha
   for (int r = kRows - 1; r >= 0; --r, gi -= N) {
     const int t = tbase + r;
     const bool rn = (r == kRows - 1) ? cy.reset_next : rsf[r + 1];
-    float rt = __fadd_rn(a[r], v[r]);  // value_target = adv + v'[:-1]   mappo.py:143
+    float rt = gae_value_target(a[r], v[r]);
     if (EDGE) rt = (t < L - 1) ? rt : 0.f;
     const bool store = EDGE ? (live && t < L) : live;  // row L-1 is the zero padding row of mappo.py:254-256
     // loss rows [row_lo, row_hi), mask = 1 - on_reset[t+1]   mappo.py:259-261
@@ -200,19 +158,11 @@ __device__ __forceinline__ void run_stage(const GaeParams& p, const unsigned cha
         const float* sol = reinterpret_cast<const float*>(slot + SL::old_logp);
         const bool keep = EDGE ? (!rn && t < L - 1) : !rn;
         __stcg(reinterpret_cast<float4*>(p.pack) + pack_index(t, N, col),
-               make_float4(sol[r * LPW + lane], sv[r * LPW + lane], rt, keep ? a[r] : __int_as_float(0x7fc00000)));
+               pack_item(sol[r * LPW + lane], sv[r * LPW + lane], rt, a[r], keep));
       }
     }
 #endif
-    const double x = static_cast<double>(mk ? a[r] : 0.f);
-    const double y = static_cast<double>(mk ? rt : 0.f);
-    st.cnt += mk ? 1 : 0;
-    st.s1 += x;
-    st.s2 = __fma_rn(x, x, st.s2);
-    st.s3 += y;
-    st.s4 = __fma_rn(y, y, st.s4);
-    st.dn += (in_rows && dnf[r]) ? 1 : 0;
-    st.tr += (in_rows && trf[r]) ? 1 : 0;
+    st.add(in_rows, mk, a[r], rt, dnf[r], trf[r]);
   }
   cy.vd_next = vd[0];
   cy.reset_next = rsf[0];
@@ -238,10 +188,9 @@ __global__ void __launch_bounds__(LPW) gae_scan_tma_kernel(const __grid_constant
 
   if (lane == 0) {
     const CUtensorMap* maps[] = {&q.maps.value, &q.maps.reward, &q.maps.done, &q.maps.truncated, &q.maps.on_reset};
-    for (const CUtensorMap* m : maps)
-      asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
+    for (const CUtensorMap* m : maps) prefetch_map(m);
     for (int s = 0; s < kStages; ++s) mbar_init(&bars[s], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
   __syncwarp();
   if (lane == 0) {  // prologue: fill the ring, newest rows first
@@ -309,52 +258,13 @@ __global__ void __launch_bounds__(LPW) gae_scan_tma_kernel(const __grid_constant
   if (lane == 0) pdl_wait();  // scan complete => permutation kernel complete (see gae_scan_ws.cu)
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(sym);
-  }
-  return fn;
-}
-
-// [rows, N] row-major tensor of `elem` bytes per element, box = [kRows, lpw lanes]
-int make_map(CUtensorMap* m, const void* base, int rows, int N, int elem, int lpw) {
-  EncodeTiledFn fn = encode_fn();
-  SRL_REQUIRE(fn != nullptr, SRL_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
-  const cuuint64_t dims[2] = {static_cast<cuuint64_t>(N), static_cast<cuuint64_t>(rows)};
-  const cuuint64_t strides[1] = {static_cast<cuuint64_t>(N) * elem};
-  const cuuint32_t box[2] = {static_cast<cuuint32_t>(lpw), kRows};
-  const cuuint32_t estr[2] = {1, 1};
-  const CUresult r = fn(m, elem == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 2,
-                        const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  SRL_REQUIRE(r == CUDA_SUCCESS, SRL_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d (rows=%d N=%d elem=%d)",
-              static_cast<int>(r), rows, N, elem);
-  return SRL_OK;
-}
-
 template <bool VTRACE, bool PACK, bool SPEC, bool POPART, int LPW>
 int launch(const GaeTmaParams& q, cudaStream_t st) {
   using SL = StageLayout<VTRACE, PACK || VTRACE, LPW>;
   const size_t smem = static_cast<size_t>(kStages) * SL::stride + kStages * sizeof(uint64_t);
-  auto kern = gae_scan_tma_kernel<VTRACE, PACK, SPEC, POPART, LPW>;
-  static bool opted_in[64] = {};
-  int dev = 0;
-  SRL_CUDA(cudaGetDevice(&dev));
-  if (dev < 64 && !opted_in[dev]) {
-    SRL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    opted_in[dev] = true;
-  }
+  constexpr auto kern = gae_scan_tma_kernel<VTRACE, PACK, SPEC, POPART, LPW>;
+  const int rc = opt_in_smem<kern>(smem);
+  if (rc != SRL_OK) return rc;
   const int grid = (q.p.N + LPW - 1) / LPW;
   SRL_CUDA(launch_pdl_scan(kern, dim3(grid), dim3(LPW), smem, st, q));
   return SRL_OK;
@@ -364,7 +274,7 @@ int launch(const GaeTmaParams& q, cudaStream_t st) {
 
 bool gae_tma_eligible(const GaeParams& p) {
   // TMA needs 16-byte aligned bases and row pitches: N % 16 == 0 covers the uint8 flag tensors (and N*4 for fp32)
-  if (p.N % 16 != 0 || encode_fn() == nullptr) return false;
+  if (p.N % 16 != 0 || tma::encode_fn() == nullptr) return false;
   const void* ptrs[] = {p.reward, p.value, p.done, p.truncated, p.on_reset};
   for (const void* q : ptrs)
     if (!aligned(q, 16)) return false;
@@ -381,22 +291,22 @@ int launch_gae_tma_lpw(const GaeParams& p, cudaStream_t st) {
   GaeTmaParams q;
   q.p = p;
   int rc;
-  if ((rc = make_map(&q.maps.value, p.value, p.L, p.N, 4, LPW)) != SRL_OK) return rc;
-  if ((rc = make_map(&q.maps.reward, p.reward, p.L, p.N, 4, LPW)) != SRL_OK) return rc;
-  if ((rc = make_map(&q.maps.done, p.done, p.L, p.N, 1, LPW)) != SRL_OK) return rc;
-  if ((rc = make_map(&q.maps.truncated, p.truncated, p.L, p.N, 1, LPW)) != SRL_OK) return rc;
-  if ((rc = make_map(&q.maps.on_reset, p.on_reset, p.L, p.N, 1, LPW)) != SRL_OK) return rc;
+  if ((rc = make_map(&q.maps.value, p.value, p.L, p.N, 4, LPW, kRows)) != SRL_OK) return rc;
+  if ((rc = make_map(&q.maps.reward, p.reward, p.L, p.N, 4, LPW, kRows)) != SRL_OK) return rc;
+  if ((rc = make_map(&q.maps.done, p.done, p.L, p.N, 1, LPW, kRows)) != SRL_OK) return rc;
+  if ((rc = make_map(&q.maps.truncated, p.truncated, p.L, p.N, 1, LPW, kRows)) != SRL_OK) return rc;
+  if ((rc = make_map(&q.maps.on_reset, p.on_reset, p.L, p.N, 1, LPW, kRows)) != SRL_OK) return rc;
   const bool vtrace = p.vt_new_logp != nullptr;
   const bool pack = p.pack != nullptr;
   if (vtrace) {  // [L-1, N]: the last row of the top stage reads as zero and is never used
-    if ((rc = make_map(&q.maps.vt_new, p.vt_new_logp, p.L - 1, p.N, 4, LPW)) != SRL_OK) return rc;
-    if ((rc = make_map(&q.maps.old_logp, p.vt_old_logp, p.L - 1, p.N, 4, LPW)) != SRL_OK) return rc;
+    if ((rc = make_map(&q.maps.vt_new, p.vt_new_logp, p.L - 1, p.N, 4, LPW, kRows)) != SRL_OK) return rc;
+    if ((rc = make_map(&q.maps.old_logp, p.vt_old_logp, p.L - 1, p.N, 4, LPW, kRows)) != SRL_OK) return rc;
     // the pack's old_logp is the sample leaf the V-trace ratio uses as well
     return pack ? launch<true, true, false, false, LPW>(q, st) : launch<true, false, false, false, LPW>(q, st);
   }
   const bool full = p.N % LPW == 0, popart = p.popart != nullptr;
   if (pack) {
-    if ((rc = make_map(&q.maps.old_logp, p.old_logp, p.L, p.N, 4, LPW)) != SRL_OK) return rc;
+    if ((rc = make_map(&q.maps.old_logp, p.old_logp, p.L, p.N, 4, LPW, kRows)) != SRL_OK) return rc;
     if (!full) return launch<false, true, false, false, LPW>(q, st);
     return popart ? launch<false, true, true, true, LPW>(q, st) : launch<false, true, true, false, LPW>(q, st);
   }

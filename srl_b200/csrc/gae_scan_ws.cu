@@ -11,10 +11,8 @@
 // handing chunks over through mbarriers (tma_full -> pass1_done -> scanned -> empty), so the scan of chunk k overlaps the
 // loads of chunk k+2, the delta pass of k+1 and the store pass of k-1, and the chain runs at ~22 cycles per row instead
 // of ~200.  The extra row of every box (row t+16) gives each chunk its own copy of the next-row inputs: no state crosses
-// chunks except the scanner's A.  Per-cell arithmetic is the TMA kernel's, operation for operation (bit-identical).
+// chunks except the scanner's A.  The per-cell arithmetic is gae_common.cuh's, shared with the other scan kernels.
 // V-trace is not handled here (the other two kernels do).
-#include <stdlib.h>
-
 #include "gae_common.cuh"
 #include "tma_util.cuh"
 
@@ -23,10 +21,9 @@ namespace {
 
 using namespace srl::tma;
 
-__device__ __forceinline__ void st_cg256(float4* p, float a0, float a1, float a2, float a3, float b0, float b1, float b2,
-                                         float b3) {
-  asm volatile("st.global.cg.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "f"(a0), "f"(a1), "f"(a2), "f"(a3),
-               "f"(b0), "f"(b1), "f"(b2), "f"(b3)
+__device__ __forceinline__ void st_cg256(float4* p, float4 a, float4 b) {
+  asm volatile("st.global.cg.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "f"(a.x), "f"(a.y), "f"(a.z), "f"(a.w),
+               "f"(b.x), "f"(b.y), "f"(b.z), "f"(b.w)
                : "memory");
 }
 
@@ -128,7 +125,7 @@ __global__ void __launch_bounds__(32 * (2 + kW)) gae_scan_ws_kernel(const __grid
       SRL_TL(1, blockIdx.x, 2);
     }
   } else if (warp == 1) {
-    // ---- scanner: A_t = delta_t + m_t * A_{t+1}, separate multiply and add as the reference's two torch ops (gae.py:92)
+    // ---- scanner: A_t = delta_t + m_t * A_{t+1} ---------------------------------------------------------------------
     const double gl = p.gamma_lmbda;
     double g = 0.0;
     for (int c = 0; c < n_chunks; ++c) {
@@ -146,11 +143,11 @@ __global__ void __launch_bounds__(32 * (2 + kW)) gae_scan_ws_kernel(const __grid
 #pragma unroll
       for (int r = 0; r < kR; ++r) {
         d[r] = sd[r * 32 + lane];
-        m[r] = sm[r * 32 + lane] ? gl : 0.0;
+        m[r] = gae_carry(sm[r * 32 + lane] != 0, gl);
       }
 #pragma unroll
       for (int r = kR - 1; r >= 0; --r) {
-        g = __dadd_rn(d[r], __dmul_rn(m[r], g));
+        g = gae_step(d[r], m[r], g);
         sa[r * 32 + lane] = static_cast<float>(g);  // adv.float(), gae.py:97
       }
       __syncwarp();
@@ -205,14 +202,7 @@ __global__ void __launch_bounds__(32 * (2 + kW)) gae_scan_ws_kernel(const __grid
         s_mb[i] = static_cast<uint8_t>(slot);
       }
     }
-    double s1 = 0, s2 = 0, s3 = 0, s4 = 0;
-    int cnt = 0, n_dn = 0, n_tr = 0;
-
-    auto vprime_of = [&](float x, bool dn) {
-      if (popart)  // RunningMeanStd.denormalize: (x.double() * std + mean).float()   utils.py:146-151
-        x = static_cast<float>(__dadd_rn(__dmul_rn(static_cast<double>(x), pa_std), pa_mean));
-      return __fmul_rn(x, dn ? 0.f : 1.f);  // value * (1 - done), fp32   mappo.py:120-124
-    };
+    LaneStats st;
     // pass 1 of chunk c: v', delta_t and the carry flag of this warp's rows
     auto pass1 = [&](int c) {
       const int s = c % kS;
@@ -232,17 +222,13 @@ __global__ void __launch_bounds__(32 * (2 + kW)) gae_scan_ws_kernel(const __grid
       for (int i = 0; i < kRowsPerWorker; ++i) {
         const int r = w * kRowsPerWorker + i;
         const int t = tbase + r;
-        const float v0 = vprime_of(sv[r * 32 + lane], sdn[r * 32 + lane] != 0);
-        const float v1 = vprime_of(sv[(r + 1) * 32 + lane], sdn[(r + 1) * 32 + lane] != 0);
+        const float v0 = gae_vprime(sv[r * 32 + lane], sdn[r * 32 + lane] != 0, popart, pa_mean, pa_std);
+        const float v1 = gae_vprime(sv[(r + 1) * 32 + lane], sdn[(r + 1) * 32 + lane] != 0, popart, pa_mean, pa_std);
         const bool rn = srs[(r + 1) * 32 + lane] != 0, tn = str_[(r + 1) * 32 + lane] != 0;
-        // gae.py:63  reward + gamma * value[1:] * (1 - on_reset[1:]) - value[:-1]
-        double dlt = __dmul_rn(__dmul_rn(gamma, static_cast<double>(v1)), rn ? 0.0 : 1.0);
-        dlt = __dadd_rn(static_cast<double>(sr[r * 32 + lane]), dlt);
-        dlt = __dsub_rn(dlt, static_cast<double>(v0));
+        const double dlt = gae_delta(&sr[r * 32 + lane], v0, v1, rn, gamma);
         const bool scanned = t < L - 1;  // row L-1 (padding row) and the zero-filled rows beyond carry no advantage
         sd[r * 32 + lane] = scanned ? dlt : 0.0;
-        // gae.py:87  gamma * lmbda * (1 - on_reset[1:]) * (1 - truncated[1:]): exactly 0 or gamma*lmbda
-        sm[r * 32 + lane] = (scanned && !rn && !tn) ? 1 : 0;
+        sm[r * 32 + lane] = (scanned && !rn && !tn) ? 1 : 0;  // the scanner's gae_carry flag
         svp[r * 32 + lane] = v0;
       }
       __syncwarp();
@@ -266,7 +252,7 @@ __global__ void __launch_bounds__(32 * (2 + kW)) gae_scan_ws_kernel(const __grid
         const int r = w * kRowsPerWorker + i;
         const int t = tbase + r;
         const float a = sa[r * 32 + lane];
-        const float rt = (t < L - 1) ? __fadd_rn(a, svp[r * 32 + lane]) : 0.f;  // value_target = adv + v'[:-1]   mappo.py:143
+        const float rt = (t < L - 1) ? gae_value_target(a, svp[r * 32 + lane]) : 0.f;
         const bool rn = srs[(r + 1) * 32 + lane] != 0;
         if (live && t < L) {  // row L-1 is the zero padding row of mappo.py:254-256
           const size_t gi = static_cast<size_t>(t) * N + col;
@@ -275,26 +261,17 @@ __global__ void __launch_bounds__(32 * (2 + kW)) gae_scan_ws_kernel(const __grid
           if (PACK && (r & 1) == 0) {
             // the pack's row pair (t, t + 1) as ONE 32-byte store: chunks start at even rows, and everything row t + 1
             // needs (its advantage, v', flags) is in this chunk's slot once the scanner has signalled it
-            const float nan = __int_as_float(0x7fc00000);
             const float a1 = sa[(r + 1) * 32 + lane];
-            const float rt1 = (t + 1 < L - 1) ? __fadd_rn(a1, svp[(r + 1) * 32 + lane]) : 0.f;
+            const float rt1 = (t + 1 < L - 1) ? gae_value_target(a1, svp[(r + 1) * 32 + lane]) : 0.f;
             const bool keep1 = t + 1 < L - 1 && srs[(r + 2) * 32 + lane] == 0;
-            st_cg256(reinterpret_cast<float4*>(p.pack) + pack_index(t, N, col), sol[r * 32 + lane], sv[r * 32 + lane], rt,
-                     (!rn && t < L - 1) ? a : nan, sol[(r + 1) * 32 + lane], sv[(r + 1) * 32 + lane], rt1, keep1 ? a1 : nan);
+            st_cg256(reinterpret_cast<float4*>(p.pack) + pack_index(t, N, col),
+                     pack_item(sol[r * 32 + lane], sv[r * 32 + lane], rt, a, !rn && t < L - 1),
+                     pack_item(sol[(r + 1) * 32 + lane], sv[(r + 1) * 32 + lane], rt1, a1, keep1));
           }
         }
         // loss rows [row_lo, row_hi), mask = 1 - on_reset[t+1]   mappo.py:259-261
         const bool in_rows = t >= p.row_lo && t < p.row_hi;
-        const bool mk = in_rows && !rn;
-        const double x = static_cast<double>(mk ? a : 0.f);
-        const double y = static_cast<double>(mk ? rt : 0.f);
-        cnt += mk ? 1 : 0;
-        s1 += x;
-        s2 = __fma_rn(x, x, s2);
-        s3 += y;
-        s4 = __fma_rn(y, y, s4);
-        n_dn += (in_rows && sdn[r * 32 + lane] != 0) ? 1 : 0;
-        n_tr += (in_rows && str_[r * 32 + lane] != 0) ? 1 : 0;
+        st.add(in_rows, in_rows && !rn, a, rt, sdn[r * 32 + lane] != 0, str_[r * 32 + lane] != 0);
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(&bars->empty[s]);
@@ -309,37 +286,28 @@ __global__ void __launch_bounds__(32 * (2 + kW)) gae_scan_ws_kernel(const __grid
     // per-lane statistics of this worker -> shared memory; the workers' tables are added in worker order below (fixed)
     if (p.lane_part != nullptr) {
       double* red = reinterpret_cast<double*>(smem + kS * SL::bytes + kStatsOff) + (w * 7) * 32;  // [kW][7][32] f64, own region
-      red[0 * 32 + lane] = static_cast<double>(cnt);
-      red[1 * 32 + lane] = s1;
-      red[2 * 32 + lane] = s2;
-      red[3 * 32 + lane] = s3;
-      red[4 * 32 + lane] = s4;
-      red[5 * 32 + lane] = static_cast<double>(n_dn);
-      red[6 * 32 + lane] = static_cast<double>(n_tr);
+      red[0 * 32 + lane] = static_cast<double>(st.cnt);
+      red[1 * 32 + lane] = st.s1;
+      red[2 * 32 + lane] = st.s2;
+      red[3 * 32 + lane] = st.s3;
+      red[4 * 32 + lane] = st.s4;
+      red[5 * 32 + lane] = static_cast<double>(st.dn);
+      red[6 * 32 + lane] = static_cast<double>(st.tr);
     }
   }
   __syncthreads();
   if (p.lane_part != nullptr) {
     const double* red = reinterpret_cast<const double*>(smem + kS * SL::bytes + kStatsOff);
-    for (int o = threadIdx.x; o < SRL_LANE_PART * 32; o += kThreads) {
-      const int k = o >> 5, ln = o & 31;
-      const int c2 = col0 + ln;
-      if (c2 < N) {
-        double sum = 0.0;
-        if (k < 7)
-          for (int ww = 0; ww < kW; ++ww) sum += red[(ww * 7 + k) * 32 + ln];
-        p.lane_part[static_cast<size_t>(k) * N + c2] = sum;
-        if (p.lane_aos != nullptr && k < 4) p.lane_aos[static_cast<size_t>(c2) * 4 + k] = k < 3 ? sum : 0.0;
-        if (k < 3) reinterpret_cast<double*>(smem + kS * SL::bytes + kPartOff)[k * 32 + ln] = sum;
-      }
-    }
+    double* lsum = reinterpret_cast<double*>(smem + kS * SL::bytes + kPartOff);  // the minibatch shares' lane sums
+    fold_lane_sums<32, kW, kThreads>(p, red, [&](int k, int ln, double sum) {
+      if (k < 3) lsum[k * 32 + ln] = sum;
+    });
     if (p.perm.out != nullptr && p.perm.part != nullptr) {
       // this CTA's share of every minibatch's {count, sum, sum of squares}, part[slot][cta][4]: the loss kernel adds
       // gridDim.x shares per minibatch (one coalesced round of loads) instead of gathering the minibatch's lane items
       // through the permutation (two dependent rounds).  Four threads per output, 8 lanes each in lane order, then
       // (q0 + q1) + (q2 + q3): a fixed order.
       __syncthreads();
-      const double* lsum = reinterpret_cast<const double*>(smem + kS * SL::bytes + kPartOff);
       const uint8_t* s_mb = smem + kS * SL::bytes + kPartOff + 3 * 32 * sizeof(double);
       const int outs = p.perm.n_epochs * p.perm.minibatches * 4;
       for (int i = threadIdx.x; i < ((outs * 4 + 31) & ~31); i += kThreads) {  // whole warps iterate together
@@ -373,14 +341,9 @@ int launch_ws(const WsParams& q, cudaStream_t st) {
   const size_t smem = 3 * 32 * sizeof(double) + kPartEpochs * 32 +  // lane sums + lane -> minibatch map (srl_gae_scan_perm)
                       static_cast<size_t>(kS) * Slot<PACK>::bytes + (sizeof(Bars<kS>) + 255) / 256 * 256 +
                       static_cast<size_t>(kW) * 7 * 32 * sizeof(double);
-  auto kern = gae_scan_ws_kernel<PACK, kW, kS>;
-  static bool opted_in[64] = {};
-  int dev = 0;
-  SRL_CUDA(cudaGetDevice(&dev));
-  if (dev < 64 && !opted_in[dev]) {
-    SRL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    opted_in[dev] = true;
-  }
+  constexpr auto kern = gae_scan_ws_kernel<PACK, kW, kS>;
+  const int rc = opt_in_smem<kern>(smem);
+  if (rc != SRL_OK) return rc;
   const int grid = (q.p.N + 31) / 32;
   SRL_CUDA(launch_pdl_scan(kern, dim3(grid), dim3(32 * (2 + kW)), smem, st, q));
   return SRL_OK;
@@ -391,27 +354,14 @@ int launch_ws(const WsParams& q, cudaStream_t st) {
 SRL_TL_SETTER(srl_tl_set_gae)
 namespace srl {
 
-bool gae_ws_eligible(const GaeParams& p) {
-  // same TMA requirements as the one-warp kernel (16-byte aligned bases and row pitches); no V-trace
-  if (p.vt_new_logp != nullptr || p.N % 16 != 0 || tma::encode_fn() == nullptr) return false;
-  const void* ptrs[] = {p.reward, p.value, p.done, p.truncated, p.on_reset};
-  for (const void* q : ptrs)
-    if (!aligned(q, 16)) return false;
-  if (p.pack && !aligned(p.old_logp, 16)) return false;
-  return true;
-}
+bool gae_ws_eligible(const GaeParams& p) { return p.vt_new_logp == nullptr && gae_tma_eligible(p); }
 
 int launch_gae_ws(const GaeParams& p, cudaStream_t st) {
   WsParams q;
   q.p = p;
   int rc;
   // at most one CTA per SM anyway: spend the SM's shared memory on a ring that holds the whole trajectory
-  // (SRL_GAE_WS_DEEP=0: the 3-slot ring, a tuning knob for profiles/)
-  static const bool deep_ok = [] {
-    const char* e = getenv("SRL_GAE_WS_DEEP");
-    return e == nullptr || e[0] != '0';
-  }();
-  const bool deep = deep_ok && (p.N + 31) / 32 <= sm_count();
+  const bool deep = (p.N + 31) / 32 <= sm_count();
   if ((rc = tma::make_map(&q.maps.value, p.value, p.L, p.N, 4, 32, kR + 1)) != SRL_OK) return rc;
   if ((rc = tma::make_map(&q.maps.reward, p.reward, p.L, p.N, 4, 32, kR)) != SRL_OK) return rc;
   if ((rc = tma::make_map(&q.maps.done, p.done, p.L, p.N, 1, 32, kR + 1)) != SRL_OK) return rc;

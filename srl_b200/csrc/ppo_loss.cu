@@ -31,6 +31,7 @@
 #include <string.h>
 
 #include "ppo_loss.cuh"
+#include "tma_util.cuh"
 
 namespace srl {
 namespace loss {
@@ -67,8 +68,8 @@ struct LogitsParams {
 // the staged [256, SK + 1] block was walked once per pass (max, exp / sum, entropy, gradient) with a run-time trip count,
 // staged in and out element by element with an integer division each, every shared-memory store behind its own global
 // load -- 98 us for 91 MB, neither bandwidth- nor issue-bound.  Now:
-//  * staging is ONE bulk asynchronous copy per tile and direction (cp.async.bulk, completion on an mbarrier / a bulk
-//    group): the block is contiguous in global memory and dense in shared memory;
+//  * staging is ONE bulk asynchronous copy per tile and direction (tma::bulk_load / bulk_store, completion on an mbarrier /
+//    a bulk group): the block is contiguous in global memory and dense in shared memory;
 //  * a head of <= 32 actions lives in registers for the forward passes and again for the gradient pass, in instantiations
 //    of 4, 8, ... 32 registers (loops unrolled, addresses immediate); e_k = exp(z_k - max) is kept in a second dense block
 //    when both fit (CACHE_E), so the gradient pass needs no exponential; wider heads keep the row walk;
@@ -77,8 +78,6 @@ struct LogitsParams {
 #define SRL_K4B_MIN_BLOCKS 2
 #endif
 constexpr int kStage = 9;  // manual staging batch per thread (last, partial tile only)
-
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
 
 // forward passes of one head held in registers: log-sum-exp, 1 / sum, entropy; e_k to `ez` when CACHE_E
 template <int KM, bool CACHE_E>
@@ -156,8 +155,8 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
   float* erow = srow + 256 * SK;
   uint64_t* bar = reinterpret_cast<uint64_t*>(srow + (CACHE_E ? 2 : 1) * 256 * SK);
   if (threadIdx.x == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(bar)));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    tma::mbar_init(bar, 1);
+    tma::mbar_fence_init();
   }
   __syncthreads();
   uint32_t parity = 0;
@@ -174,11 +173,8 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
     if (bulk) {
       if (threadIdx.x == 0) {
         const uint32_t bytes = static_cast<uint32_t>(total) * 4u;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                         smem_addr(srow)),
-                     "l"(src), "r"(bytes), "r"(smem_addr(bar))
-                     : "memory");
+        tma::mbar_expect_tx(bar, bytes);
+        tma::bulk_load(srow, src, bytes, bar);
       }
     } else {
       for (int e0 = threadIdx.x; e0 < total; e0 += 256 * kStage) {
@@ -209,18 +205,7 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
       for (int hd = 0; hd < SRL_MAX_HEADS; ++hd) act[hd] = hd < q.heads ? q.action[i * q.heads + hd] : 0;
     }
     if (bulk) {
-      uint32_t done = 0;
-      while (!done) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n"
-            : "=r"(done)
-            : "r"(smem_addr(bar)), "r"(parity)
-            : "memory");
-      }
+      tma::mbar_wait(bar, parity);
       parity ^= 1u;
     } else {
       __syncthreads();
@@ -293,15 +278,9 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
       }
     }
     if (bulk) {
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the gradients above, before the bulk copy reads them
+      tma::fence_proxy_async_smem();  // the gradients above, before the bulk copy reads them
       __syncthreads();
-      if (threadIdx.x == 0) {
-        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_addr(srow)),
-                     "r"(static_cast<uint32_t>(total) * 4u)
-                     : "memory");
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-        asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // the block may be overwritten by the next tile
-      }
+      if (threadIdx.x == 0) tma::bulk_store(dst, srow, static_cast<uint32_t>(total) * 4u);  // read before the next tile
       __syncthreads();
     } else {
       __syncthreads();
@@ -594,14 +573,8 @@ extern "C" int srl_ppo_loss_from_logits(const float* logits, const int32_t* acti
   pr.out = out;
   pr.out_f32 = out_f32;
   pr.slot = reinterpret_cast<SlotHeader*>(workspace);
-  static bool opted_in[64] = {};
-  int dev = 0;
-  SRL_CUDA(cudaGetDevice(&dev));
-  if (dev < 64 && !opted_in[dev]) {
-    SRL_CUDA(cudaFuncSetAttribute(ppo_loss_logits_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    SRL_CUDA(cudaFuncSetAttribute(ppo_loss_logits_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    opted_in[dev] = true;
-  }
+  if ((rc = opt_in_smem<ppo_loss_logits_kernel<true>>(200 * 1024)) != SRL_OK) return rc;
+  if ((rc = opt_in_smem<ppo_loss_logits_kernel<false>>(200 * 1024)) != SRL_OK) return rc;
   const long long tiles = (static_cast<long long>(T) * n + 255) / 256;
   // one wave: as many CTAs as are resident with this much shared memory (2048 tiles on 1184 assumed slots were 1024 CTAs on
   // the 740 real ones -- a second, partial wave)

@@ -1,4 +1,5 @@
-// mbarrier / TMA helpers for the warp-specialised GAE scan (gae_scan_ws.cu).
+// mbarrier, TMA and bulk-copy helpers: the GAE scan kernels (gae_scan_tma.cu, gae_scan_ws.cu) and the loss-from-logits
+// kernel (ppo_loss.cu).
 #pragma once
 #include <cuda.h>
 
@@ -43,6 +44,21 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
 }
 __device__ __forceinline__ void prefetch_map(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
+}
+// `bytes` (a multiple of 16, both addresses 16-byte aligned) from global to shared memory; completes on `bar`
+__device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
+               "l"(src), "r"(bytes), "r"(smem_u32(bar))
+               : "memory");
+}
+// the calling threads' shared-memory writes, before a bulk copy reads them
+__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+// `bytes` from shared to global memory; returns once the source has been read (it may be overwritten then)
+__device__ __forceinline__ void bulk_store(void* dst, const void* src, uint32_t bytes) {
+  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(src)), "r"(bytes)
+               : "memory");
+  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+  asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 #endif  // __CUDACC__
 
