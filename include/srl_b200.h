@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SRL_B200_ABI_VERSION 9
+#define SRL_B200_ABI_VERSION 10
 
 typedef void* srl_stream_t; /* cudaStream_t */
 
@@ -335,6 +335,38 @@ int srl_ppo_loss_from_logits(
     const srl_ppo_hyper* hyper, float* g_logits, /* [T, n, sumK] out */
     float* g_value,                               /* [T, n] out */
     float* logp_out, float* entropy_out,          /* [T, n] out or NULL */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
+ * K4c  Same loss, but starting from a diagonal-Gaussian actor head (continuous actions, D = 1 .. 64 dimensions).
+ * NEW capability: the reference's policies are categorical, so no reference line pins this head; the definition is
+ * torch.distributions.Normal(mean, exp(log_std)), summed over the action dimensions, as any PyTorch Gaussian policy
+ * computes it (sigma = exp(s)):
+ *   logp = sum_d [ -(a_d - mu_d)^2 / (2 sigma_d^2) - log sigma_d - log sqrt(2 pi) ]     (.log_prob(a).sum(-1))
+ *   H    = sum_d [ 0.5 + 0.5 log(2 pi) + log sigma_d ]                                    (.entropy().sum(-1))
+ * The loss, the ten outputs and the masking are K4's.  Writes
+ *   g_mean[i, d]    = g_lp (a_d - mu_d) / sigma_d^2
+ *   g_log_std[i, d] = g_lp ((a_d - mu_d)^2 / sigma_d^2 - 1) + g_en
+ * with (g_lp, g_en) = d loss / d (logp, H) of transition i, and d loss / d v_pred.  log_std_shared != 0: log_std is ONE
+ * [D] vector for every transition (a state-independent parameter) and g_log_std[d] is the sum of the expression above
+ * over the T * n transitions, added in float64 in a fixed order (deterministic for a given launch shape) and complete
+ * when the launch completes, in both finalisation modes.
+ * The workspace (zero before first use, left zero) starts with a K4 slot of srl_ppo_loss_workspace_bytes(T, n) bytes, so
+ * out == NULL followed by srl_ppo_loss_finalize(workspace, srl_ppo_loss_gaussian_workspace_bytes(...), 1, ...) works as
+ * for srl_ppo_loss_fwd_bwd; with a shared log_std the float64 partial rows of its gradient follow the slot.
+ * D outside [1, 64] is an invalid argument.
+ * ------------------------------------------------------------------------------------------ */
+size_t srl_ppo_loss_gaussian_workspace_bytes(int T, int n, int D, int log_std_shared);
+int srl_ppo_loss_from_gaussian(
+    const float* mean, const float* log_std, int log_std_shared, /* [T,n,D]; log_std [T,n,D] or [D] */
+    const float* action, int D,                                    /* [T,n,D] float32                    */
+    const float* v_pred,                                           /* [T,n]                              */
+    const float* old_logp, const float* old_value, const float* ret, const float* adv,
+    const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper,
+    float* g_mean, float* g_log_std /* [T,n,D] or [D] */, float* g_value,
+    float* logp_out, float* entropy_out,                           /* [T,n] or NULL                      */
     double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------

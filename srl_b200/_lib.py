@@ -20,7 +20,7 @@ SRL_LOSS_OUT_LEN = 16
 SRL_MAX_LEAVES = 32
 SRL_MAX_HEADS = 8
 SRL_MAX_LOSS_BATCH = 32
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 # enum srl_loss_out
 OUT_LOSS, OUT_POLICY_LOSS, OUT_VALUE_LOSS, OUT_ENTROPY_LOSS = 0, 1, 2, 3
@@ -106,6 +106,12 @@ SIGNATURES = {
                                          c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_size_t, c_void_p]),
+    "srl_ppo_loss_gaussian_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
+    "srl_ppo_loss_from_gaussian": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
+                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                           c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                           c_void_p, c_size_t, c_void_p]),
     "srl_philox_perm": (c_int, [c_uint64, c_uint32, c_int, c_int, c_int, c_void_p, c_void_p]),
     "srl_philox4x32_10": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "srl_batch_gather": (c_int, [POINTER(LeafDesc), c_int, c_void_p, c_int, c_int, c_void_p]),

@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "libsrl_b200.so")
 SOURCES = ["api.cu", "gae_scan.cu", "gae_scan_tma.cu", "gae_scan_ws.cu", "ppo_loss.cu", "ppo_loss_dense.cu", "ppo_loss_gather.cu",
-           "ppo_loss_pack.cu", "ppo_loss_pair.cu", "stats.cu", "perm.cu", "gather.cu", "xchg.cu", "nstep.cu", "gae_general.cu", "host_copy.cu", "rnn_chunk.cu", "blosc_decode.cu"]
+           "ppo_loss_pack.cu", "ppo_loss_pair.cu", "ppo_loss_gaussian.cu", "stats.cu", "perm.cu", "gather.cu", "xchg.cu", "nstep.cu", "gae_general.cu", "host_copy.cu", "rnn_chunk.cu", "blosc_decode.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",  # B200 only; no PTX for other archs, no fallback

@@ -299,6 +299,8 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
 }
 #undef SRL_HEAD_DISPATCH
 
+}  // namespace
+
 int fill_loss_hyper(const srl_ppo_hyper* hyper, const double* popart_mean_std, LossHyperDev& h) {
   SRL_REQUIRE(hyper != nullptr, SRL_ERR_INVALID_ARG, "ppo loss: null hyper pointer");
   SRL_REQUIRE(hyper->value_loss >= SRL_VL_MSE && hyper->value_loss <= SRL_VL_SMOOTHL1, SRL_ERR_INVALID_ARG,
@@ -320,7 +322,6 @@ int fill_loss_hyper(const srl_ppo_hyper* hyper, const double* popart_mean_std, L
   return SRL_OK;
 }
 
-}  // namespace
 }  // namespace loss
 }  // namespace srl
 

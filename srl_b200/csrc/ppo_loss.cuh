@@ -611,6 +611,8 @@ int launch_loss_mode(LossBatch& b, int n_problems, bool lanes4, cudaStream_t st)
   return launch_loss_static<4, MODE>(b, n_problems, st);
 }
 
+// ppo_loss.cu: the host-side check of the hyper-parameters, shared by every loss entry point
+int fill_loss_hyper(const srl_ppo_hyper* hyper, const double* popart_mean_std, LossHyperDev& h);
 // defined in ppo_loss_dense.cu / ppo_loss_gather.cu / ppo_loss_pack.cu
 int launch_loss_dense(LossBatch& b, int n_problems, bool lanes4, cudaStream_t st);
 int launch_loss_gather(LossBatch& b, int n_problems, bool lanes4, cudaStream_t st);

@@ -626,6 +626,118 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     return g_logits, g_value, out, out_f32, logp, ent
 
 
+GAUSSIAN_MAX_D = 64
+_gaussian_workspaces = {}
+
+
+def gaussian_loss_workspace_bytes(T: int, n: int, D: int, log_std_shared: bool) -> int:
+    return int(_lib.load_library().srl_ppo_loss_gaussian_workspace_bytes(int(T), int(n), int(D), int(bool(log_std_shared))))
+
+
+def new_gaussian_loss_workspace(device, T: int = 1, n: int = 1, D: int = GAUSSIAN_MAX_D,
+                                log_std_shared: bool = True) -> torch.Tensor:
+    """Zero-initialised scratch for ppo_loss_from_gaussian (uint8); the default size serves every shape.  Its first
+    bytes are a loss slot, so a deferred launch is folded by loss_finalize(ws.view(1, -1), out)."""
+    return torch.zeros(gaussian_loss_workspace_bytes(T, n, D, log_std_shared), dtype=torch.uint8, device=device)
+
+
+def gaussian_loss_workspace(device) -> torch.Tensor:
+    """Default scratch of ppo_loss_from_gaussian: one buffer per (device, stream)."""
+    key = (torch.device(device).index, _stream())
+    ws = _gaussian_workspaces.get(key)
+    if ws is None:
+        ws = _gaussian_workspaces[key] = new_gaussian_loss_workspace(device)
+    return ws
+
+
+def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, ret, adv, on_reset_next, norm_stats,
+                           hyper: LossHyper, local_stats=None, popart_mean_std=None, lane_idx=None,
+                           want_logp_entropy: bool = False, workspace=None, defer: bool = False):
+    """Loss starting from a diagonal-Gaussian actor head: `mean` and float32 `action` `[T, n, D]`, `log_std` either
+    `[T, n, D]` (one per transition) or `[D]` (one parameter shared by every transition), D <= 64.  The head's log-prob
+    and entropy are torch.distributions.Normal(mean, log_std.exp()).log_prob(action).sum(-1) / .entropy().sum(-1); the
+    loss is ppo_loss_fwd_bwd's.  Returns (g_mean, g_log_std, g_value, out, out_f32, logp, entropy): g_log_std has
+    log_std's shape (a shared log_std gets the sum over the minibatch); logp / entropy `[T, n]` only with
+    want_logp_entropy.  `defer` (needs an explicit `workspace`): out / out_f32 are None and loss_finalize folds the
+    slot later; the gradients are complete either way."""
+    _check(v_pred, torch.float32, "v_pred")
+    T, n = _rows_lanes(v_pred)
+    _check(mean, torch.float32, "mean")
+    _check(action, torch.float32, "action")
+    D = mean.shape[-1] if mean.dim() >= 2 else 0
+    if mean.dim() < 2 or mean.shape[0] != T or mean.numel() != T * n * D:
+        raise ValueError(f"mean: expected [T, n, D] with [T, n] = [{T}, {n}] (v_pred), got shape {tuple(mean.shape)}")
+    if not 1 <= D <= GAUSSIAN_MAX_D:
+        raise ValueError(f"mean: D = {D} action dimensions, supported are 1 .. {GAUSSIAN_MAX_D}")
+    if tuple(action.shape) != tuple(mean.shape):
+        raise ValueError(f"action: shape {tuple(action.shape)} does not match mean {tuple(mean.shape)}")
+    if not isinstance(log_std, torch.Tensor):
+        raise ValueError("log_std: expected a CUDA tensor")
+    if tuple(log_std.shape) == (D,):
+        shared = True
+    elif tuple(log_std.shape) == tuple(mean.shape):
+        shared = False
+        if 0 in log_std.stride():
+            raise ValueError("log_std: a stride-0 expand of a [D] parameter; pass the [D] tensor itself (a shared log_std "
+                             "gets its gradient summed over the minibatch in the kernel)")
+    else:
+        raise ValueError(f"log_std: expected [D] = [{D}] (shared) or mean's shape {tuple(mean.shape)} (per transition), "
+                         f"got {tuple(log_std.shape)}")
+    _check(log_std, torch.float32, "log_std")
+    ld_smp = _sample_side(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, hyper.clip_value)
+    _check(norm_stats, torch.float64, "norm_stats")
+    local_stats = norm_stats if local_stats is None else _check(local_stats, torch.float64, "local_stats")
+    if popart_mean_std is not None:
+        _check(popart_mean_std, torch.float64, "popart_mean_std")
+    dev = mean.device
+    g_mean = torch.empty_like(mean)
+    g_log_std = torch.empty_like(log_std)
+    g_value = torch.empty_like(v_pred)
+    logp = torch.empty_like(v_pred) if want_logp_entropy else None
+    ent = torch.empty_like(v_pred) if want_logp_entropy else None
+    if defer:
+        if workspace is None:
+            raise ValueError("deferred finalisation needs an explicit workspace")
+        out = out_f32 = None
+    else:
+        out = torch.empty(SRL_LOSS_OUT_LEN, dtype=torch.float64, device=dev)
+        out_f32 = torch.empty(4, dtype=torch.float32, device=dev)
+    ws = gaussian_loss_workspace(dev) if workspace is None else _check(workspace, torch.uint8, "workspace")
+    hc = hyper.to_c()
+    _lib.call("srl_ppo_loss_from_gaussian", _ptr(mean), _ptr(log_std), int(shared), _ptr(action), D, _ptr(v_pred),
+              _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp, _ptr(lane_idx), T, n,
+              _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc), _ptr(g_mean),
+              _ptr(g_log_std), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws), ws.numel(),
+              _stream())
+    return g_mean, g_log_std, g_value, out, out_f32, logp, ent
+
+
+class PPOGaussianLossFunction(torch.autograd.Function):
+    """Autograd node for a continuous-action policy: forward returns the scalar loss (float32) and the float64 stats
+    vector of ppo_loss_from_gaussian; backward hands the gradients the same launch produced to mean, log_std ([D]
+    parameter or [T, n, D]) and v_pred.
+
+        loss, out = PPOGaussianLossFunction.apply(mean, log_std, action, v_pred, old_logp, old_value, ret, adv,
+                                                  on_reset_next, norm_stats, local_stats, popart_mean_std, lane_idx, hyper)
+        loss.backward()
+    """
+
+    @staticmethod
+    def forward(ctx, mean, log_std, action, v_pred, old_logp, old_value, ret, adv, on_reset_next, norm_stats, local_stats,
+                popart_mean_std, lane_idx, hyper):
+        g_mean, g_ls, g_v, out, out_f32, _, _ = ppo_loss_from_gaussian(
+            mean.detach(), log_std.detach(), action, v_pred.detach(), old_logp, old_value, ret, adv, on_reset_next,
+            norm_stats, hyper, local_stats=local_stats, popart_mean_std=popart_mean_std, lane_idx=lane_idx)
+        ctx.save_for_backward(g_mean, g_ls, g_v.view(v_pred.shape))
+        ctx.mark_non_differentiable(out)
+        return out_f32[0], out
+
+    @staticmethod
+    def backward(ctx, grad_loss, _grad_out):
+        g_mean, g_ls, g_v = ctx.saved_tensors
+        return (g_mean * grad_loss, g_ls * grad_loss, None, g_v * grad_loss) + (None,) * 10
+
+
 class PPOLossFunction(torch.autograd.Function):
     """Autograd node at the SampleAnalyzedResult boundary (mappo.py:21-33): forward returns the scalar
     loss (float32) and the float64 stats vector; the gradients were already produced by the same launch."""
