@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SRL_B200_ABI_VERSION 10
+#define SRL_B200_ABI_VERSION 11
 
 typedef void* srl_stream_t; /* cudaStream_t */
 
@@ -249,7 +249,7 @@ enum srl_loss_out {
  * before the slot is used again.  Launches that may overlap in time need distinct slots. */
 size_t srl_ppo_loss_workspace_bytes(int T, int n);
 
-/* Deferred finalisation: when srl_ppo_loss_fwd_bwd / srl_ppo_loss_from_logits are called with out == NULL they
+/* Deferred finalisation: when srl_ppo_loss_fwd_bwd / srl_ppo_loss_from_logits(_masked) are called with out == NULL they
  * stop after writing gradients and partial rows.  This folds n_slots consecutive slots (slot k at
  * workspace + k * slot_bytes) into out[k][SRL_LOSS_OUT_LEN] (and out_f32[k][4] if not NULL) in one launch, and
  * clears the rows it folded. */
@@ -322,12 +322,36 @@ int srl_ppo_loss_fwd_bwd_batched(const srl_loss_problem* problems_host, int n_pr
  * ActorCriticPolicy.__get_log_prob_and_entropy / get_action_distribution
  * (legacy/algorithm/ppo/actor_critic_policies/actor_critic_policy.py:303-324): per head h with K_h
  * logits z: lp = z - logsumexp(z); logp = sum_h lp[a_h]; H = sum_h -sum_k softmax(z)_k lp_k.
- * Writes d loss / d logits ([T, n, sumK]) and d loss / d v_pred.
+ * Writes d loss / d logits ([T, n, sumK]) and d loss / d v_pred.  sumK above SRL_K4B_MAX_SUM_K is SRL_ERR_UNSUPPORTED.
  * ------------------------------------------------------------------------------------------ */
 #define SRL_MAX_HEADS 8
+#define SRL_K4B_MAX_SUM_K 199
+#define SRL_K4B_MAX_SUM_K_MASKED 159
 int srl_ppo_loss_from_logits(
     const float* logits,   /* [T, n, sumK] dense */
     const int32_t* action, /* [T, n, heads]      */
+    const int32_t* head_sizes_host, int heads, const float* v_pred, /* [T, n] dense */
+    const float* old_logp, const float* old_value, const float* ret, const float* adv,
+    const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper, float* g_logits, /* [T, n, sumK] out */
+    float* g_value,                               /* [T, n] out */
+    float* logp_out, float* entropy_out,          /* [T, n] out or NULL */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+
+/* The same with an availability mask (SMAC's available_action): the reference's categorical policy replaces unavailable
+ * logits before it builds the distributions, logits.masked_fill(available_action == 0, -1e10)
+ * (legacy/algorithm/ppo/actor_critic_policies/actor_critic_policy.py:135-136).  available is one byte per logit, aligned
+ * with the logits across all heads; 0 = unavailable: that logit is float32(-1e10) for the log-prob, the entropy and the ten
+ * outputs, and its g_logits entry is exactly 0 (masked_fill passes no gradient), also where it is the chosen action (logp
+ * about -1e10, ratio 0, everything finite).  A head with no available action adds 0 to logp and to the entropy, as in torch
+ * (its log-sum-exp rounds to -1e10).  available must not be NULL; sumK above SRL_K4B_MAX_SUM_K_MASKED (the mask is staged
+ * in shared memory beside the logits) is SRL_ERR_UNSUPPORTED.  Everything else, the deferred mode included, is
+ * srl_ppo_loss_from_logits'. */
+int srl_ppo_loss_from_logits_masked(
+    const float* logits,      /* [T, n, sumK] dense */
+    const uint8_t* available, /* [T, n, sumK] dense, non-zero = available */
+    const int32_t* action,    /* [T, n, heads]      */
     const int32_t* head_sizes_host, int heads, const float* v_pred, /* [T, n] dense */
     const float* old_logp, const float* old_value, const float* ret, const float* adv,
     const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,

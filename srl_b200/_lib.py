@@ -19,8 +19,10 @@ SRL_LANE_PART = 8
 SRL_LOSS_OUT_LEN = 16
 SRL_MAX_LEAVES = 32
 SRL_MAX_HEADS = 8
+SRL_K4B_MAX_SUM_K = 199
+SRL_K4B_MAX_SUM_K_MASKED = 159
 SRL_MAX_LOSS_BATCH = 32
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 # enum srl_loss_out
 OUT_LOSS, OUT_POLICY_LOSS, OUT_VALUE_LOSS, OUT_ENTROPY_LOSS = 0, 1, 2, 3
@@ -106,6 +108,11 @@ SIGNATURES = {
                                          c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_size_t, c_void_p]),
+    "srl_ppo_loss_from_logits_masked": (c_int, [c_void_p, c_void_p, c_void_p, POINTER(c_int32), c_int, c_void_p,
+                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                                c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                c_size_t, c_void_p]),
     "srl_ppo_loss_gaussian_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
     "srl_ppo_loss_from_gaussian": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,

@@ -62,6 +62,7 @@ struct LogitsParams {
   float* entropy_out;     // [T*n] or null
   int heads, SK;
   int head_size[SRL_MAX_HEADS];
+  const uint8_t* available;  // [T*n, SK], 0 = unavailable (MASKED instantiations only)
 };
 
 // How the kernel got here (ncu, T=128 N=4096 K=18: profiles/r2_notes.md).  First version: 2180 instructions per transition --
@@ -79,12 +80,24 @@ struct LogitsParams {
 #endif
 constexpr int kStage = 9;  // manual staging batch per thread (last, partial tile only)
 
-// forward passes of one head held in registers: log-sum-exp, 1 / sum, entropy; e_k to `ez` when CACHE_E
-template <int KM, bool CACHE_E>
-__device__ __forceinline__ void head_forward(const float* z, float* ez, int K, float& l, float& inv, float& hh) {
+// actor_critic_policy.py:135-136: logits.masked_fill(available_action == 0, -1e10) before the Categorical
+constexpr float kUnavailableLogit = -1e10f;
+
+// logit k of a row as the Categorical sees it
+template <bool MASKED>
+__device__ __forceinline__ float logit_at(const float* z, const uint8_t* m, int k) {
+  return (MASKED && m[k] == 0) ? kUnavailableLogit : z[k];
+}
+
+// forward passes of one head held in registers: log-sum-exp, 1 / sum, entropy; e_k to `ez` when CACHE_E.  With MASKED,
+// `m` is the head's availability bytes and an unavailable logit reads as kUnavailableLogit (its e_k is 0 unless the whole
+// head is unavailable: then every lp_k is 0, as in torch, and the head adds nothing to logp or the entropy)
+template <int KM, bool CACHE_E, bool MASKED>
+__device__ __forceinline__ void head_forward(const float* z, float* ez, const uint8_t* m, int K, float& l, float& inv,
+                                             float& hh) {
   float v[KM];
 #pragma unroll
-  for (int k = 0; k < KM; ++k) v[k] = k < K ? z[k] : -INFINITY;
+  for (int k = 0; k < KM; ++k) v[k] = k < K ? logit_at<MASKED>(z, m, k) : -INFINITY;
   float mx = v[0];
 #pragma unroll
   for (int k = 1; k < KM; ++k) mx = fmaxf(mx, v[k]);
@@ -109,10 +122,11 @@ __device__ __forceinline__ void head_forward(const float* z, float* ez, int K, f
   }
 }
 
-// gradient pass of one head: z_k <- d loss / d z_k
-template <int KM, bool CACHE_E>
-__device__ __forceinline__ void head_backward(float* z, const float* ez, int K, int a, float l, float inv, float hh, float g_lp,
-                                              float g_en) {
+// gradient pass of one head: z_k <- d loss / d z_k; with MASKED an unavailable logit gets exactly 0 (masked_fill passes
+// no gradient), also when it is the chosen action, where the expression below is not 0
+template <int KM, bool CACHE_E, bool MASKED>
+__device__ __forceinline__ void head_backward(float* z, const float* ez, const uint8_t* m, int K, int a, float l, float inv,
+                                              float hh, float g_lp, float g_en) {
   float v[KM], e[KM];
 #pragma unroll
   for (int k = 0; k < KM; ++k) {
@@ -125,26 +139,30 @@ __device__ __forceinline__ void head_backward(float* z, const float* ez, int K, 
       const float lp = v[k] - l;
       const float pk = CACHE_E ? e[k] * inv : expf(lp);
       // d logp / d z_k = [k == a] - p_k ;  d H / d z_k = -p_k (lp_k + H)
-      z[k] = g_lp * ((k == a ? 1.f : 0.f) - pk) - g_en * pk * (fmaxf(lp, -FLT_MAX) + hh);
+      const float g = g_lp * ((k == a ? 1.f : 0.f) - pk) - g_en * pk * (fmaxf(lp, -FLT_MAX) + hh);
+      z[k] = (MASKED && m[k] == 0) ? 0.f : g;
     }
   }
 }
 
-#define SRL_HEAD_DISPATCH(FN, K, ...)                  \
-  do {                                                 \
-    if ((K) <= 4) FN<4, CACHE_E>(__VA_ARGS__);         \
-    else if ((K) <= 8) FN<8, CACHE_E>(__VA_ARGS__);    \
-    else if ((K) <= 12) FN<12, CACHE_E>(__VA_ARGS__);  \
-    else if ((K) <= 16) FN<16, CACHE_E>(__VA_ARGS__);  \
-    else if ((K) <= 20) FN<20, CACHE_E>(__VA_ARGS__);  \
-    else if ((K) <= 24) FN<24, CACHE_E>(__VA_ARGS__);  \
-    else if ((K) <= 28) FN<28, CACHE_E>(__VA_ARGS__);  \
-    else FN<32, CACHE_E>(__VA_ARGS__);                 \
+#define SRL_HEAD_DISPATCH(FN, K, ...)                         \
+  do {                                                        \
+    if ((K) <= 4) FN<4, CACHE_E, MASKED>(__VA_ARGS__);        \
+    else if ((K) <= 8) FN<8, CACHE_E, MASKED>(__VA_ARGS__);   \
+    else if ((K) <= 12) FN<12, CACHE_E, MASKED>(__VA_ARGS__); \
+    else if ((K) <= 16) FN<16, CACHE_E, MASKED>(__VA_ARGS__); \
+    else if ((K) <= 20) FN<20, CACHE_E, MASKED>(__VA_ARGS__); \
+    else if ((K) <= 24) FN<24, CACHE_E, MASKED>(__VA_ARGS__); \
+    else if ((K) <= 28) FN<28, CACHE_E, MASKED>(__VA_ARGS__); \
+    else FN<32, CACHE_E, MASKED>(__VA_ARGS__);                \
   } while (0)
 
-template <bool CACHE_E>
+// MASKED: the [256, SK] availability bytes of the tile follow the float blocks in shared memory, brought in with the logits
+// (same mbarrier and expect_tx, or the same element-wise staging); every pass over a head reads them.
+template <bool CACHE_E, bool MASKED>
 __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kernel(const __grid_constant__ LogitsParams q) {
-  extern __shared__ __align__(128) float srow[];  // [256 * SK] dense (+ [256 * SK] with CACHE_E), then the mbarrier
+  // [256 * SK] dense (+ [256 * SK] with CACHE_E), (+ [256 * SK] bytes with MASKED), then the mbarrier
+  extern __shared__ __align__(128) float srow[];
   const LossShared& p = q.s;
   const Problem& pr = q.pr;
   const LossHyperDev& h = p.h;
@@ -153,14 +171,16 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
   Acc acc;
   const int SK = q.SK;
   float* erow = srow + 256 * SK;
-  uint64_t* bar = reinterpret_cast<uint64_t*>(srow + (CACHE_E ? 2 : 1) * 256 * SK);
+  uint8_t* mrow = reinterpret_cast<uint8_t*>(srow + (CACHE_E ? 2 : 1) * 256 * SK);
+  uint64_t* bar = reinterpret_cast<uint64_t*>(mrow + (MASKED ? 256 * SK : 0));  // 256 * SK bytes keep it 8-byte aligned
   if (threadIdx.x == 0) {
     tma::mbar_init(bar, 1);
     tma::mbar_fence_init();
   }
   __syncthreads();
   uint32_t parity = 0;
-  const bool bulk_ok = ((reinterpret_cast<uintptr_t>(q.logits) | reinterpret_cast<uintptr_t>(q.g_logits)) & 15) == 0;
+  const bool bulk_ok = ((reinterpret_cast<uintptr_t>(q.logits) | reinterpret_cast<uintptr_t>(q.g_logits) |
+                         (MASKED ? reinterpret_cast<uintptr_t>(q.available) : 0)) & 15) == 0;
   const long long W = static_cast<long long>(p.T) * p.n;
   const long long tiles = (W + 255) / 256;
   for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
@@ -169,12 +189,15 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
     const int total = cnt * SK;
     const float* src = q.logits + i0 * SK;
     float* dst = q.g_logits + i0 * SK;
-    const bool bulk = bulk_ok && cnt == 256;  // 256 * SK * 4 bytes: a multiple of 16 at a 16-byte aligned address
+    // 256 * SK * 4 bytes of logits and 256 * SK bytes of mask: multiples of 16 at 16-byte aligned addresses
+    const bool bulk = bulk_ok && cnt == 256;
+    const uint8_t* msrc = MASKED ? q.available + i0 * SK : nullptr;
     if (bulk) {
       if (threadIdx.x == 0) {
         const uint32_t bytes = static_cast<uint32_t>(total) * 4u;
-        tma::mbar_expect_tx(bar, bytes);
+        tma::mbar_expect_tx(bar, MASKED ? bytes + static_cast<uint32_t>(total) : bytes);
         tma::bulk_load(srow, src, bytes, bar);
+        if (MASKED) tma::bulk_load(mrow, msrc, static_cast<uint32_t>(total), bar);
       }
     } else {
       for (int e0 = threadIdx.x; e0 < total; e0 += 256 * kStage) {
@@ -184,6 +207,16 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
 #pragma unroll
         for (int b = 0; b < kStage; ++b)
           if (e0 + b * 256 < total) srow[e0 + b * 256] = v[b];
+      }
+      if (MASKED) {
+        for (int e0 = threadIdx.x; e0 < total; e0 += 256 * kStage) {
+          uint8_t v[kStage];
+#pragma unroll
+          for (int b = 0; b < kStage; ++b) v[b] = (e0 + b * 256 < total) ? __ldg(msrc + e0 + b * 256) : 0;
+#pragma unroll
+          for (int b = 0; b < kStage; ++b)
+            if (e0 + b * 256 < total) mrow[e0 + b * 256] = v[b];
+        }
       }
     }
     // the sample side of this thread's transition, in flight while the block lands
@@ -213,6 +246,7 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
     if (mine) {
       float* z = srow + threadIdx.x * SK;
       float* ez = erow + threadIdx.x * SK;
+      const uint8_t* m = mrow + threadIdx.x * SK;
       // (the head loops are NOT unrolled: with the dispatch over eight widths inlined in each of SRL_MAX_HEADS slots the kernel
       // was 128 copies of the passes and spent 27 % of its warp samples waiting for instructions; the per-head scalars
       // below are indexed at run time and live in local memory -- four words per head)
@@ -225,13 +259,13 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
           const int K = q.head_size[hd];
           float l, inv, hh;
           if (K <= 32) {
-            SRL_HEAD_DISPATCH(head_forward, K, z + off, ez + off, K, l, inv, hh);
+            SRL_HEAD_DISPATCH(head_forward, K, z + off, ez + off, m + off, K, l, inv, hh);
           } else {
             float mx = -INFINITY;
-            for (int k = 0; k < K; ++k) mx = fmaxf(mx, z[off + k]);
+            for (int k = 0; k < K; ++k) mx = fmaxf(mx, logit_at<MASKED>(z, m, off + k));
             float se = 0.f;
             for (int k = 0; k < K; ++k) {
-              const float ek = expf(z[off + k] - mx);
+              const float ek = expf(logit_at<MASKED>(z, m, off + k) - mx);
               if (CACHE_E) ez[off + k] = ek;
               se += ek;
             }
@@ -239,7 +273,7 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
             inv = 1.f / se;
             hh = 0.f;
             for (int k = 0; k < K; ++k) {
-              const float lp = fmaxf(z[off + k] - l, -FLT_MAX);
+              const float lp = fmaxf(logit_at<MASKED>(z, m, off + k) - l, -FLT_MAX);
               const float pk = CACHE_E ? ez[off + k] * inv : expf(lp);
               hh -= pk * lp;
             }
@@ -247,7 +281,7 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
           lse[hd] = l;
           rse[hd] = inv;
           hent[hd] = hh;
-          logp += z[off + act[hd]] - l;
+          logp += logit_at<MASKED>(z, m, off + act[hd]) - l;
           ent += hh;
           off += K;
         }
@@ -265,12 +299,14 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
         {
           const int K = q.head_size[hd];
           if (K <= 32) {
-            SRL_HEAD_DISPATCH(head_backward, K, z + off, ez + off, K, act[hd], lse[hd], rse[hd], hent[hd], g_lp, g_en);
+            SRL_HEAD_DISPATCH(head_backward, K, z + off, ez + off, m + off, K, act[hd], lse[hd], rse[hd], hent[hd], g_lp,
+                              g_en);
           } else {
             for (int k = 0; k < K; ++k) {
               const float lp = z[off + k] - lse[hd];
               const float pk = CACHE_E ? ez[off + k] * rse[hd] : expf(lp);
-              z[off + k] = g_lp * ((k == act[hd] ? 1.f : 0.f) - pk) - g_en * pk * (fmaxf(lp, -FLT_MAX) + hent[hd]);
+              const float g = g_lp * ((k == act[hd] ? 1.f : 0.f) - pk) - g_en * pk * (fmaxf(lp, -FLT_MAX) + hent[hd]);
+              z[off + k] = (MASKED && m[off + k] == 0) ? 0.f : g;
             }
           }
           off += K;
@@ -298,6 +334,115 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
   reduce_and_finalize(pr, h, acc, mask_sum, blockIdx.x, gridDim.x);
 }
 #undef SRL_HEAD_DISPATCH
+
+// the largest sum K whose staged block(s) fit the 200 KiB opt-in below (include/srl_b200.h states both limits)
+static_assert(256 * SRL_K4B_MAX_SUM_K * 4 + 16 <= 200 * 1024 && 256 * (SRL_K4B_MAX_SUM_K + 1) * 4 + 16 > 200 * 1024, "");
+static_assert(256 * SRL_K4B_MAX_SUM_K_MASKED * 5 + 16 <= 200 * 1024 && 256 * (SRL_K4B_MAX_SUM_K_MASKED + 1) * 5 + 16 > 200 * 1024,
+              "");
+
+// one resident wave of ppo_loss_logits_kernel<CACHE_E, MASKED> over the T * n transitions of q
+template <bool MASKED>
+int launch_logits(const LogitsParams& q, bool cache_e, size_t smem, cudaStream_t stream) {
+  int rc;
+  if ((rc = opt_in_smem<ppo_loss_logits_kernel<true, MASKED>>(200 * 1024)) != SRL_OK) return rc;
+  if ((rc = opt_in_smem<ppo_loss_logits_kernel<false, MASKED>>(200 * 1024)) != SRL_OK) return rc;
+  const long long tiles = (static_cast<long long>(q.s.T) * q.s.n + 255) / 256;
+  // one wave: as many CTAs as are resident with this much shared memory (2048 tiles on 1184 assumed slots were 1024 CTAs on
+  // the 740 real ones -- a second, partial wave)
+  int per_sm = 0;
+  if ((cache_e ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<true, MASKED>, 256, smem)
+               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<false, MASKED>, 256, smem)) !=
+          cudaSuccess ||
+      per_sm < 1)
+    per_sm = 1;
+  const long long slots = static_cast<long long>(sm_count()) * per_sm;
+  const long long cap = slots < kMaxGrid ? slots : kMaxGrid;
+  // every CTA the same number of tiles (2048 tiles on 1184 slots would leave most CTAs one tile and the rest two)
+  const long long per_cta = (tiles + cap - 1) / cap;
+  const int grid = static_cast<int>((tiles + per_cta - 1) / per_cta);
+  if (cache_e)
+    ppo_loss_logits_kernel<true, MASKED><<<grid, 256, smem, stream>>>(q);
+  else
+    ppo_loss_logits_kernel<false, MASKED><<<grid, 256, smem, stream>>>(q);
+  SRL_CUDA(cudaGetLastError());
+  return SRL_OK;
+}
+
+// srl_ppo_loss_from_logits (available == NULL) and srl_ppo_loss_from_logits_masked
+int ppo_loss_from_logits(const char* fn, const float* logits, const uint8_t* available, const int32_t* action,
+                         const int32_t* head_sizes_host, int heads, const float* v_pred, const float* old_logp,
+                         const float* old_value, const float* ret, const float* adv, const uint8_t* on_reset_next,
+                         int64_t ld_smp, const int32_t* lane_idx, int T, int n, const double* norm_stats,
+                         const double* local_stats, const double* popart_mean_std, const srl_ppo_hyper* hyper,
+                         float* g_logits, float* g_value, float* logp_out, float* entropy_out, double* out, float* out_f32,
+                         void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  SRL_REQUIRE(T >= 1 && n >= 1, SRL_ERR_INVALID_ARG, "%s: need T >= 1 and n >= 1", fn);
+  SRL_REQUIRE(heads >= 1 && heads <= SRL_MAX_HEADS && head_sizes_host, SRL_ERR_INVALID_ARG,
+              "%s: heads=%d outside [1, %d]", fn, heads, SRL_MAX_HEADS);
+  SRL_REQUIRE(logits && action && v_pred && old_logp && ret && adv && on_reset_next && g_logits && g_value &&
+                  norm_stats && local_stats && workspace,
+              SRL_ERR_INVALID_ARG, "%s: null pointer", fn);
+  SRL_REQUIRE(ld_smp >= (lane_idx ? 1 : n), SRL_ERR_INVALID_ARG, "%s: ld_smp smaller than the row", fn);
+  SRL_REQUIRE(workspace_bytes >= srl_ppo_loss_workspace_bytes(T, n), SRL_ERR_INVALID_ARG,
+              "%s: workspace too small (%zu bytes)", fn, workspace_bytes);
+  LogitsParams q;
+  int rc = fill_loss_hyper(hyper, popart_mean_std, q.s.h);
+  if (rc != SRL_OK) return rc;
+  SRL_REQUIRE(!(q.s.h.clip_value && old_value == nullptr), SRL_ERR_INVALID_ARG, "%s: clip_value needs old_value", fn);
+  int sk = 0;
+  for (int i = 0; i < SRL_MAX_HEADS; ++i) {
+    q.head_size[i] = i < heads ? head_sizes_host[i] : 0;
+    SRL_REQUIRE(i >= heads || head_sizes_host[i] >= 1, SRL_ERR_INVALID_ARG, "%s: head %d has no actions", fn, i);
+    sk += q.head_size[i];
+  }
+  const bool masked = available != nullptr;
+  const size_t row_bytes = static_cast<size_t>(256) * sk * sizeof(float);  // dense [256, sum K] block
+  const size_t mask_bytes = masked ? static_cast<size_t>(256) * sk : 0;    // + its [256, sum K] availability bytes
+  const int max_sk = masked ? SRL_K4B_MAX_SUM_K_MASKED : SRL_K4B_MAX_SUM_K;
+  SRL_REQUIRE(row_bytes + mask_bytes + 16 <= 200 * 1024, SRL_ERR_UNSUPPORTED, "%s: sum K = %d too wide (max %d)", fn, sk,
+              max_sk);
+  const bool cache_e = 2 * row_bytes + mask_bytes + 16 <= 200 * 1024;  // both blocks fit: one exponential per logit
+  const size_t smem = (cache_e ? 2 * row_bytes : row_bytes) + mask_bytes + 16;  // + the mbarrier of the bulk copies
+  q.heads = heads;
+  q.SK = sk;
+  q.logits = logits;
+  q.available = available;
+  q.action = action;
+  q.g_logits = g_logits;
+  q.logp_out = logp_out;
+  q.entropy_out = entropy_out;
+  LossShared& p = q.s;
+  p.old_logp = old_logp;
+  p.old_value = old_value;
+  p.ret = ret;
+  p.adv = adv;
+  p.reset_next = on_reset_next;
+  p.pack = nullptr;
+  p.lane_aos = nullptr;
+  p.part = nullptr;
+  p.part_ctas = p.part_first = 0;
+  p.row_lo = 0;
+  p.popart = popart_mean_std;
+  p.ld_pol = n;
+  p.ld_grad = n;
+  p.ld_smp = ld_smp;
+  p.T = T;
+  p.n = n;
+  p.rows_per_tile = p.col_tiles = p.n_tiles = 0;
+  p.smp_vec_ok = 0;
+  Problem& pr = q.pr;
+  pr.new_logp = pr.entropy = nullptr;
+  pr.v_pred = v_pred;
+  pr.lane_idx = lane_idx;
+  pr.norm_stats = norm_stats;
+  pr.local_stats = local_stats;
+  pr.g_logp = pr.g_entropy = nullptr;
+  pr.g_value = g_value;
+  pr.out = out;
+  pr.out_f32 = out_f32;
+  pr.slot = reinterpret_cast<SlotHeader*>(workspace);
+  return masked ? launch_logits<true>(q, cache_e, smem, stream) : launch_logits<false>(q, cache_e, smem, stream);
+}
 
 }  // namespace
 
@@ -510,89 +655,26 @@ extern "C" int srl_ppo_loss_from_logits(const float* logits, const int32_t* acti
                                         float* g_value, float* logp_out, float* entropy_out, double* out,
                                         float* out_f32, void* workspace, size_t workspace_bytes,
                                         srl_stream_t stream) {
-  using namespace srl;
-  using namespace srl::loss;
-  SRL_REQUIRE(T >= 1 && n >= 1, SRL_ERR_INVALID_ARG, "srl_ppo_loss_from_logits: need T >= 1 and n >= 1");
-  SRL_REQUIRE(heads >= 1 && heads <= SRL_MAX_HEADS && head_sizes_host, SRL_ERR_INVALID_ARG,
-              "srl_ppo_loss_from_logits: heads=%d outside [1, %d]", heads, SRL_MAX_HEADS);
-  SRL_REQUIRE(logits && action && v_pred && old_logp && ret && adv && on_reset_next && g_logits && g_value &&
-                  norm_stats && local_stats && workspace,
-              SRL_ERR_INVALID_ARG, "srl_ppo_loss_from_logits: null pointer");
-  SRL_REQUIRE(ld_smp >= (lane_idx ? 1 : n), SRL_ERR_INVALID_ARG, "srl_ppo_loss_from_logits: ld_smp smaller than the row");
-  SRL_REQUIRE(workspace_bytes >= srl_ppo_loss_workspace_bytes(T, n), SRL_ERR_INVALID_ARG,
-              "srl_ppo_loss_from_logits: workspace too small (%zu bytes)", workspace_bytes);
-  LogitsParams q;
-  int rc = fill_loss_hyper(hyper, popart_mean_std, q.s.h);
-  if (rc != SRL_OK) return rc;
-  SRL_REQUIRE(!(q.s.h.clip_value && old_value == nullptr), SRL_ERR_INVALID_ARG,
-              "srl_ppo_loss_from_logits: clip_value needs old_value");
-  int sk = 0;
-  for (int i = 0; i < SRL_MAX_HEADS; ++i) {
-    q.head_size[i] = i < heads ? head_sizes_host[i] : 0;
-    SRL_REQUIRE(i >= heads || head_sizes_host[i] >= 1, SRL_ERR_INVALID_ARG,
-                "srl_ppo_loss_from_logits: head %d has no actions", i);
-    sk += q.head_size[i];
-  }
-  const size_t row_bytes = static_cast<size_t>(256) * sk * sizeof(float);  // dense [256, sum K] block
-  SRL_REQUIRE(row_bytes + 16 <= 200 * 1024, SRL_ERR_UNSUPPORTED, "srl_ppo_loss_from_logits: sum K = %d too wide (max 199)", sk);
-  const bool cache_e = 2 * row_bytes + 16 <= 200 * 1024;  // both blocks fit: one exponential per logit
-  const size_t smem = (cache_e ? 2 * row_bytes : row_bytes) + 16;  // + the mbarrier of the bulk copies
-  q.heads = heads;
-  q.SK = sk;
-  q.logits = logits;
-  q.action = action;
-  q.g_logits = g_logits;
-  q.logp_out = logp_out;
-  q.entropy_out = entropy_out;
-  LossShared& p = q.s;
-  p.old_logp = old_logp;
-  p.old_value = old_value;
-  p.ret = ret;
-  p.adv = adv;
-  p.reset_next = on_reset_next;
-  p.pack = nullptr;
-  p.lane_aos = nullptr;
-  p.part = nullptr;
-  p.part_ctas = p.part_first = 0;
-  p.row_lo = 0;
-  p.popart = popart_mean_std;
-  p.ld_pol = n;
-  p.ld_grad = n;
-  p.ld_smp = ld_smp;
-  p.T = T;
-  p.n = n;
-  p.rows_per_tile = p.col_tiles = p.n_tiles = 0;
-  p.smp_vec_ok = 0;
-  Problem& pr = q.pr;
-  pr.new_logp = pr.entropy = nullptr;
-  pr.v_pred = v_pred;
-  pr.lane_idx = lane_idx;
-  pr.norm_stats = norm_stats;
-  pr.local_stats = local_stats;
-  pr.g_logp = pr.g_entropy = nullptr;
-  pr.g_value = g_value;
-  pr.out = out;
-  pr.out_f32 = out_f32;
-  pr.slot = reinterpret_cast<SlotHeader*>(workspace);
-  if ((rc = opt_in_smem<ppo_loss_logits_kernel<true>>(200 * 1024)) != SRL_OK) return rc;
-  if ((rc = opt_in_smem<ppo_loss_logits_kernel<false>>(200 * 1024)) != SRL_OK) return rc;
-  const long long tiles = (static_cast<long long>(T) * n + 255) / 256;
-  // one wave: as many CTAs as are resident with this much shared memory (2048 tiles on 1184 assumed slots were 1024 CTAs on
-  // the 740 real ones -- a second, partial wave)
-  int per_sm = 0;
-  if ((cache_e ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<true>, 256, smem)
-               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<false>, 256, smem)) != cudaSuccess ||
-      per_sm < 1)
-    per_sm = 1;
-  const long long slots = static_cast<long long>(sm_count()) * per_sm;
-  const long long cap = slots < kMaxGrid ? slots : kMaxGrid;
-  // every CTA the same number of tiles (2048 tiles on 1184 slots would leave most CTAs one tile and the rest two)
-  const long long per_cta = (tiles + cap - 1) / cap;
-  const int grid = static_cast<int>((tiles + per_cta - 1) / per_cta);
-  if (cache_e)
-    ppo_loss_logits_kernel<true><<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(q);
-  else
-    ppo_loss_logits_kernel<false><<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(q);
-  SRL_CUDA(cudaGetLastError());
-  return SRL_OK;
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits", logits, nullptr, action, head_sizes_host, heads, v_pred,
+                                         old_logp, old_value, ret, adv, on_reset_next, ld_smp, lane_idx, T, n, norm_stats,
+                                         local_stats, popart_mean_std, hyper, g_logits, g_value, logp_out, entropy_out, out,
+                                         out_f32, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int srl_ppo_loss_from_logits_masked(const float* logits, const uint8_t* available, const int32_t* action,
+                                               const int32_t* head_sizes_host, int heads, const float* v_pred,
+                                               const float* old_logp, const float* old_value, const float* ret,
+                                               const float* adv, const uint8_t* on_reset_next, int64_t ld_smp,
+                                               const int32_t* lane_idx, int T, int n, const double* norm_stats,
+                                               const double* local_stats, const double* popart_mean_std,
+                                               const srl_ppo_hyper* hyper, float* g_logits, float* g_value,
+                                               float* logp_out, float* entropy_out, double* out, float* out_f32,
+                                               void* workspace, size_t workspace_bytes, srl_stream_t stream) {
+  SRL_REQUIRE(available != nullptr, SRL_ERR_INVALID_ARG,
+              "srl_ppo_loss_from_logits_masked: null pointer available (use srl_ppo_loss_from_logits without a mask)");
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked", logits, available, action, head_sizes_host, heads,
+                                         v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp, lane_idx, T, n,
+                                         norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value, logp_out,
+                                         entropy_out, out, out_f32, workspace, workspace_bytes,
+                                         static_cast<cudaStream_t>(stream));
 }

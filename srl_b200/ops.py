@@ -587,11 +587,38 @@ def ppo_loss_batched(problems: Sequence[dict], old_logp, old_value, ret, adv, on
               _ptr(popart_mean_std), ctypes.byref(hc), slot_bytes, None if exchange is None else exchange._h, _stream())
 
 
+def _availability(available, logits) -> torch.Tensor:
+    """The availability mask as the kernel reads it: one byte per logit, non-zero = available."""
+    if not isinstance(available, torch.Tensor):
+        raise ValueError(f"available: expected a tensor, got {type(available).__name__}")
+    if tuple(available.shape) != tuple(logits.shape):
+        raise ValueError(f"available: shape {tuple(available.shape)} does not match logits {tuple(logits.shape)}")
+    if any(st == 0 and sz > 1 for st, sz in zip(available.stride(), available.shape)):
+        raise ValueError(f"available: a stride-0 expand (strides {available.stride()}); the mask is read per logit, pass "
+                         f"a dense [T, n, sum K] tensor")
+    if not available.is_contiguous():
+        raise ValueError(f"available: expected a contiguous tensor, got strides {available.stride()}")
+    if available.dtype.is_floating_point:
+        available = available != 0  # the reference's `available_action == 0` test, negated
+    elif available.dtype not in (torch.uint8, torch.bool):
+        raise ValueError(f"available: expected dtype torch.uint8, torch.bool or a floating dtype, got {available.dtype}")
+    if not available.is_cuda or available.device != logits.device:
+        raise ValueError(f"available: expected a CUDA tensor on {logits.device}, got one on {available.device}")
+    return available
+
+
 def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_logp, old_value, ret, adv, on_reset_next,
                          norm_stats, hyper: LossHyper, local_stats=None, popart_mean_std=None, lane_idx=None,
-                         want_logp_entropy: bool = False):
+                         want_logp_entropy: bool = False, available=None, workspace=None, defer: bool = False):
     """Loss starting from the actor head's logits `[T, n, sum K]` and int32 actions `[T, n, heads]`
-    (actor_critic_policy.py:303-324 fused in).  Returns (g_logits, g_value, out, out_f32, logp, entropy)."""
+    (actor_critic_policy.py:303-324 fused in).  Returns (g_logits, g_value, out, out_f32, logp, entropy).
+
+    `available` (SMAC's available_action, the logits' shape): where it is 0 the logit is replaced by -1e10 before the
+    Categorical (actor_critic_policy.py:135-136) and its gradient is 0.  torch.uint8 and torch.bool are read in place; a
+    floating mask costs one extra pass (`available != 0`).  At most 159 logits per transition with a mask, 199 without.
+    `defer` (needs an explicit `workspace` slot): out / out_f32 are None and loss_finalize folds the slot later."""
+    if available is not None:
+        available = _availability(available, logits)
     _check(logits, torch.float32, "logits")
     _check(action, torch.int32, "action")
     _check(v_pred, torch.float32, "v_pred")
@@ -614,15 +641,23 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     g_value = torch.empty_like(v_pred)
     logp = torch.empty_like(v_pred) if want_logp_entropy else None
     ent = torch.empty_like(v_pred) if want_logp_entropy else None
-    out = torch.empty(SRL_LOSS_OUT_LEN, dtype=torch.float64, device=dev)
-    out_f32 = torch.empty(4, dtype=torch.float32, device=dev)
-    ws = loss_workspace(dev)
+    if defer:
+        if workspace is None:
+            raise ValueError("deferred finalisation needs an explicit workspace slot")
+        out = out_f32 = None
+    else:
+        out = torch.empty(SRL_LOSS_OUT_LEN, dtype=torch.float64, device=dev)
+        out_f32 = torch.empty(4, dtype=torch.float32, device=dev)
+    ws = loss_workspace(dev) if workspace is None else _check(workspace, torch.uint8, "workspace")
     hc = hyper.to_c()
     hs = (ctypes.c_int32 * heads)(*[int(k) for k in head_sizes])
-    _lib.call("srl_ppo_loss_from_logits", _ptr(logits), _ptr(action), hs, heads, _ptr(v_pred), _ptr(old_logp),
-              _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp, _ptr(lane_idx), T, n,
-              _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc), _ptr(g_logits),
-              _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws), ws.numel(), _stream())
+    tail = (hs, heads, _ptr(v_pred), _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp,
+            _ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
+            _ptr(g_logits), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws), ws.numel(), _stream())
+    if available is None:
+        _lib.call("srl_ppo_loss_from_logits", _ptr(logits), _ptr(action), *tail)
+    else:
+        _lib.call("srl_ppo_loss_from_logits_masked", _ptr(logits), _ptr(available), _ptr(action), *tail)
     return g_logits, g_value, out, out_f32, logp, ent
 
 
@@ -736,6 +771,33 @@ class PPOGaussianLossFunction(torch.autograd.Function):
     def backward(ctx, grad_loss, _grad_out):
         g_mean, g_ls, g_v = ctx.saved_tensors
         return (g_mean * grad_loss, g_ls * grad_loss, None, g_v * grad_loss) + (None,) * 10
+
+
+class PPOCategoricalLossFunction(torch.autograd.Function):
+    """Autograd node for a categorical policy (K4b): forward returns the scalar loss (float32) and the float64 stats
+    vector of ppo_loss_from_logits; backward hands the gradients the same launch produced to the logits (exactly 0 where
+    `available` is 0) and v_pred.  `available` is the availability mask or None.
+
+        loss, out = PPOCategoricalLossFunction.apply(logits, available, action, head_sizes, v_pred, old_logp, old_value,
+                                                     ret, adv, on_reset_next, norm_stats, local_stats, popart_mean_std,
+                                                     lane_idx, hyper)
+        loss.backward()
+    """
+
+    @staticmethod
+    def forward(ctx, logits, available, action, head_sizes, v_pred, old_logp, old_value, ret, adv, on_reset_next,
+                norm_stats, local_stats, popart_mean_std, lane_idx, hyper):
+        g_logits, g_v, out, out_f32, _, _ = ppo_loss_from_logits(
+            logits.detach(), action, head_sizes, v_pred.detach(), old_logp, old_value, ret, adv, on_reset_next, norm_stats,
+            hyper, local_stats=local_stats, popart_mean_std=popart_mean_std, lane_idx=lane_idx, available=available)
+        ctx.save_for_backward(g_logits, g_v)
+        ctx.mark_non_differentiable(out)
+        return out_f32[0], out
+
+    @staticmethod
+    def backward(ctx, grad_loss, _grad_out):
+        g_logits, g_v = ctx.saved_tensors
+        return (g_logits * grad_loss, None, None, None, g_v * grad_loss) + (None,) * 10
 
 
 class PPOLossFunction(torch.autograd.Function):

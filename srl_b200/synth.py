@@ -121,8 +121,8 @@ def make_policy_outputs(cfg: PathConfig, sample: Dict[str, np.ndarray], seed: in
 
 
 def make_logits_actions(cfg: PathConfig, lead_shape, seed: int = 2):
-    """For the from-logits loss variant: logits ~ N(0,1) `[*lead, sum K]` float32, actions `[*lead, heads]`
-    int32 sampled from them, optional availability mask (SMAC) with action 0 always available."""
+    """For the from-logits loss variant: logits ~ N(0,1) `[*lead, sum K]` float32 and actions `[*lead, heads]`
+    int32 sampled from them (make_masked_logits_actions adds an availability mask)."""
     rng = np.random.Generator(np.random.PCG64(seed + 104729))
     K = int(sum(cfg.num_actions))
     logits = rng.standard_normal(tuple(lead_shape) + (K,), dtype=np.float32)
@@ -136,6 +136,32 @@ def make_logits_actions(cfg: PathConfig, lead_shape, seed: int = 2):
         actions[..., h] = np.minimum((p.cumsum(-1) < u).sum(-1), k - 1)
         off += k
     return logits, actions
+
+
+def make_masked_logits_actions(cfg: PathConfig, lead_shape, seed: int = 2, p_unavailable: float = 0.3):
+    """For the from-logits loss with SMAC's availability mask: logits ~ N(0,1) `[*lead, sum K]` float32, `available`
+    `[*lead, sum K]` uint8 (each action unavailable with probability p_unavailable, action 0 of every head always
+    available, as SMAC's no-op is) and actions `[*lead, heads]` int32 sampled from the masked distribution.
+    Returns (logits, actions, available)."""
+    rng = np.random.Generator(np.random.PCG64(seed + 1299709))
+    lead = tuple(lead_shape)
+    K = int(sum(cfg.num_actions))
+    logits = rng.standard_normal(lead + (K,), dtype=np.float32)
+    available = (rng.random(lead + (K,)) >= p_unavailable).astype(np.uint8)
+    actions = np.zeros(lead + (len(cfg.num_actions),), dtype=np.int32)
+    off = 0
+    for h, k in enumerate(cfg.num_actions):
+        available[..., off] = 1
+        z = logits[..., off:off + k].astype(np.float64)
+        p = np.exp(z - z.max(-1, keepdims=True)) * available[..., off:off + k]
+        p /= p.sum(-1, keepdims=True)
+        u = rng.random(lead + (1,))
+        a = np.minimum((p.cumsum(-1) < u).sum(-1), k - 1)
+        # the float64 cumsum can end a hair below u: take the last available action instead of an unavailable one
+        last = k - 1 - np.argmax(available[..., off:off + k][..., ::-1], axis=-1)
+        actions[..., h] = np.minimum(a, last)
+        off += k
+    return logits, actions, available
 
 
 def make_obs(cfg: PathConfig, L: int, B: int, seed: int = 3) -> np.ndarray:
