@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SRL_B200_ABI_VERSION 11
+#define SRL_B200_ABI_VERSION 12
 
 typedef void* srl_stream_t; /* cudaStream_t */
 
@@ -249,7 +249,7 @@ enum srl_loss_out {
  * before the slot is used again.  Launches that may overlap in time need distinct slots. */
 size_t srl_ppo_loss_workspace_bytes(int T, int n);
 
-/* Deferred finalisation: when srl_ppo_loss_fwd_bwd / srl_ppo_loss_from_logits(_masked) are called with out == NULL they
+/* Deferred finalisation: when srl_ppo_loss_fwd_bwd / srl_ppo_loss_from_logits(_masked)(_bf16) are called with out == NULL they
  * stop after writing gradients and partial rows.  This folds n_slots consecutive slots (slot k at
  * workspace + k * slot_bytes) into out[k][SRL_LOSS_OUT_LEN] (and out_f32[k][4] if not NULL) in one launch, and
  * clears the rows it folded. */
@@ -359,6 +359,40 @@ int srl_ppo_loss_from_logits_masked(
     const srl_ppo_hyper* hyper, float* g_logits, /* [T, n, sumK] out */
     float* g_value,                               /* [T, n] out */
     float* logp_out, float* entropy_out,          /* [T, n] out or NULL */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+
+/* The two entries above with a bfloat16 policy side, for policies trained under torch.autocast(dtype=torch.bfloat16), whose
+ * last nn.Linear layers produce bfloat16 logits and values.  Same arguments in the same order; logits, v_pred, g_logits and
+ * g_value are bfloat16 bit patterns (uint16_t, the upper half of the float32 pattern), everything else is as above:
+ * logp_out / entropy_out, the sample side and the ten outputs stay float32.  Each logit and v_pred is widened to float32
+ * exactly where it is read and all arithmetic is float32, as torch runs logsumexp / log_softmax / softmax on upcast bfloat16
+ * values; each g_logits and g_value entry is the float32 result rounded to bfloat16 once (round to nearest even).  So the
+ * results are the float32 entry's on the widened values, with the gradients rounded, wherever the two make the same
+ * choice of caching exponentials (sum K <= 99 without a mask and <= 88 with one; the bfloat16 entries cache them up to 133
+ * and 114).  The widest rows are the float32 entries' limits, SRL_K4B_MAX_SUM_K and SRL_K4B_MAX_SUM_K_MASKED; wider rows
+ * are SRL_ERR_UNSUPPORTED.  The masked entry rejects a NULL mask.  Deferred finalisation works as above. */
+int srl_ppo_loss_from_logits_bf16(
+    const uint16_t* logits, /* [T, n, sumK] dense bfloat16 */
+    const int32_t* action,  /* [T, n, heads]               */
+    const int32_t* head_sizes_host, int heads, const uint16_t* v_pred, /* [T, n] dense bfloat16 */
+    const float* old_logp, const float* old_value, const float* ret, const float* adv,
+    const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper, uint16_t* g_logits, /* [T, n, sumK] bfloat16 out */
+    uint16_t* g_value,                               /* [T, n] bfloat16 out */
+    float* logp_out, float* entropy_out,             /* [T, n] float32 out or NULL */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+int srl_ppo_loss_from_logits_masked_bf16(
+    const uint16_t* logits,   /* [T, n, sumK] dense bfloat16 */
+    const uint8_t* available, /* [T, n, sumK] dense, non-zero = available */
+    const int32_t* action,    /* [T, n, heads]               */
+    const int32_t* head_sizes_host, int heads, const uint16_t* v_pred, /* [T, n] dense bfloat16 */
+    const float* old_logp, const float* old_value, const float* ret, const float* adv,
+    const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper, uint16_t* g_logits, /* [T, n, sumK] bfloat16 out */
+    uint16_t* g_value,                               /* [T, n] bfloat16 out */
+    float* logp_out, float* entropy_out,             /* [T, n] float32 out or NULL */
     double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------

@@ -22,7 +22,7 @@ SRL_MAX_HEADS = 8
 SRL_K4B_MAX_SUM_K = 199
 SRL_K4B_MAX_SUM_K_MASKED = 159
 SRL_MAX_LOSS_BATCH = 32
-ABI_VERSION = 11
+ABI_VERSION = 12
 
 # enum srl_loss_out
 OUT_LOSS, OUT_POLICY_LOSS, OUT_VALUE_LOSS, OUT_ENTROPY_LOSS = 0, 1, 2, 3
@@ -113,6 +113,17 @@ SIGNATURES = {
                                                 c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
                                                 c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                                 c_size_t, c_void_p]),
+    # the _bf16 twins take the same arguments (logits, v_pred, g_logits, g_value: bfloat16 device pointers)
+    "srl_ppo_loss_from_logits_bf16": (c_int, [c_void_p, c_void_p, POINTER(c_int32), c_int, c_void_p,
+                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                              c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                              c_size_t, c_void_p]),
+    "srl_ppo_loss_from_logits_masked_bf16": (c_int, [c_void_p, c_void_p, c_void_p, POINTER(c_int32), c_int, c_void_p,
+                                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                                     c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                     c_size_t, c_void_p]),
     "srl_ppo_loss_gaussian_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
     "srl_ppo_loss_from_gaussian": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,

@@ -1,5 +1,6 @@
 // Shared helpers for the srl_b200 kernels (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -64,10 +65,12 @@ __device__ __forceinline__ float4 ldg_stream(const float4* p) { return __ldcs(p)
 __device__ __forceinline__ uint32_t ldg_stream(const uint32_t* p) { return __ldcs(p); }
 __device__ __forceinline__ uint8_t ldg_stream(const uint8_t* p) { return __ldcs(p); }
 __device__ __forceinline__ int4 ldg_stream(const int4* p) { return __ldcs(p); }
+__device__ __forceinline__ __nv_bfloat16 ldg_stream(const __nv_bfloat16* p) { return __ldcs(p); }
 __device__ __forceinline__ void stg_stream(float* p, float v) { __stcs(p, v); }
 __device__ __forceinline__ void stg_stream(float2* p, float2 v) { __stcs(p, v); }
 __device__ __forceinline__ void stg_stream(float4* p, float4 v) { __stcs(p, v); }
 __device__ __forceinline__ void stg_stream(int4* p, int4 v) { __stcs(p, v); }
+__device__ __forceinline__ void stg_stream(__nv_bfloat16* p, __nv_bfloat16 v) { __stcs(p, v); }
 
 // griddepcontrol.wait returns once every prerequisite grid has COMPLETED and its memory is visible (immediately when the
 // kernel was launched without the programmatic attribute).

@@ -52,12 +52,14 @@ __global__ void __launch_bounds__(256) loss_finalize_kernel(unsigned char* __res
 // A CTA takes 256 consecutive transitions; their [256, sumK] logits block is contiguous in memory, so
 // it is staged through shared memory with coalesced loads (row stride sumK+1 words: conflict-free
 // per-thread row walks), turned into d loss / d logits in place, and streamed back out coalesced.
+// The policy side (logits, v_pred, g_logits, g_value) is float or bfloat16, the kernel's element type T; pr.v_pred and
+// pr.g_value point at T as well (Problem is K4's struct, typed float).  Everything else, the arithmetic included, is float.
 struct LogitsParams {
   LossShared s;
   Problem pr;             // new_logp / entropy / g_logp / g_entropy are unused here
-  const float* logits;    // [T*n, SK]
+  const void* logits;     // [T*n, SK] of T
   const int32_t* action;  // [T*n, heads]
-  float* g_logits;        // [T*n, SK]
+  void* g_logits;         // [T*n, SK] of T
   float* logp_out;        // [T*n] or null
   float* entropy_out;     // [T*n] or null
   int heads, SK;
@@ -83,17 +85,28 @@ constexpr int kStage = 9;  // manual staging batch per thread (last, partial til
 // actor_critic_policy.py:135-136: logits.masked_fill(available_action == 0, -1e10) before the Categorical
 constexpr float kUnavailableLogit = -1e10f;
 
+// A policy-side element as the arithmetic reads it (bfloat16 -> float is exact), and a result stored back in the element
+// type (bfloat16: rounded to nearest even, once, where the float result is final).
+__device__ __forceinline__ float to_float(float x) { return x; }
+__device__ __forceinline__ float to_float(__nv_bfloat16 x) { return __bfloat162float(x); }
+template <typename T>
+__device__ __forceinline__ T from_float(float x);
+template <>
+__device__ __forceinline__ float from_float<float>(float x) { return x; }
+template <>
+__device__ __forceinline__ __nv_bfloat16 from_float<__nv_bfloat16>(float x) { return __float2bfloat16_rn(x); }
+
 // logit k of a row as the Categorical sees it
-template <bool MASKED>
-__device__ __forceinline__ float logit_at(const float* z, const uint8_t* m, int k) {
-  return (MASKED && m[k] == 0) ? kUnavailableLogit : z[k];
+template <bool MASKED, typename T>
+__device__ __forceinline__ float logit_at(const T* z, const uint8_t* m, int k) {
+  return (MASKED && m[k] == 0) ? kUnavailableLogit : to_float(z[k]);
 }
 
 // forward passes of one head held in registers: log-sum-exp, 1 / sum, entropy; e_k to `ez` when CACHE_E.  With MASKED,
 // `m` is the head's availability bytes and an unavailable logit reads as kUnavailableLogit (its e_k is 0 unless the whole
 // head is unavailable: then every lp_k is 0, as in torch, and the head adds nothing to logp or the entropy)
-template <int KM, bool CACHE_E, bool MASKED>
-__device__ __forceinline__ void head_forward(const float* z, float* ez, const uint8_t* m, int K, float& l, float& inv,
+template <int KM, bool CACHE_E, bool MASKED, typename T>
+__device__ __forceinline__ void head_forward(const T* z, float* ez, const uint8_t* m, int K, float& l, float& inv,
                                              float& hh) {
   float v[KM];
 #pragma unroll
@@ -124,13 +137,13 @@ __device__ __forceinline__ void head_forward(const float* z, float* ez, const ui
 
 // gradient pass of one head: z_k <- d loss / d z_k; with MASKED an unavailable logit gets exactly 0 (masked_fill passes
 // no gradient), also when it is the chosen action, where the expression below is not 0
-template <int KM, bool CACHE_E, bool MASKED>
-__device__ __forceinline__ void head_backward(float* z, const float* ez, const uint8_t* m, int K, int a, float l, float inv,
+template <int KM, bool CACHE_E, bool MASKED, typename T>
+__device__ __forceinline__ void head_backward(T* z, const float* ez, const uint8_t* m, int K, int a, float l, float inv,
                                               float hh, float g_lp, float g_en) {
   float v[KM], e[KM];
 #pragma unroll
   for (int k = 0; k < KM; ++k) {
-    v[k] = k < K ? z[k] : 0.f;
+    v[k] = k < K ? to_float(z[k]) : 0.f;
     e[k] = (CACHE_E && k < K) ? ez[k] : 0.f;
   }
 #pragma unroll
@@ -140,7 +153,7 @@ __device__ __forceinline__ void head_backward(float* z, const float* ez, const u
       const float pk = CACHE_E ? e[k] * inv : expf(lp);
       // d logp / d z_k = [k == a] - p_k ;  d H / d z_k = -p_k (lp_k + H)
       const float g = g_lp * ((k == a ? 1.f : 0.f) - pk) - g_en * pk * (fmaxf(lp, -FLT_MAX) + hh);
-      z[k] = (MASKED && m[k] == 0) ? 0.f : g;
+      z[k] = from_float<T>((MASKED && m[k] == 0) ? 0.f : g);
     }
   }
 }
@@ -159,10 +172,12 @@ __device__ __forceinline__ void head_backward(float* z, const float* ez, const u
 
 // MASKED: the [256, SK] availability bytes of the tile follow the float blocks in shared memory, brought in with the logits
 // (same mbarrier and expect_tx, or the same element-wise staging); every pass over a head reads them.
-template <bool CACHE_E, bool MASKED>
+// T: the policy side's element type (float or __nv_bfloat16); the staged block holds T, the cached exponentials float.
+template <bool CACHE_E, bool MASKED, typename T>
 __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kernel(const __grid_constant__ LogitsParams q) {
-  // [256 * SK] dense (+ [256 * SK] with CACHE_E), (+ [256 * SK] bytes with MASKED), then the mbarrier
-  extern __shared__ __align__(128) float srow[];
+  // [256 * SK] of T, dense (+ [256 * SK] floats with CACHE_E), (+ [256 * SK] bytes with MASKED), then the mbarrier
+  extern __shared__ __align__(128) float smem[];
+  constexpr int kElem = sizeof(T);
   const LossShared& p = q.s;
   const Problem& pr = q.pr;
   const LossHyperDev& h = p.h;
@@ -170,8 +185,11 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
   const Uniforms u = load_uniforms(pr.norm_stats, pr.local_stats, p.popart, h.adv_eps, mask_sum);
   Acc acc;
   const int SK = q.SK;
-  float* erow = srow + 256 * SK;
-  uint8_t* mrow = reinterpret_cast<uint8_t*>(srow + (CACHE_E ? 2 : 1) * 256 * SK);
+  // offsets in floats: the staged block is 256 * SK * kElem bytes = 64 * kElem * SK floats (a multiple of 16 bytes), the
+  // exponentials 256 * SK floats
+  T* srow = reinterpret_cast<T*>(smem);
+  float* erow = smem + 64 * kElem * SK;
+  uint8_t* mrow = reinterpret_cast<uint8_t*>(smem + (CACHE_E ? 64 * kElem + 256 : 64 * kElem) * SK);
   uint64_t* bar = reinterpret_cast<uint64_t*>(mrow + (MASKED ? 256 * SK : 0));  // 256 * SK bytes keep it 8-byte aligned
   if (threadIdx.x == 0) {
     tma::mbar_init(bar, 1);
@@ -187,23 +205,24 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
     const long long i0 = tile * 256;
     const int cnt = static_cast<int>(min(256ll, W - i0));
     const int total = cnt * SK;
-    const float* src = q.logits + i0 * SK;
-    float* dst = q.g_logits + i0 * SK;
-    // 256 * SK * 4 bytes of logits and 256 * SK bytes of mask: multiples of 16 at 16-byte aligned addresses
+    const T* src = static_cast<const T*>(q.logits) + i0 * SK;
+    T* dst = static_cast<T*>(q.g_logits) + i0 * SK;
+    // 256 * SK * kElem bytes of logits and 256 * SK bytes of mask: multiples of 16 at 16-byte aligned addresses
     const bool bulk = bulk_ok && cnt == 256;
     const uint8_t* msrc = MASKED ? q.available + i0 * SK : nullptr;
     if (bulk) {
       if (threadIdx.x == 0) {
-        const uint32_t bytes = static_cast<uint32_t>(total) * 4u;
+        const uint32_t bytes = static_cast<uint32_t>(total) * kElem;
         tma::mbar_expect_tx(bar, MASKED ? bytes + static_cast<uint32_t>(total) : bytes);
         tma::bulk_load(srow, src, bytes, bar);
         if (MASKED) tma::bulk_load(mrow, msrc, static_cast<uint32_t>(total), bar);
       }
     } else {
       for (int e0 = threadIdx.x; e0 < total; e0 += 256 * kStage) {
-        float v[kStage];
+        T v[kStage];
 #pragma unroll
-        for (int b = 0; b < kStage; ++b) v[b] = (e0 + b * 256 < total) ? ldg_stream(src + e0 + b * 256) : 0.f;
+        for (int b = 0; b < kStage; ++b)
+          v[b] = (e0 + b * 256 < total) ? ldg_stream(src + e0 + b * 256) : from_float<T>(0.f);
 #pragma unroll
         for (int b = 0; b < kStage; ++b)
           if (e0 + b * 256 < total) srow[e0 + b * 256] = v[b];
@@ -230,7 +249,7 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
       const int j = static_cast<int>(i - static_cast<long long>(t) * p.n);
       const int c = pr.lane_idx ? pr.lane_idx[j] : j;
       const long long os = t * p.ld_smp + c;
-      vp = ldg_stream(pr.v_pred + i);
+      vp = to_float(ldg_stream(reinterpret_cast<const T*>(pr.v_pred) + i));
       ol = __ldg(p.old_logp + os), rt = __ldg(p.ret + os), ad = __ldg(p.adv + os);
       ov = h.clip_value ? __ldg(p.old_value + os) : 0.f;
       valid = __ldg(p.reset_next + os) == 0;
@@ -244,7 +263,7 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
       __syncthreads();
     }
     if (mine) {
-      float* z = srow + threadIdx.x * SK;
+      T* z = srow + threadIdx.x * SK;
       float* ez = erow + threadIdx.x * SK;
       const uint8_t* m = mrow + threadIdx.x * SK;
       // (the head loops are NOT unrolled: with the dispatch over eight widths inlined in each of SRL_MAX_HEADS slots the kernel
@@ -290,7 +309,7 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
       RowSums rs;
       element<RuntimeCfg>(h, u, logp, vp, ent, ol, ov, rt, ad, valid, g_lp, g_v, g_en, rs);
       acc.add(rs);
-      stg_stream(pr.g_value + i, g_v);
+      stg_stream(reinterpret_cast<T*>(pr.g_value) + i, from_float<T>(g_v));
       if (q.logp_out) q.logp_out[i] = logp;
       if (q.entropy_out) q.entropy_out[i] = ent;
       off = 0;
@@ -303,10 +322,10 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
                               g_en);
           } else {
             for (int k = 0; k < K; ++k) {
-              const float lp = z[off + k] - lse[hd];
+              const float lp = to_float(z[off + k]) - lse[hd];
               const float pk = CACHE_E ? ez[off + k] * rse[hd] : expf(lp);
               const float g = g_lp * ((k == act[hd] ? 1.f : 0.f) - pk) - g_en * pk * (fmaxf(lp, -FLT_MAX) + hent[hd]);
-              z[off + k] = (MASKED && m[off + k] == 0) ? 0.f : g;
+              z[off + k] = from_float<T>((MASKED && m[off + k] == 0) ? 0.f : g);
             }
           }
           off += K;
@@ -316,14 +335,14 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
     if (bulk) {
       tma::fence_proxy_async_smem();  // the gradients above, before the bulk copy reads them
       __syncthreads();
-      if (threadIdx.x == 0) tma::bulk_store(dst, srow, static_cast<uint32_t>(total) * 4u);  // read before the next tile
+      if (threadIdx.x == 0) tma::bulk_store(dst, srow, static_cast<uint32_t>(total) * kElem);  // read before the next tile
       __syncthreads();
     } else {
       __syncthreads();
       for (int e0 = threadIdx.x; e0 < total; e0 += 256 * kStage) {
-        float v[kStage];
+        T v[kStage];
 #pragma unroll
-        for (int b = 0; b < kStage; ++b) v[b] = (e0 + b * 256 < total) ? srow[e0 + b * 256] : 0.f;
+        for (int b = 0; b < kStage; ++b) v[b] = (e0 + b * 256 < total) ? srow[e0 + b * 256] : from_float<T>(0.f);
 #pragma unroll
         for (int b = 0; b < kStage; ++b)
           if (e0 + b * 256 < total) stg_stream(dst + e0 + b * 256, v[b]);
@@ -335,23 +354,25 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
 }
 #undef SRL_HEAD_DISPATCH
 
-// the largest sum K whose staged block(s) fit the 200 KiB opt-in below (include/srl_b200.h states both limits)
+// The widest rows, the same for both element types: the largest sum K whose float32 block (and mask bytes) fit the 200 KiB
+// opt-in below (include/srl_b200.h states both limits).  A bfloat16 block is half as wide, so it fits there as well.
 static_assert(256 * SRL_K4B_MAX_SUM_K * 4 + 16 <= 200 * 1024 && 256 * (SRL_K4B_MAX_SUM_K + 1) * 4 + 16 > 200 * 1024, "");
 static_assert(256 * SRL_K4B_MAX_SUM_K_MASKED * 5 + 16 <= 200 * 1024 && 256 * (SRL_K4B_MAX_SUM_K_MASKED + 1) * 5 + 16 > 200 * 1024,
               "");
+static_assert(256 * SRL_K4B_MAX_SUM_K * 2 + 16 <= 200 * 1024 && 256 * SRL_K4B_MAX_SUM_K_MASKED * 3 + 16 <= 200 * 1024, "");
 
-// one resident wave of ppo_loss_logits_kernel<CACHE_E, MASKED> over the T * n transitions of q
-template <bool MASKED>
+// one resident wave of ppo_loss_logits_kernel<CACHE_E, MASKED, T> over the T * n transitions of q
+template <bool MASKED, typename T>
 int launch_logits(const LogitsParams& q, bool cache_e, size_t smem, cudaStream_t stream) {
   int rc;
-  if ((rc = opt_in_smem<ppo_loss_logits_kernel<true, MASKED>>(200 * 1024)) != SRL_OK) return rc;
-  if ((rc = opt_in_smem<ppo_loss_logits_kernel<false, MASKED>>(200 * 1024)) != SRL_OK) return rc;
+  if ((rc = opt_in_smem<ppo_loss_logits_kernel<true, MASKED, T>>(200 * 1024)) != SRL_OK) return rc;
+  if ((rc = opt_in_smem<ppo_loss_logits_kernel<false, MASKED, T>>(200 * 1024)) != SRL_OK) return rc;
   const long long tiles = (static_cast<long long>(q.s.T) * q.s.n + 255) / 256;
   // one wave: as many CTAs as are resident with this much shared memory (2048 tiles on 1184 assumed slots were 1024 CTAs on
   // the 740 real ones -- a second, partial wave)
   int per_sm = 0;
-  if ((cache_e ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<true, MASKED>, 256, smem)
-               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<false, MASKED>, 256, smem)) !=
+  if ((cache_e ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<true, MASKED, T>, 256, smem)
+               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<false, MASKED, T>, 256, smem)) !=
           cudaSuccess ||
       per_sm < 1)
     per_sm = 1;
@@ -361,21 +382,22 @@ int launch_logits(const LogitsParams& q, bool cache_e, size_t smem, cudaStream_t
   const long long per_cta = (tiles + cap - 1) / cap;
   const int grid = static_cast<int>((tiles + per_cta - 1) / per_cta);
   if (cache_e)
-    ppo_loss_logits_kernel<true, MASKED><<<grid, 256, smem, stream>>>(q);
+    ppo_loss_logits_kernel<true, MASKED, T><<<grid, 256, smem, stream>>>(q);
   else
-    ppo_loss_logits_kernel<false, MASKED><<<grid, 256, smem, stream>>>(q);
+    ppo_loss_logits_kernel<false, MASKED, T><<<grid, 256, smem, stream>>>(q);
   SRL_CUDA(cudaGetLastError());
   return SRL_OK;
 }
 
-// srl_ppo_loss_from_logits (available == NULL) and srl_ppo_loss_from_logits_masked
-int ppo_loss_from_logits(const char* fn, const float* logits, const uint8_t* available, const int32_t* action,
-                         const int32_t* head_sizes_host, int heads, const float* v_pred, const float* old_logp,
-                         const float* old_value, const float* ret, const float* adv, const uint8_t* on_reset_next,
-                         int64_t ld_smp, const int32_t* lane_idx, int T, int n, const double* norm_stats,
-                         const double* local_stats, const double* popart_mean_std, const srl_ppo_hyper* hyper,
-                         float* g_logits, float* g_value, float* logp_out, float* entropy_out, double* out, float* out_f32,
-                         void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+// srl_ppo_loss_from_logits (available == NULL) and srl_ppo_loss_from_logits_masked (elem_bytes = 4), and their _bf16 twins
+// (elem_bytes = 2: logits, v_pred, g_logits and g_value are bfloat16)
+int ppo_loss_from_logits(const char* fn, size_t elem_bytes, const void* logits, const uint8_t* available,
+                         const int32_t* action, const int32_t* head_sizes_host, int heads, const void* v_pred,
+                         const float* old_logp, const float* old_value, const float* ret, const float* adv,
+                         const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+                         const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+                         const srl_ppo_hyper* hyper, void* g_logits, void* g_value, float* logp_out, float* entropy_out,
+                         double* out, float* out_f32, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   SRL_REQUIRE(T >= 1 && n >= 1, SRL_ERR_INVALID_ARG, "%s: need T >= 1 and n >= 1", fn);
   SRL_REQUIRE(heads >= 1 && heads <= SRL_MAX_HEADS && head_sizes_host, SRL_ERR_INVALID_ARG,
               "%s: heads=%d outside [1, %d]", fn, heads, SRL_MAX_HEADS);
@@ -389,22 +411,22 @@ int ppo_loss_from_logits(const char* fn, const float* logits, const uint8_t* ava
   int rc = fill_loss_hyper(hyper, popart_mean_std, q.s.h);
   if (rc != SRL_OK) return rc;
   SRL_REQUIRE(!(q.s.h.clip_value && old_value == nullptr), SRL_ERR_INVALID_ARG, "%s: clip_value needs old_value", fn);
-  int sk = 0;
+  long long sk = 0;
   for (int i = 0; i < SRL_MAX_HEADS; ++i) {
     q.head_size[i] = i < heads ? head_sizes_host[i] : 0;
     SRL_REQUIRE(i >= heads || head_sizes_host[i] >= 1, SRL_ERR_INVALID_ARG, "%s: head %d has no actions", fn, i);
     sk += q.head_size[i];
   }
   const bool masked = available != nullptr;
-  const size_t row_bytes = static_cast<size_t>(256) * sk * sizeof(float);  // dense [256, sum K] block
-  const size_t mask_bytes = masked ? static_cast<size_t>(256) * sk : 0;    // + its [256, sum K] availability bytes
   const int max_sk = masked ? SRL_K4B_MAX_SUM_K_MASKED : SRL_K4B_MAX_SUM_K;
-  SRL_REQUIRE(row_bytes + mask_bytes + 16 <= 200 * 1024, SRL_ERR_UNSUPPORTED, "%s: sum K = %d too wide (max %d)", fn, sk,
-              max_sk);
-  const bool cache_e = 2 * row_bytes + mask_bytes + 16 <= 200 * 1024;  // both blocks fit: one exponential per logit
-  const size_t smem = (cache_e ? 2 * row_bytes : row_bytes) + mask_bytes + 16;  // + the mbarrier of the bulk copies
+  SRL_REQUIRE(sk <= max_sk, SRL_ERR_UNSUPPORTED, "%s: sum K = %lld too wide (max %d)", fn, sk, max_sk);
+  const size_t row_bytes = static_cast<size_t>(256) * sk * elem_bytes;     // dense [256, sum K] block of the element type
+  const size_t e_bytes = static_cast<size_t>(256) * sk * sizeof(float);    // the cached exponentials, float either way
+  const size_t mask_bytes = masked ? static_cast<size_t>(256) * sk : 0;    // + its [256, sum K] availability bytes
+  const bool cache_e = row_bytes + e_bytes + mask_bytes + 16 <= 200 * 1024;  // all fit: one exponential per logit
+  const size_t smem = row_bytes + (cache_e ? e_bytes : 0) + mask_bytes + 16;  // + the mbarrier of the bulk copies
   q.heads = heads;
-  q.SK = sk;
+  q.SK = static_cast<int>(sk);
   q.logits = logits;
   q.available = available;
   q.action = action;
@@ -432,16 +454,19 @@ int ppo_loss_from_logits(const char* fn, const float* logits, const uint8_t* ava
   p.smp_vec_ok = 0;
   Problem& pr = q.pr;
   pr.new_logp = pr.entropy = nullptr;
-  pr.v_pred = v_pred;
+  pr.v_pred = static_cast<const float*>(v_pred);  // of the element type, as g_value
   pr.lane_idx = lane_idx;
   pr.norm_stats = norm_stats;
   pr.local_stats = local_stats;
   pr.g_logp = pr.g_entropy = nullptr;
-  pr.g_value = g_value;
+  pr.g_value = static_cast<float*>(g_value);
   pr.out = out;
   pr.out_f32 = out_f32;
   pr.slot = reinterpret_cast<SlotHeader*>(workspace);
-  return masked ? launch_logits<true>(q, cache_e, smem, stream) : launch_logits<false>(q, cache_e, smem, stream);
+  if (elem_bytes == sizeof(__nv_bfloat16))
+    return masked ? launch_logits<true, __nv_bfloat16>(q, cache_e, smem, stream)
+                  : launch_logits<false, __nv_bfloat16>(q, cache_e, smem, stream);
+  return masked ? launch_logits<true, float>(q, cache_e, smem, stream) : launch_logits<false, float>(q, cache_e, smem, stream);
 }
 
 }  // namespace
@@ -655,10 +680,11 @@ extern "C" int srl_ppo_loss_from_logits(const float* logits, const int32_t* acti
                                         float* g_value, float* logp_out, float* entropy_out, double* out,
                                         float* out_f32, void* workspace, size_t workspace_bytes,
                                         srl_stream_t stream) {
-  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits", logits, nullptr, action, head_sizes_host, heads, v_pred,
-                                         old_logp, old_value, ret, adv, on_reset_next, ld_smp, lane_idx, T, n, norm_stats,
-                                         local_stats, popart_mean_std, hyper, g_logits, g_value, logp_out, entropy_out, out,
-                                         out_f32, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits", sizeof(float), logits, nullptr, action, head_sizes_host,
+                                         heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp, lane_idx, T, n,
+                                         norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value, logp_out,
+                                         entropy_out, out, out_f32, workspace, workspace_bytes,
+                                         static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int srl_ppo_loss_from_logits_masked(const float* logits, const uint8_t* available, const int32_t* action,
@@ -672,9 +698,44 @@ extern "C" int srl_ppo_loss_from_logits_masked(const float* logits, const uint8_
                                                void* workspace, size_t workspace_bytes, srl_stream_t stream) {
   SRL_REQUIRE(available != nullptr, SRL_ERR_INVALID_ARG,
               "srl_ppo_loss_from_logits_masked: null pointer available (use srl_ppo_loss_from_logits without a mask)");
-  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked", logits, available, action, head_sizes_host, heads,
-                                         v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp, lane_idx, T, n,
-                                         norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value, logp_out,
-                                         entropy_out, out, out_f32, workspace, workspace_bytes,
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked", sizeof(float), logits, available, action,
+                                         head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp,
+                                         lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value,
+                                         logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
+                                         static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int srl_ppo_loss_from_logits_bf16(const uint16_t* logits, const int32_t* action, const int32_t* head_sizes_host,
+                                             int heads, const uint16_t* v_pred, const float* old_logp,
+                                             const float* old_value, const float* ret, const float* adv,
+                                             const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T,
+                                             int n, const double* norm_stats, const double* local_stats,
+                                             const double* popart_mean_std, const srl_ppo_hyper* hyper, uint16_t* g_logits,
+                                             uint16_t* g_value, float* logp_out, float* entropy_out, double* out,
+                                             float* out_f32, void* workspace, size_t workspace_bytes,
+                                             srl_stream_t stream) {
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_bf16", sizeof(__nv_bfloat16), logits, nullptr, action,
+                                         head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp,
+                                         lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value,
+                                         logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
+                                         static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int srl_ppo_loss_from_logits_masked_bf16(const uint16_t* logits, const uint8_t* available, const int32_t* action,
+                                                    const int32_t* head_sizes_host, int heads, const uint16_t* v_pred,
+                                                    const float* old_logp, const float* old_value, const float* ret,
+                                                    const float* adv, const uint8_t* on_reset_next, int64_t ld_smp,
+                                                    const int32_t* lane_idx, int T, int n, const double* norm_stats,
+                                                    const double* local_stats, const double* popart_mean_std,
+                                                    const srl_ppo_hyper* hyper, uint16_t* g_logits, uint16_t* g_value,
+                                                    float* logp_out, float* entropy_out, double* out, float* out_f32,
+                                                    void* workspace, size_t workspace_bytes, srl_stream_t stream) {
+  SRL_REQUIRE(available != nullptr, SRL_ERR_INVALID_ARG,
+              "srl_ppo_loss_from_logits_masked_bf16: null pointer available (use srl_ppo_loss_from_logits_bf16 without a "
+              "mask)");
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked_bf16", sizeof(__nv_bfloat16), logits, available,
+                                         action, head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next,
+                                         ld_smp, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits,
+                                         g_value, logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
                                          static_cast<cudaStream_t>(stream));
 }

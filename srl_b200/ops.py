@@ -613,15 +613,25 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     """Loss starting from the actor head's logits `[T, n, sum K]` and int32 actions `[T, n, heads]`
     (actor_critic_policy.py:303-324 fused in).  Returns (g_logits, g_value, out, out_f32, logp, entropy).
 
+    `logits` and `v_pred` are torch.float32 or torch.bfloat16, the same for both (a bfloat16 policy under
+    torch.autocast passes its outputs as they are); g_logits and g_value come back in that dtype, logp / entropy and the
+    statistics are float32.  bfloat16 inputs are widened exactly and the arithmetic is float32; each gradient is rounded
+    to bfloat16 once (nearest even).
     `available` (SMAC's available_action, the logits' shape): where it is 0 the logit is replaced by -1e10 before the
     Categorical (actor_critic_policy.py:135-136) and its gradient is 0.  torch.uint8 and torch.bool are read in place; a
     floating mask costs one extra pass (`available != 0`).  At most 159 logits per transition with a mask, 199 without.
     `defer` (needs an explicit `workspace` slot): out / out_f32 are None and loss_finalize folds the slot later."""
     if available is not None:
         available = _availability(available, logits)
-    _check(logits, torch.float32, "logits")
+    dtype = logits.dtype if isinstance(logits, torch.Tensor) else torch.float32
+    if dtype not in (torch.float32, torch.bfloat16):
+        raise ValueError(f"logits: expected dtype torch.float32 or torch.bfloat16, got {dtype}")
+    if isinstance(v_pred, torch.Tensor) and v_pred.dtype != dtype:
+        raise ValueError(f"v_pred has dtype {v_pred.dtype} but logits have {dtype}; both must have the same dtype, cast "
+                         f"one of them")
+    _check(logits, dtype, "logits")
     _check(action, torch.int32, "action")
-    _check(v_pred, torch.float32, "v_pred")
+    _check(v_pred, dtype, "v_pred")
     heads = len(head_sizes)
     if not 1 <= heads <= SRL_MAX_HEADS:
         raise ValueError(f"between 1 and {SRL_MAX_HEADS} action heads are supported, got {heads}")
@@ -639,8 +649,8 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     dev = logits.device
     g_logits = torch.empty_like(logits)
     g_value = torch.empty_like(v_pred)
-    logp = torch.empty_like(v_pred) if want_logp_entropy else None
-    ent = torch.empty_like(v_pred) if want_logp_entropy else None
+    logp = torch.empty_like(v_pred, dtype=torch.float32) if want_logp_entropy else None
+    ent = torch.empty_like(v_pred, dtype=torch.float32) if want_logp_entropy else None
     if defer:
         if workspace is None:
             raise ValueError("deferred finalisation needs an explicit workspace slot")
@@ -654,10 +664,11 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     tail = (hs, heads, _ptr(v_pred), _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp,
             _ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
             _ptr(g_logits), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws), ws.numel(), _stream())
+    suffix = "_bf16" if dtype == torch.bfloat16 else ""
     if available is None:
-        _lib.call("srl_ppo_loss_from_logits", _ptr(logits), _ptr(action), *tail)
+        _lib.call("srl_ppo_loss_from_logits" + suffix, _ptr(logits), _ptr(action), *tail)
     else:
-        _lib.call("srl_ppo_loss_from_logits_masked", _ptr(logits), _ptr(available), _ptr(action), *tail)
+        _lib.call("srl_ppo_loss_from_logits_masked" + suffix, _ptr(logits), _ptr(available), _ptr(action), *tail)
     return g_logits, g_value, out, out_f32, logp, ent
 
 
@@ -776,7 +787,10 @@ class PPOGaussianLossFunction(torch.autograd.Function):
 class PPOCategoricalLossFunction(torch.autograd.Function):
     """Autograd node for a categorical policy (K4b): forward returns the scalar loss (float32) and the float64 stats
     vector of ppo_loss_from_logits; backward hands the gradients the same launch produced to the logits (exactly 0 where
-    `available` is 0) and v_pred.  `available` is the availability mask or None.
+    `available` is 0) and v_pred.  `available` is the availability mask or None.  A bfloat16 policy (torch.autocast(
+    "cuda", dtype=torch.bfloat16)) passes its bfloat16 logits and value as they are, with no casts: the launch reads
+    bfloat16, and backward hands the launch's bfloat16 gradients (the float32 ones rounded once) times the incoming
+    gradient to the bfloat16 inputs.
 
         loss, out = PPOCategoricalLossFunction.apply(logits, available, action, head_sizes, v_pred, old_logp, old_value,
                                                      ret, adv, on_reset_next, norm_stats, local_stats, popart_mean_std,
