@@ -426,6 +426,31 @@ int srl_ppo_loss_from_gaussian(
     float* g_mean, float* g_log_std /* [T,n,D] or [D] */, float* g_value,
     float* logp_out, float* entropy_out,                           /* [T,n] or NULL                      */
     double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+/* The entry above with a bfloat16 policy side, for Gaussian policies trained under torch.autocast(dtype=torch.bfloat16),
+ * whose last nn.Linear layers produce bfloat16 means and values.  Same arguments in the same order; mean, v_pred, g_mean
+ * and g_value are bfloat16 bit patterns (uint16_t).  log_std and g_log_std are untyped because their element type follows
+ * log_std_shared: bfloat16 [T,n,D] per transition (the output of a head), float32 [D] when shared (an nn.Parameter, which
+ * autocast leaves float32; its gradient, a sum over the minibatch, feeds float32 master weights and is not rounded).
+ * action stays float32: old_logp was computed on the sampled float32 action, and a rounded one would bias every ratio.
+ * logp_out / entropy_out, the sample side and the ten outputs stay float32.  Each bfloat16 input is widened to float32
+ * exactly where it is read and all arithmetic is the entry above's, so logp and entropy are bit-identical to
+ * srl_ppo_loss_from_gaussian's on the widened values, and each bfloat16 gradient is that entry's float32 result rounded
+ * to bfloat16 once (round to nearest even).  out, out_f32 and a shared g_log_std are float64 sums added in an order the
+ * launch grid fixes; they are bit-identical too whenever both entries launch the same grid, which is always the case
+ * for T * n <= 256 * (number of SMs), and at any size unless the smaller bfloat16 blocks fit 2 CTAs per SM where the
+ * float32 ones fit 1 (on a B200: D = 37 .. 55 per transition, D = 54 .. 64 shared).  D is 1 .. 64, the workspace is the
+ * one srl_ppo_loss_gaussian_workspace_bytes sizes, and deferred finalisation works as above. */
+int srl_ppo_loss_from_gaussian_bf16(
+    const uint16_t* mean, const void* log_std, int log_std_shared, /* [T,n,D] bf16; log_std [T,n,D] bf16 or [D] f32 */
+    const float* action, int D,                                      /* [T,n,D] float32                              */
+    const uint16_t* v_pred,                                          /* [T,n] bfloat16                               */
+    const float* old_logp, const float* old_value, const float* ret, const float* adv,
+    const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper,
+    uint16_t* g_mean, void* g_log_std /* [T,n,D] bf16 or [D] f32 */, uint16_t* g_value, /* bfloat16 out */
+    float* logp_out, float* entropy_out,                             /* [T,n] float32 or NULL                        */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * K5a  Philox-keyed permutation of the environment axis (NEW capability: the reference has no

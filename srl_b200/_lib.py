@@ -130,6 +130,12 @@ SIGNATURES = {
                                            c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                            c_void_p, c_size_t, c_void_p]),
+    # mean, v_pred, g_mean, g_value: bfloat16 device pointers; log_std, g_log_std: bfloat16 per row, float32 when shared
+    "srl_ppo_loss_from_gaussian_bf16": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
+                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                                c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                c_void_p, c_size_t, c_void_p]),
     "srl_philox_perm": (c_int, [c_uint64, c_uint32, c_int, c_int, c_int, c_void_p, c_void_p]),
     "srl_philox4x32_10": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "srl_batch_gather": (c_int, [POINTER(LeafDesc), c_int, c_void_p, c_int, c_int, c_void_p]),

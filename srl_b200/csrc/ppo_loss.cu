@@ -85,17 +85,6 @@ constexpr int kStage = 9;  // manual staging batch per thread (last, partial til
 // actor_critic_policy.py:135-136: logits.masked_fill(available_action == 0, -1e10) before the Categorical
 constexpr float kUnavailableLogit = -1e10f;
 
-// A policy-side element as the arithmetic reads it (bfloat16 -> float is exact), and a result stored back in the element
-// type (bfloat16: rounded to nearest even, once, where the float result is final).
-__device__ __forceinline__ float to_float(float x) { return x; }
-__device__ __forceinline__ float to_float(__nv_bfloat16 x) { return __bfloat162float(x); }
-template <typename T>
-__device__ __forceinline__ T from_float(float x);
-template <>
-__device__ __forceinline__ float from_float<float>(float x) { return x; }
-template <>
-__device__ __forceinline__ __nv_bfloat16 from_float<__nv_bfloat16>(float x) { return __float2bfloat16_rn(x); }
-
 // logit k of a row as the Categorical sees it
 template <bool MASKED, typename T>
 __device__ __forceinline__ float logit_at(const T* z, const uint8_t* m, int k) {

@@ -38,6 +38,17 @@ __device__ __forceinline__ unsigned long long box(double x) { return static_cast
 __device__ __forceinline__ double unbox(unsigned long long w) { return __longlong_as_double(static_cast<long long>(w ^ kBoxKey)); }
 static_assert(sizeof(SlotHeader) == kPartialsOffset, "slot header must stay 64 bytes");
 
+// A policy-side element of K4b / K4c as the arithmetic reads it (bfloat16 -> float is exact), and a result stored back in
+// the element type (bfloat16: rounded to nearest even, once, where the float result is final).
+__device__ __forceinline__ float to_float(float x) { return x; }
+__device__ __forceinline__ float to_float(__nv_bfloat16 x) { return __bfloat162float(x); }
+template <typename T>
+__device__ __forceinline__ T from_float(float x);
+template <>
+__device__ __forceinline__ float from_float<float>(float x) { return x; }
+template <>
+__device__ __forceinline__ __nv_bfloat16 from_float<__nv_bfloat16>(float x) { return __float2bfloat16_rn(x); }
+
 struct LossHyperDev {
   float clip_lo, clip_hi;  // (float)(1 -/+ eps_clip)
   float veps;

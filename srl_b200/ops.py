@@ -705,10 +705,34 @@ def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, r
     loss is ppo_loss_fwd_bwd's.  Returns (g_mean, g_log_std, g_value, out, out_f32, logp, entropy): g_log_std has
     log_std's shape (a shared log_std gets the sum over the minibatch); logp / entropy `[T, n]` only with
     want_logp_entropy.  `defer` (needs an explicit `workspace`): out / out_f32 are None and loss_finalize folds the
-    slot later; the gradients are complete either way."""
-    _check(v_pred, torch.float32, "v_pred")
+    slot later; the gradients are complete either way.
+
+    `mean`, `v_pred` and a per-transition `log_std` are torch.float32 or torch.bfloat16, the same for all three (a Gaussian
+    policy under torch.autocast passes its bfloat16 outputs as they are); their gradients come back in that dtype, logp /
+    entropy and the statistics are float32.  bfloat16 inputs are widened exactly and the arithmetic is the float32
+    entry's; each bfloat16 gradient is the float32 one rounded once (nearest even).  A shared `[D]` log_std is float32
+    (an nn.Parameter, which autocast leaves alone) or bfloat16 (a module cast with .bfloat16()) with either mean dtype:
+    it is widened (D elements), its gradient is summed in float64 as always, and comes back float32 or rounded to
+    bfloat16 once, in log_std's dtype.  `action` is float32 always: the actions the actors sampled, on which old_logp
+    was computed."""
+    dtype = mean.dtype if isinstance(mean, torch.Tensor) else torch.float32
+    if dtype not in (torch.float32, torch.bfloat16):
+        raise ValueError(f"mean: expected dtype torch.float32 or torch.bfloat16, got {dtype}")
+    if isinstance(v_pred, torch.Tensor) and v_pred.dtype != dtype:
+        raise ValueError(f"v_pred has dtype {v_pred.dtype} but mean has {dtype}; both must have the same dtype, cast "
+                         f"one of them")
+    if isinstance(log_std, torch.Tensor):
+        if log_std.dim() > 1 and log_std.dtype != dtype:
+            raise ValueError(f"log_std has dtype {log_std.dtype} but mean has {dtype}; a per-transition log_std must have "
+                             f"mean's dtype, cast one of them")
+        if log_std.dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError(f"log_std: expected dtype torch.float32 or torch.bfloat16, got {log_std.dtype}")
+    if isinstance(action, torch.Tensor) and action.dtype != torch.float32:
+        raise ValueError(f"action: expected dtype torch.float32, got {action.dtype}; pass the float32 actions the actors "
+                         f"sampled (old_logp was computed on them, and a rounded action would bias every ratio)")
+    _check(v_pred, dtype, "v_pred")
     T, n = _rows_lanes(v_pred)
-    _check(mean, torch.float32, "mean")
+    _check(mean, dtype, "mean")
     _check(action, torch.float32, "action")
     D = mean.shape[-1] if mean.dim() >= 2 else 0
     if mean.dim() < 2 or mean.shape[0] != T or mean.numel() != T * n * D:
@@ -729,7 +753,11 @@ def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, r
     else:
         raise ValueError(f"log_std: expected [D] = [{D}] (shared) or mean's shape {tuple(mean.shape)} (per transition), "
                          f"got {tuple(log_std.shape)}")
-    _check(log_std, torch.float32, "log_std")
+    _check(log_std, log_std.dtype, "log_std")
+    # a shared bfloat16 [D] log_std: the kernel reads float32 [D] for both policy dtypes
+    ls_dtype = log_std.dtype
+    if shared and ls_dtype == torch.bfloat16:
+        log_std = log_std.float()
     ld_smp = _sample_side(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, hyper.clip_value)
     _check(norm_stats, torch.float64, "norm_stats")
     local_stats = norm_stats if local_stats is None else _check(local_stats, torch.float64, "local_stats")
@@ -739,8 +767,8 @@ def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, r
     g_mean = torch.empty_like(mean)
     g_log_std = torch.empty_like(log_std)
     g_value = torch.empty_like(v_pred)
-    logp = torch.empty_like(v_pred) if want_logp_entropy else None
-    ent = torch.empty_like(v_pred) if want_logp_entropy else None
+    logp = torch.empty_like(v_pred, dtype=torch.float32) if want_logp_entropy else None
+    ent = torch.empty_like(v_pred, dtype=torch.float32) if want_logp_entropy else None
     if defer:
         if workspace is None:
             raise ValueError("deferred finalisation needs an explicit workspace")
@@ -750,18 +778,25 @@ def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, r
         out_f32 = torch.empty(4, dtype=torch.float32, device=dev)
     ws = gaussian_loss_workspace(dev) if workspace is None else _check(workspace, torch.uint8, "workspace")
     hc = hyper.to_c()
-    _lib.call("srl_ppo_loss_from_gaussian", _ptr(mean), _ptr(log_std), int(shared), _ptr(action), D, _ptr(v_pred),
-              _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp, _ptr(lane_idx), T, n,
-              _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc), _ptr(g_mean),
-              _ptr(g_log_std), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws), ws.numel(),
-              _stream())
+    suffix = "_bf16" if dtype == torch.bfloat16 else ""
+    _lib.call("srl_ppo_loss_from_gaussian" + suffix, _ptr(mean), _ptr(log_std), int(shared), _ptr(action), D,
+              _ptr(v_pred), _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp,
+              _ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
+              _ptr(g_mean), _ptr(g_log_std), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws),
+              ws.numel(), _stream())
+    if g_log_std.dtype != ls_dtype:
+        g_log_std = g_log_std.to(ls_dtype)  # what autograd's cast hands a bfloat16 parameter through .float()
     return g_mean, g_log_std, g_value, out, out_f32, logp, ent
 
 
 class PPOGaussianLossFunction(torch.autograd.Function):
     """Autograd node for a continuous-action policy: forward returns the scalar loss (float32) and the float64 stats
     vector of ppo_loss_from_gaussian; backward hands the gradients the same launch produced to mean, log_std ([D]
-    parameter or [T, n, D]) and v_pred.
+    parameter or [T, n, D]) and v_pred.  A policy under torch.autocast("cuda", dtype=torch.bfloat16) passes its bfloat16
+    mean, value and per-transition log_std as they are, with no casts, and a float32 (or, in a module cast with
+    .bfloat16(), bfloat16) [D] log_std parameter; the action stays float32.  Each input gets a gradient of its own dtype:
+    the launch's bfloat16 gradients (the float32 ones rounded once) for the bfloat16 inputs, the float32 [D] gradient for
+    a float32 parameter, rounded once for a bfloat16 one.
 
         loss, out = PPOGaussianLossFunction.apply(mean, log_std, action, v_pred, old_logp, old_value, ret, adv,
                                                   on_reset_next, norm_stats, local_stats, popart_mean_std, lane_idx, hyper)
