@@ -249,7 +249,7 @@ enum srl_loss_out {
  * before the slot is used again.  Launches that may overlap in time need distinct slots. */
 size_t srl_ppo_loss_workspace_bytes(int T, int n);
 
-/* Deferred finalisation: when srl_ppo_loss_fwd_bwd / srl_ppo_loss_from_logits(_masked)(_bf16) are called with out == NULL they
+/* Deferred finalisation: when srl_ppo_loss_fwd_bwd / srl_ppo_loss_from_logits(_masked)(_bf16)(_pack) are called with out == NULL they
  * stop after writing gradients and partial rows.  This folds n_slots consecutive slots (slot k at
  * workspace + k * slot_bytes) into out[k][SRL_LOSS_OUT_LEN] (and out_f32[k][4] if not NULL) in one launch, and
  * clears the rows it folded. */
@@ -395,6 +395,27 @@ int srl_ppo_loss_from_logits_masked_bf16(
     float* logp_out, float* entropy_out,             /* [T, n] float32 out or NULL */
     double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
 
+/* srl_ppo_loss_from_logits(_masked)(_bf16) with the sample side read from K2's loss pack (srl_gae_scan's `pack`: the BASE of
+ * the buffer, pack_lanes = its N lanes, pack_row_lo = the absolute sample row of loss row 0) instead of the five leaves:
+ * transition (t, j) reads ONE 16-byte item {old_logp, value, ret, mask ? adv : NaN} at lane c = lane_idx ? lane_idx[j] : j
+ * and row pack_row_lo + t -- what a permuted minibatch of the trainer has.  elem_bytes = 4 (float32) or 2 (bfloat16)
+ * selects the policy side's element type with the rules of the _bf16 entries; available may be NULL (no mask) or the mask
+ * of srl_ppo_loss_from_logits_masked.  Same grid, same per-element arithmetic and the same fold order as the leaf entry
+ * with the same lane_idx: the results are bit-identical to it on the leaves the pack was written from.  Invalid arguments
+ * besides the leaf entries': a NULL or not 16-byte aligned pack, pack_row_lo < 0, lane_idx == NULL with pack_lanes < n,
+ * elem_bytes other than 2 or 4.  Deferred finalisation works as above. */
+int srl_ppo_loss_from_logits_pack(
+    const void* logits, int elem_bytes, /* [T, n, sumK] dense, float32 or bfloat16 */
+    const uint8_t* available,           /* [T, n, sumK] dense or NULL               */
+    const int32_t* action,              /* [T, n, heads]                            */
+    const int32_t* head_sizes_host, int heads, const void* v_pred, /* [T, n] dense, the logits' type */
+    const float* pack, int64_t pack_lanes, int pack_row_lo, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper, void* g_logits, /* [T, n, sumK] out, the logits' type */
+    void* g_value,                               /* [T, n] out, the logits' type */
+    float* logp_out, float* entropy_out,         /* [T, n] float32 out or NULL */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * K4c  Same loss, but starting from a diagonal-Gaussian actor head (continuous actions, D = 1 .. 64 dimensions).
  * NEW capability: the reference's policies are categorical, so no reference line pins this head; the definition is
@@ -450,6 +471,22 @@ int srl_ppo_loss_from_gaussian_bf16(
     const srl_ppo_hyper* hyper,
     uint16_t* g_mean, void* g_log_std /* [T,n,D] bf16 or [D] f32 */, uint16_t* g_value, /* bfloat16 out */
     float* logp_out, float* entropy_out,                             /* [T,n] float32 or NULL                        */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+
+/* srl_ppo_loss_from_gaussian(_bf16) with the sample side read from K2's loss pack, as srl_ppo_loss_from_logits_pack reads
+ * it (pack_lanes, pack_row_lo, lane_idx: see there).  elem_bytes = 4 or 2 selects the float32 or bfloat16 policy side with
+ * the rules of the _bf16 entry (a shared [D] log_std and its gradient are float32 either way).  Bit-identical to the leaf
+ * entry with the same lane_idx on the leaves the pack was written from; the same argument checks as
+ * srl_ppo_loss_from_logits_pack besides the leaf entries' (D, workspace size, deferred mode). */
+int srl_ppo_loss_from_gaussian_pack(
+    const void* mean, const void* log_std, int log_std_shared, /* [T,n,D]; log_std [T,n,D] (mean's type) or [D] f32 */
+    const float* action, int D,                                  /* [T,n,D] float32                                   */
+    int elem_bytes, const void* v_pred,                          /* [T,n], mean's type                                */
+    const float* pack, int64_t pack_lanes, int pack_row_lo, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper,
+    void* g_mean, void* g_log_std /* [T,n,D] or [D] f32 */, void* g_value,
+    float* logp_out, float* entropy_out,                         /* [T,n] float32 or NULL                             */
     double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------

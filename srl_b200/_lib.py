@@ -136,6 +136,17 @@ SIGNATURES = {
                                                 c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
                                                 c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                                 c_void_p, c_size_t, c_void_p]),
+    # sample side from K2's pack; elem_bytes 4 / 2 selects the float32 / bfloat16 policy side
+    "srl_ppo_loss_from_logits_pack": (c_int, [c_void_p, c_int, c_void_p, c_void_p, POINTER(c_int32), c_int, c_void_p,
+                                              c_void_p, c_int64, c_int, c_void_p,
+                                              c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                              c_size_t, c_void_p]),
+    "srl_ppo_loss_from_gaussian_pack": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p,
+                                                c_void_p, c_int64, c_int, c_void_p,
+                                                c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                c_void_p, c_size_t, c_void_p]),
     "srl_philox_perm": (c_int, [c_uint64, c_uint32, c_int, c_int, c_int, c_void_p, c_void_p]),
     "srl_philox4x32_10": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "srl_batch_gather": (c_int, [POINTER(LeafDesc), c_int, c_void_p, c_int, c_int, c_void_p]),

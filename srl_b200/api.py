@@ -10,11 +10,14 @@ Inside an SRL checkout, use SRL's own classes: `srl_b200.srl_plugin.register_int
   PytorchTrainer       api/trainer.py:160-193    (policy property, distributed(), device selection)
   register / make      api/trainer.py:231-246
   TrajPostprocessor, register_traj_postprocessor / make_traj_postprocessor   api/trainer.py:84-99,249-262
+
+and one record of this package's own, `PPOHeadAnalyzedResult`: what a policy that declares `ppo_head = True` returns from
+`analyze(sample, target="ppo_head", ...)`.
 """
 from __future__ import annotations
 
 import dataclasses
-from typing import Any, Dict, Optional
+from typing import Any, Dict, Optional, Sequence
 
 import numpy as np
 import torch
@@ -43,6 +46,37 @@ class AnalyzedResult(NamedArray):
 
     def __init__(self, value=None, log_probs=None, adv=None, ret=None, **extra):
         super().__init__(value=value, log_probs=log_probs, adv=adv, ret=ret, **extra)
+
+
+@dataclasses.dataclass
+class PPOHeadAnalyzedResult:
+    """The actor head and the value of a policy, for a trainer that computes log-probabilities and entropies itself.
+
+    A policy opts in by declaring the class attribute `ppo_head = True`; `MultiAgentPPOB200` then calls
+    `policy.analyze(sample, target="ppo_head", burn_in_steps=...)` instead of `target="ppo"` and trains through the fused
+    head losses (K4b / K4c): the policy builds no torch.distributions object, and the trainer hands the gradients of the
+    loss with respect to the fields below to autograd.  Return them as the network produced them (still attached to the
+    graph).  Shapes lead with the analyzed rows and lanes `[T', B, (A,)]` of the sample, burn-in rows already dropped, as
+    `target="ppo"` returns its tensors; float32 or bfloat16 (torch.autocast) on the policy's device.
+
+    Exactly one head kind:
+      categorical (actor_critic_policy.py:303-324): `logits [T', B, (A,) sum K]` -- what the policy would hand to
+        `Categorical(logits=...)`, the heads side by side -- `head_sizes` (the K of each head, at most 8 heads, sum K <= 199,
+        <= 159 with a mask) and optionally `available` (SMAC's available_action, the logits' shape, non-zero = available;
+        an unavailable logit is treated as masked_fill(-1e10), actor_critic_policy.py:135-136).  `action [T', B, (A,)
+        heads]` of any integer dtype or integer-valued floats (SRL stores `action.x` as float32); the trainer converts it
+        to int32 once.
+      diagonal Gaussian: `mean [T', B, (A,) D]`, `log_std` either one `[D]` parameter shared by every transition or the
+        mean's shape, D <= 64; `action` the float32 actions the actors sampled, the mean's shape.
+    `state_values [T', B, (A,) 1]` in the head's dtype (a scalar critic; with PopArt, the normalised value).
+    """
+    state_values: Any
+    action: Any
+    logits: Any = None
+    head_sizes: Optional[Sequence[int]] = None
+    available: Any = None
+    mean: Any = None
+    log_std: Any = None
 
 
 @dataclasses.dataclass

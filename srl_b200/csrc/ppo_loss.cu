@@ -162,7 +162,8 @@ __device__ __forceinline__ void head_backward(T* z, const float* ez, const uint8
 // MASKED: the [256, SK] availability bytes of the tile follow the float blocks in shared memory, brought in with the logits
 // (same mbarrier and expect_tx, or the same element-wise staging); every pass over a head reads them.
 // T: the policy side's element type (float or __nv_bfloat16); the staged block holds T, the cached exponentials float.
-template <bool CACHE_E, bool MASKED, typename T>
+// PACK: the sample side is K2's loss pack (load_pack_item, ppo_loss.cuh), else the five leaves.
+template <bool CACHE_E, bool MASKED, typename T, bool PACK>
 __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kernel(const __grid_constant__ LogitsParams q) {
   // [256 * SK] of T, dense (+ [256 * SK] floats with CACHE_E), (+ [256 * SK] bytes with MASKED), then the mbarrier
   extern __shared__ __align__(128) float smem[];
@@ -237,11 +238,16 @@ __global__ void __launch_bounds__(256, SRL_K4B_MIN_BLOCKS) ppo_loss_logits_kerne
       const int t = static_cast<int>(i / p.n);
       const int j = static_cast<int>(i - static_cast<long long>(t) * p.n);
       const int c = pr.lane_idx ? pr.lane_idx[j] : j;
-      const long long os = t * p.ld_smp + c;
-      vp = to_float(ldg_stream(reinterpret_cast<const T*>(pr.v_pred) + i));
-      ol = __ldg(p.old_logp + os), rt = __ldg(p.ret + os), ad = __ldg(p.adv + os);
-      ov = h.clip_value ? __ldg(p.old_value + os) : 0.f;
-      valid = __ldg(p.reset_next + os) == 0;
+      if constexpr (PACK) {
+        vp = to_float(ldg_stream(reinterpret_cast<const T*>(pr.v_pred) + i));
+        load_pack_item(p, t, c, ol, ov, rt, ad, valid);
+      } else {
+        const long long os = t * p.ld_smp + c;
+        vp = to_float(ldg_stream(reinterpret_cast<const T*>(pr.v_pred) + i));
+        ol = __ldg(p.old_logp + os), rt = __ldg(p.ret + os), ad = __ldg(p.adv + os);
+        ov = h.clip_value ? __ldg(p.old_value + os) : 0.f;
+        valid = __ldg(p.reset_next + os) == 0;
+      }
 #pragma unroll
       for (int hd = 0; hd < SRL_MAX_HEADS; ++hd) act[hd] = hd < q.heads ? q.action[i * q.heads + hd] : 0;
     }
@@ -350,18 +356,19 @@ static_assert(256 * SRL_K4B_MAX_SUM_K_MASKED * 5 + 16 <= 200 * 1024 && 256 * (SR
               "");
 static_assert(256 * SRL_K4B_MAX_SUM_K * 2 + 16 <= 200 * 1024 && 256 * SRL_K4B_MAX_SUM_K_MASKED * 3 + 16 <= 200 * 1024, "");
 
-// one resident wave of ppo_loss_logits_kernel<CACHE_E, MASKED, T> over the T * n transitions of q
-template <bool MASKED, typename T>
+// one resident wave of ppo_loss_logits_kernel<CACHE_E, MASKED, T, PACK> over the T * n transitions of q
+template <bool MASKED, typename T, bool PACK>
 int launch_logits(const LogitsParams& q, bool cache_e, size_t smem, cudaStream_t stream) {
   int rc;
-  if ((rc = opt_in_smem<ppo_loss_logits_kernel<true, MASKED, T>>(200 * 1024)) != SRL_OK) return rc;
-  if ((rc = opt_in_smem<ppo_loss_logits_kernel<false, MASKED, T>>(200 * 1024)) != SRL_OK) return rc;
+  if ((rc = opt_in_smem<ppo_loss_logits_kernel<true, MASKED, T, PACK>>(200 * 1024)) != SRL_OK) return rc;
+  if ((rc = opt_in_smem<ppo_loss_logits_kernel<false, MASKED, T, PACK>>(200 * 1024)) != SRL_OK) return rc;
   const long long tiles = (static_cast<long long>(q.s.T) * q.s.n + 255) / 256;
   // one wave: as many CTAs as are resident with this much shared memory (2048 tiles on 1184 assumed slots were 1024 CTAs on
   // the 740 real ones -- a second, partial wave)
   int per_sm = 0;
-  if ((cache_e ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<true, MASKED, T>, 256, smem)
-               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<false, MASKED, T>, 256, smem)) !=
+  if ((cache_e ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<true, MASKED, T, PACK>, 256, smem)
+               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppo_loss_logits_kernel<false, MASKED, T, PACK>, 256,
+                                                               smem)) !=
           cudaSuccess ||
       per_sm < 1)
     per_sm = 1;
@@ -371,35 +378,39 @@ int launch_logits(const LogitsParams& q, bool cache_e, size_t smem, cudaStream_t
   const long long per_cta = (tiles + cap - 1) / cap;
   const int grid = static_cast<int>((tiles + per_cta - 1) / per_cta);
   if (cache_e)
-    ppo_loss_logits_kernel<true, MASKED, T><<<grid, 256, smem, stream>>>(q);
+    ppo_loss_logits_kernel<true, MASKED, T, PACK><<<grid, 256, smem, stream>>>(q);
   else
-    ppo_loss_logits_kernel<false, MASKED, T><<<grid, 256, smem, stream>>>(q);
+    ppo_loss_logits_kernel<false, MASKED, T, PACK><<<grid, 256, smem, stream>>>(q);
   SRL_CUDA(cudaGetLastError());
   return SRL_OK;
 }
 
-// srl_ppo_loss_from_logits (available == NULL) and srl_ppo_loss_from_logits_masked (elem_bytes = 4), and their _bf16 twins
-// (elem_bytes = 2: logits, v_pred, g_logits and g_value are bfloat16)
+// srl_ppo_loss_from_logits (available == NULL) and srl_ppo_loss_from_logits_masked (elem_bytes = 4), their _bf16 twins
+// (elem_bytes = 2: logits, v_pred, g_logits and g_value are bfloat16) and srl_ppo_loss_from_logits_pack (pack != NULL: the
+// sample side is K2's pack, ld_smp its lanes, pack_row_lo the absolute row of loss row 0; the five leaves are not read)
 int ppo_loss_from_logits(const char* fn, size_t elem_bytes, const void* logits, const uint8_t* available,
                          const int32_t* action, const int32_t* head_sizes_host, int heads, const void* v_pred,
                          const float* old_logp, const float* old_value, const float* ret, const float* adv,
-                         const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
-                         const double* norm_stats, const double* local_stats, const double* popart_mean_std,
-                         const srl_ppo_hyper* hyper, void* g_logits, void* g_value, float* logp_out, float* entropy_out,
-                         double* out, float* out_f32, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+                         const uint8_t* on_reset_next, int64_t ld_smp, const float* pack, int pack_row_lo,
+                         const int32_t* lane_idx, int T, int n, const double* norm_stats, const double* local_stats,
+                         const double* popart_mean_std, const srl_ppo_hyper* hyper, void* g_logits, void* g_value,
+                         float* logp_out, float* entropy_out, double* out, float* out_f32, void* workspace,
+                         size_t workspace_bytes, cudaStream_t stream) {
   SRL_REQUIRE(T >= 1 && n >= 1, SRL_ERR_INVALID_ARG, "%s: need T >= 1 and n >= 1", fn);
   SRL_REQUIRE(heads >= 1 && heads <= SRL_MAX_HEADS && head_sizes_host, SRL_ERR_INVALID_ARG,
               "%s: heads=%d outside [1, %d]", fn, heads, SRL_MAX_HEADS);
-  SRL_REQUIRE(logits && action && v_pred && old_logp && ret && adv && on_reset_next && g_logits && g_value &&
+  SRL_REQUIRE(logits && action && v_pred && (pack || (old_logp && ret && adv && on_reset_next)) && g_logits && g_value &&
                   norm_stats && local_stats && workspace,
               SRL_ERR_INVALID_ARG, "%s: null pointer", fn);
-  SRL_REQUIRE(ld_smp >= (lane_idx ? 1 : n), SRL_ERR_INVALID_ARG, "%s: ld_smp smaller than the row", fn);
+  SRL_REQUIRE(ld_smp >= (lane_idx ? 1 : n), SRL_ERR_INVALID_ARG, "%s: %s smaller than the row", fn,
+              pack ? "pack_lanes" : "ld_smp");
   SRL_REQUIRE(workspace_bytes >= srl_ppo_loss_workspace_bytes(T, n), SRL_ERR_INVALID_ARG,
               "%s: workspace too small (%zu bytes)", fn, workspace_bytes);
   LogitsParams q;
   int rc = fill_loss_hyper(hyper, popart_mean_std, q.s.h);
   if (rc != SRL_OK) return rc;
-  SRL_REQUIRE(!(q.s.h.clip_value && old_value == nullptr), SRL_ERR_INVALID_ARG, "%s: clip_value needs old_value", fn);
+  SRL_REQUIRE(pack || !(q.s.h.clip_value && old_value == nullptr), SRL_ERR_INVALID_ARG, "%s: clip_value needs old_value",
+              fn);
   long long sk = 0;
   for (int i = 0; i < SRL_MAX_HEADS; ++i) {
     q.head_size[i] = i < heads ? head_sizes_host[i] : 0;
@@ -428,11 +439,11 @@ int ppo_loss_from_logits(const char* fn, size_t elem_bytes, const void* logits, 
   p.ret = ret;
   p.adv = adv;
   p.reset_next = on_reset_next;
-  p.pack = nullptr;
+  p.pack = reinterpret_cast<const float4*>(pack);
   p.lane_aos = nullptr;
   p.part = nullptr;
   p.part_ctas = p.part_first = 0;
-  p.row_lo = 0;
+  p.row_lo = pack ? pack_row_lo : 0;
   p.popart = popart_mean_std;
   p.ld_pol = n;
   p.ld_grad = n;
@@ -452,10 +463,19 @@ int ppo_loss_from_logits(const char* fn, size_t elem_bytes, const void* logits, 
   pr.out = out;
   pr.out_f32 = out_f32;
   pr.slot = reinterpret_cast<SlotHeader*>(workspace);
-  if (elem_bytes == sizeof(__nv_bfloat16))
-    return masked ? launch_logits<true, __nv_bfloat16>(q, cache_e, smem, stream)
-                  : launch_logits<false, __nv_bfloat16>(q, cache_e, smem, stream);
-  return masked ? launch_logits<true, float>(q, cache_e, smem, stream) : launch_logits<false, float>(q, cache_e, smem, stream);
+  const bool bf16 = elem_bytes == sizeof(__nv_bfloat16);
+  if (pack) {
+    if (bf16)
+      return masked ? launch_logits<true, __nv_bfloat16, true>(q, cache_e, smem, stream)
+                    : launch_logits<false, __nv_bfloat16, true>(q, cache_e, smem, stream);
+    return masked ? launch_logits<true, float, true>(q, cache_e, smem, stream)
+                  : launch_logits<false, float, true>(q, cache_e, smem, stream);
+  }
+  if (bf16)
+    return masked ? launch_logits<true, __nv_bfloat16, false>(q, cache_e, smem, stream)
+                  : launch_logits<false, __nv_bfloat16, false>(q, cache_e, smem, stream);
+  return masked ? launch_logits<true, float, false>(q, cache_e, smem, stream)
+                : launch_logits<false, float, false>(q, cache_e, smem, stream);
 }
 
 }  // namespace
@@ -670,7 +690,7 @@ extern "C" int srl_ppo_loss_from_logits(const float* logits, const int32_t* acti
                                         float* out_f32, void* workspace, size_t workspace_bytes,
                                         srl_stream_t stream) {
   return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits", sizeof(float), logits, nullptr, action, head_sizes_host,
-                                         heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp, lane_idx, T, n,
+                                         heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp, nullptr, 0, lane_idx, T, n,
                                          norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value, logp_out,
                                          entropy_out, out, out_f32, workspace, workspace_bytes,
                                          static_cast<cudaStream_t>(stream));
@@ -689,7 +709,7 @@ extern "C" int srl_ppo_loss_from_logits_masked(const float* logits, const uint8_
               "srl_ppo_loss_from_logits_masked: null pointer available (use srl_ppo_loss_from_logits without a mask)");
   return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked", sizeof(float), logits, available, action,
                                          head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp,
-                                         lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value,
+                                         nullptr, 0, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value,
                                          logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
                                          static_cast<cudaStream_t>(stream));
 }
@@ -705,7 +725,7 @@ extern "C" int srl_ppo_loss_from_logits_bf16(const uint16_t* logits, const int32
                                              srl_stream_t stream) {
   return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_bf16", sizeof(__nv_bfloat16), logits, nullptr, action,
                                          head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp,
-                                         lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value,
+                                         nullptr, 0, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value,
                                          logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
                                          static_cast<cudaStream_t>(stream));
 }
@@ -724,7 +744,30 @@ extern "C" int srl_ppo_loss_from_logits_masked_bf16(const uint16_t* logits, cons
               "mask)");
   return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked_bf16", sizeof(__nv_bfloat16), logits, available,
                                          action, head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next,
-                                         ld_smp, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits,
+                                         ld_smp, nullptr, 0, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits,
                                          g_value, logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
                                          static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int srl_ppo_loss_from_logits_pack(const void* logits, int elem_bytes, const uint8_t* available,
+                                             const int32_t* action, const int32_t* head_sizes_host, int heads,
+                                             const void* v_pred, const float* pack, int64_t pack_lanes, int pack_row_lo,
+                                             const int32_t* lane_idx, int T, int n, const double* norm_stats,
+                                             const double* local_stats, const double* popart_mean_std,
+                                             const srl_ppo_hyper* hyper, void* g_logits, void* g_value, float* logp_out,
+                                             float* entropy_out, double* out, float* out_f32, void* workspace,
+                                             size_t workspace_bytes, srl_stream_t stream) {
+  using namespace srl;
+  constexpr const char* fn = "srl_ppo_loss_from_logits_pack";
+  SRL_REQUIRE(elem_bytes == 4 || elem_bytes == 2, SRL_ERR_INVALID_ARG, "%s: elem_bytes=%d, need 4 (float32) or 2 (bfloat16)",
+              fn, elem_bytes);
+  SRL_REQUIRE(pack != nullptr && aligned(pack, 16), SRL_ERR_INVALID_ARG, "%s: pack is null or not 16-byte aligned", fn);
+  SRL_REQUIRE(pack_row_lo >= 0, SRL_ERR_INVALID_ARG, "%s: pack_row_lo=%d < 0", fn, pack_row_lo);
+  SRL_REQUIRE(lane_idx != nullptr || pack_lanes >= n, SRL_ERR_INVALID_ARG,
+              "%s: pack_lanes=%lld < n=%d without lane_idx", fn, static_cast<long long>(pack_lanes), n);
+  return srl::loss::ppo_loss_from_logits(fn, static_cast<size_t>(elem_bytes), logits, available, action, head_sizes_host,
+                                         heads, v_pred, nullptr, nullptr, nullptr, nullptr, nullptr, pack_lanes, pack,
+                                         pack_row_lo, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper,
+                                         g_logits, g_value, logp_out, entropy_out, out, out_f32, workspace,
+                                         workspace_bytes, static_cast<cudaStream_t>(stream));
 }

@@ -391,6 +391,18 @@ __device__ __forceinline__ void reduce_and_finalize(const Problem& pr, const Los
   if (threadIdx.x == 0) pr.slot->ticket = 0u;  // ready for the next launch on this slot
 }
 
+// The sample side of one K4b / K4c transition (loss row t, sample lane c) in K2's pack: ONE float4 {old_logp, value, ret,
+// mask ? adv : NaN} at pack2[(row_lo + t) / 2][c][(row_lo + t) % 2], ld_smp = the pack's N lanes -- one 16-byte gather
+// instead of five narrow ones from the leaves.
+__device__ __forceinline__ void load_pack_item(const LossShared& p, int t, int c, float& ol, float& ov, float& rt, float& ad,
+                                               bool& valid) {
+  const int ta = p.row_lo + t;
+  const float4 k = __ldg(p.pack + (static_cast<long long>(ta >> 1) * p.ld_smp + c) * 2 + (ta & 1));
+  ol = k.x, ov = k.y, rt = k.z;
+  valid = k.w == k.w;  // K2 stores NaN in the advantage slot of masked transitions
+  ad = valid ? k.w : 0.f;
+}
+
 __device__ __forceinline__ void unpack4(const float4 v, float (&a)[4]) { a[0] = v.x, a[1] = v.y, a[2] = v.z, a[3] = v.w; }
 
 // Work decomposition of the row-tile kernel (dense leaves, leaves through lane_idx, odd shapes of the pack form): grid =

@@ -89,7 +89,8 @@ __device__ __forceinline__ void stage_out(E* __restrict__ dst, const E* __restri
   }
 }
 
-template <bool SHARED, typename T>
+// PACK: the sample side is K2's loss pack (load_pack_item, ppo_loss.cuh), else the five leaves.
+template <bool SHARED, typename T, bool PACK>
 __global__ void __launch_bounds__(256, 2) ppo_loss_gaussian_kernel(const __grid_constant__ GaussianParams q) {
   // [256 * D] mean of T, [256 * D] action floats (, [256 * D] log_std of T per row), then the mbarrier; every block is a
   // multiple of 16 bytes
@@ -172,11 +173,16 @@ __global__ void __launch_bounds__(256, 2) ppo_loss_gaussian_kernel(const __grid_
       const int t = static_cast<int>(i / p.n);
       const int j = static_cast<int>(i - static_cast<long long>(t) * p.n);
       const int c = pr.lane_idx ? pr.lane_idx[j] : j;
-      const long long os = t * p.ld_smp + c;
-      vp = to_float(ldg_stream(reinterpret_cast<const T*>(pr.v_pred) + i));
-      ol = __ldg(p.old_logp + os), rt = __ldg(p.ret + os), ad = __ldg(p.adv + os);
-      ov = h.clip_value ? __ldg(p.old_value + os) : 0.f;
-      valid = __ldg(p.reset_next + os) == 0;
+      if constexpr (PACK) {
+        vp = to_float(ldg_stream(reinterpret_cast<const T*>(pr.v_pred) + i));
+        load_pack_item(p, t, c, ol, ov, rt, ad, valid);
+      } else {
+        const long long os = t * p.ld_smp + c;
+        vp = to_float(ldg_stream(reinterpret_cast<const T*>(pr.v_pred) + i));
+        ol = __ldg(p.old_logp + os), rt = __ldg(p.ret + os), ad = __ldg(p.adv + os);
+        ov = h.clip_value ? __ldg(p.old_value + os) : 0.f;
+        valid = __ldg(p.reset_next + os) == 0;
+      }
     }
     if (bulk) {
       tma::mbar_wait(bar, parity);
@@ -317,13 +323,13 @@ __global__ void __launch_bounds__(256, 2) ppo_loss_gaussian_kernel(const __grid_
   }
 }
 
-// one resident wave of ppo_loss_gaussian_kernel<SHARED, T> over the T * n transitions of q
-template <typename T>
+// one resident wave of ppo_loss_gaussian_kernel<SHARED, T, PACK> over the T * n transitions of q
+template <typename T, bool PACK>
 int launch_gaussian(const GaussianParams& q, bool shared, size_t smem, cudaStream_t stream) {
   int rc;
-  auto kern = shared ? ppo_loss_gaussian_kernel<true, T> : ppo_loss_gaussian_kernel<false, T>;
-  if ((rc = opt_in_smem<ppo_loss_gaussian_kernel<true, T>>(200 * 1024)) != SRL_OK) return rc;
-  if ((rc = opt_in_smem<ppo_loss_gaussian_kernel<false, T>>(200 * 1024)) != SRL_OK) return rc;
+  auto kern = shared ? ppo_loss_gaussian_kernel<true, T, PACK> : ppo_loss_gaussian_kernel<false, T, PACK>;
+  if ((rc = opt_in_smem<ppo_loss_gaussian_kernel<true, T, PACK>>(200 * 1024)) != SRL_OK) return rc;
+  if ((rc = opt_in_smem<ppo_loss_gaussian_kernel<false, T, PACK>>(200 * 1024)) != SRL_OK) return rc;
   const long long tiles = (static_cast<long long>(q.s.T) * q.s.n + 255) / 256;
   // ONE resident wave, as srl_ppo_loss_from_logits sizes its grid: as many CTAs as the SMs hold at once with this much
   // shared memory, at most kMaxGrid.  With a shared log_std this is also what makes CTA 0's wait for the other CTAs' rows
@@ -341,26 +347,30 @@ int launch_gaussian(const GaussianParams& q, bool shared, size_t smem, cudaStrea
 }
 
 // srl_ppo_loss_from_gaussian (elem_bytes = 4) and srl_ppo_loss_from_gaussian_bf16 (elem_bytes = 2: mean, v_pred, g_mean,
-// g_value and a per-row log_std / g_log_std are bfloat16; a shared log_std and its gradient are float either way)
+// g_value and a per-row log_std / g_log_std are bfloat16; a shared log_std and its gradient are float either way), and
+// srl_ppo_loss_from_gaussian_pack (pack != NULL: the sample side is K2's pack, ld_smp its lanes, pack_row_lo the absolute
+// row of loss row 0; the five leaves are not read)
 int ppo_loss_from_gaussian(const char* fn, size_t elem_bytes, const void* mean, const void* log_std, int log_std_shared,
                            const float* action, int D, const void* v_pred, const float* old_logp, const float* old_value,
                            const float* ret, const float* adv, const uint8_t* on_reset_next, int64_t ld_smp,
-                           const int32_t* lane_idx, int T, int n, const double* norm_stats, const double* local_stats,
+                           const float* pack, int pack_row_lo, const int32_t* lane_idx, int T, int n, const double* norm_stats, const double* local_stats,
                            const double* popart_mean_std, const srl_ppo_hyper* hyper, void* g_mean, void* g_log_std,
                            void* g_value, float* logp_out, float* entropy_out, double* out, float* out_f32,
                            void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   SRL_REQUIRE(T >= 1 && n >= 1, SRL_ERR_INVALID_ARG, "%s: need T >= 1 and n >= 1 (got %d, %d)", fn, T, n);
   SRL_REQUIRE(D >= 1 && D <= kMaxD, SRL_ERR_INVALID_ARG, "%s: D=%d action dimensions outside [1, %d]", fn, D, kMaxD);
+  const void* pk = pack;  // the pack form reads no leaf: the pack stands in for the four in the null test
   const struct {
     const void* p;
     const char* name;
   } required[] = {{mean, "mean"},         {log_std, "log_std"},     {action, "action"},     {v_pred, "v_pred"},
-                  {old_logp, "old_logp"}, {ret, "ret"},             {adv, "adv"},           {on_reset_next, "on_reset_next"},
+                  {pk ? pk : old_logp, "old_logp"}, {pk ? pk : ret, "ret"}, {pk ? pk : adv, "adv"},
+                  {pk ? pk : on_reset_next, "on_reset_next"},
                   {norm_stats, "norm_stats"}, {local_stats, "local_stats"}, {g_mean, "g_mean"}, {g_log_std, "g_log_std"},
                   {g_value, "g_value"},   {workspace, "workspace"}};
   for (const auto& r : required) SRL_REQUIRE(r.p != nullptr, SRL_ERR_INVALID_ARG, "%s: null pointer %s", fn, r.name);
-  SRL_REQUIRE(ld_smp >= (lane_idx ? 1 : n), SRL_ERR_INVALID_ARG, "%s: ld_smp=%lld smaller than the row", fn,
-              static_cast<long long>(ld_smp));
+  SRL_REQUIRE(ld_smp >= (lane_idx ? 1 : n), SRL_ERR_INVALID_ARG, "%s: %s=%lld smaller than the row", fn,
+              pack ? "pack_lanes" : "ld_smp", static_cast<long long>(ld_smp));
   const bool shared = log_std_shared != 0;
   const size_t need = srl_ppo_loss_gaussian_workspace_bytes(T, n, D, log_std_shared);
   SRL_REQUIRE(workspace_bytes >= need, SRL_ERR_INVALID_ARG, "%s: workspace too small (%zu bytes, need %zu)", fn,
@@ -368,7 +378,8 @@ int ppo_loss_from_gaussian(const char* fn, size_t elem_bytes, const void* mean, 
   GaussianParams q;
   int rc = fill_loss_hyper(hyper, popart_mean_std, q.s.h);
   if (rc != SRL_OK) return rc;
-  SRL_REQUIRE(!(q.s.h.clip_value && old_value == nullptr), SRL_ERR_INVALID_ARG, "%s: clip_value needs old_value", fn);
+  SRL_REQUIRE(pack || !(q.s.h.clip_value && old_value == nullptr), SRL_ERR_INVALID_ARG, "%s: clip_value needs old_value",
+              fn);
   const size_t blk_bytes = static_cast<size_t>(256) * D * elem_bytes;  // one dense [256, D] block of the element type
   const size_t act_bytes = static_cast<size_t>(256) * D * sizeof(float);  // the [256, D] action block
   const size_t smem = (shared ? 1 : 2) * blk_bytes + act_bytes + 16;     // + the mbarrier of the bulk copies
@@ -390,11 +401,11 @@ int ppo_loss_from_gaussian(const char* fn, size_t elem_bytes, const void* mean, 
   p.ret = ret;
   p.adv = adv;
   p.reset_next = on_reset_next;
-  p.pack = nullptr;
+  p.pack = reinterpret_cast<const float4*>(pack);
   p.lane_aos = nullptr;
   p.part = nullptr;
   p.part_ctas = p.part_first = 0;
-  p.row_lo = 0;
+  p.row_lo = pack ? pack_row_lo : 0;
   p.popart = popart_mean_std;
   p.ld_pol = n;
   p.ld_grad = n;
@@ -414,8 +425,11 @@ int ppo_loss_from_gaussian(const char* fn, size_t elem_bytes, const void* mean, 
   pr.out = out;
   pr.out_f32 = out_f32;
   pr.slot = reinterpret_cast<SlotHeader*>(workspace);
-  if (elem_bytes == sizeof(__nv_bfloat16)) return launch_gaussian<__nv_bfloat16>(q, shared, smem, stream);
-  return launch_gaussian<float>(q, shared, smem, stream);
+  const bool bf16 = elem_bytes == sizeof(__nv_bfloat16);
+  if (pack) return bf16 ? launch_gaussian<__nv_bfloat16, true>(q, shared, smem, stream)
+                        : launch_gaussian<float, true>(q, shared, smem, stream);
+  return bf16 ? launch_gaussian<__nv_bfloat16, false>(q, shared, smem, stream)
+              : launch_gaussian<float, false>(q, shared, smem, stream);
 }
 
 }  // namespace
@@ -438,7 +452,7 @@ extern "C" int srl_ppo_loss_from_gaussian(const float* mean, const float* log_st
                                           size_t workspace_bytes, srl_stream_t stream) {
   return srl::loss::ppo_loss_from_gaussian("srl_ppo_loss_from_gaussian", sizeof(float), mean, log_std, log_std_shared,
                                            action, D, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp,
-                                           lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_mean,
+                                           nullptr, 0, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_mean,
                                            g_log_std, g_value, logp_out, entropy_out, out, out_f32, workspace,
                                            workspace_bytes, static_cast<cudaStream_t>(stream));
 }
@@ -454,7 +468,30 @@ extern "C" int srl_ppo_loss_from_gaussian_bf16(const uint16_t* mean, const void*
                                                size_t workspace_bytes, srl_stream_t stream) {
   return srl::loss::ppo_loss_from_gaussian("srl_ppo_loss_from_gaussian_bf16", sizeof(__nv_bfloat16), mean, log_std,
                                            log_std_shared, action, D, v_pred, old_logp, old_value, ret, adv,
-                                           on_reset_next, ld_smp, lane_idx, T, n, norm_stats, local_stats,
+                                           on_reset_next, ld_smp, nullptr, 0, lane_idx, T, n, norm_stats, local_stats,
                                            popart_mean_std, hyper, g_mean, g_log_std, g_value, logp_out, entropy_out, out,
                                            out_f32, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int srl_ppo_loss_from_gaussian_pack(const void* mean, const void* log_std, int log_std_shared, const float* action,
+                                               int D, int elem_bytes, const void* v_pred, const float* pack,
+                                               int64_t pack_lanes, int pack_row_lo, const int32_t* lane_idx, int T, int n,
+                                               const double* norm_stats, const double* local_stats,
+                                               const double* popart_mean_std, const srl_ppo_hyper* hyper, void* g_mean,
+                                               void* g_log_std, void* g_value, float* logp_out, float* entropy_out,
+                                               double* out, float* out_f32, void* workspace, size_t workspace_bytes,
+                                               srl_stream_t stream) {
+  using namespace srl;
+  constexpr const char* fn = "srl_ppo_loss_from_gaussian_pack";
+  SRL_REQUIRE(elem_bytes == 4 || elem_bytes == 2, SRL_ERR_INVALID_ARG, "%s: elem_bytes=%d, need 4 (float32) or 2 (bfloat16)",
+              fn, elem_bytes);
+  SRL_REQUIRE(pack != nullptr && aligned(pack, 16), SRL_ERR_INVALID_ARG, "%s: pack is null or not 16-byte aligned", fn);
+  SRL_REQUIRE(pack_row_lo >= 0, SRL_ERR_INVALID_ARG, "%s: pack_row_lo=%d < 0", fn, pack_row_lo);
+  SRL_REQUIRE(lane_idx != nullptr || pack_lanes >= n, SRL_ERR_INVALID_ARG,
+              "%s: pack_lanes=%lld < n=%d without lane_idx", fn, static_cast<long long>(pack_lanes), n);
+  return srl::loss::ppo_loss_from_gaussian(fn, static_cast<size_t>(elem_bytes), mean, log_std, log_std_shared, action, D,
+                                           v_pred, nullptr, nullptr, nullptr, nullptr, nullptr, pack_lanes, pack,
+                                           pack_row_lo, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper,
+                                           g_mean, g_log_std, g_value, logp_out, entropy_out, out, out_f32, workspace,
+                                           workspace_bytes, static_cast<cudaStream_t>(stream));
 }

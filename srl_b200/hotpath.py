@@ -362,6 +362,56 @@ class HotPath:
                                     local_stats=self.local_stats[row], popart_mean_std=self.popart_mean_std(),
                                     lane_idx=idx, grads=self.grads[e][j], workspace=self.workspace[k], defer=True)
 
+    def loss_from_logits(self, e: int, j: int, logits: torch.Tensor, action: torch.Tensor, head_sizes, v_pred: torch.Tensor,
+                         available: Optional[torch.Tensor] = None):
+        """K4b for minibatch (e, j) in deferred mode, the head twin of loss(): the categorical head's logits
+        `[T, n_mb, sum K]`, int32 actions `[T, n_mb, heads]` and v_pred `[T, n_mb]` (float32 or bfloat16, both the same),
+        optionally SMAC's availability mask.  Gradients now, loss scalars + stats at finalize().  Returns (g_logits,
+        g_value) in the inputs' dtype."""
+        g_logits, g_value, _, _, _, _ = ops.ppo_loss_from_logits(
+            logits, action, head_sizes, v_pred, hyper=self.hyper, available=available, defer=True,
+            workspace=self.workspace[e * self.minibatches + j], **self._head_common(e, j))
+        return g_logits, g_value
+
+    def loss_from_gaussian(self, e: int, j: int, mean: torch.Tensor, log_std: torch.Tensor, action: torch.Tensor,
+                           v_pred: torch.Tensor):
+        """K4c for minibatch (e, j) in deferred mode, the head twin of loss(): mean and float32 actions `[T, n_mb, D]`,
+        log_std `[D]` (shared) or `[T, n_mb, D]`, v_pred `[T, n_mb]`.  Gradients now, loss scalars + stats at finalize().
+        Returns (g_mean, g_log_std, g_value) in the inputs' dtypes."""
+        shared = log_std.dim() == 1
+        self._gaussian_slots(mean.shape[-1], shared)
+        g_mean, g_log_std, g_value, _, _, _, _ = ops.ppo_loss_from_gaussian(
+            mean, log_std, action, v_pred, hyper=self.hyper, defer=True, workspace=self.workspace[e * self.minibatches + j],
+            **self._head_common(e, j))
+        return g_mean, g_log_std, g_value
+
+    def _head_common(self, e: int, j: int) -> dict:
+        """Statistics rows and sample side of a head loss for minibatch (e, j): K2's pack where this step's scan wrote it
+        and the minibatch is permuted, the leaves through lane_idx otherwise (one minibatch, cached advantages,
+        fuse_gather=False)."""
+        self._join_stats()  # the per-minibatch launch reads its statistics from the table
+        lo, hi = self.row_lo, self.row_hi
+        row = self.stats_row(e, j)
+        idx = self.minibatch_lanes(e, j)
+        kw = dict(norm_stats=self.global_stats[row], local_stats=self.local_stats[row],
+                  popart_mean_std=self.popart_mean_std(), lane_idx=idx)
+        if idx is not None and self.pack is not None and self.pack_valid:
+            kw.update(old_logp=None, old_value=None, ret=None, adv=None, on_reset_next=None, pack=self.pack, pack_row_lo=lo)
+        else:
+            lf = self.leaf
+            kw.update(old_logp=lf["old_logp"][lo:hi], old_value=lf["value"][lo:hi], ret=self.ret[lo:hi],
+                      adv=self.adv[lo:hi], on_reset_next=lf["on_reset"][lo + 1:hi + 1])
+        return kw
+
+    def _gaussian_slots(self, D: int, shared: bool) -> None:
+        """A shared log_std's partial rows follow the K4 slot (srl_ppo_loss_gaussian_workspace_bytes): widen every slot once
+        so that one loss_finalize still folds them all.  Slots already written keep their bytes."""
+        need = ops.gaussian_loss_workspace_bytes(self.T, self.n_mb, D, shared)
+        old = self.workspace
+        if need > old.shape[1]:
+            self.workspace = torch.zeros((old.shape[0], need), dtype=torch.uint8, device=self.device)
+            self.workspace[:, :old.shape[1]].copy_(old)
+
     def _problem(self, e: int, j: int, new_logp, v_pred, entropy, deferred: bool) -> dict:
         row = self.stats_row(e, j)
         k = e * self.minibatches + j

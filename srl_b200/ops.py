@@ -458,6 +458,29 @@ def _sample_side(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, c
     return ld
 
 
+def _sample_side_or_pack(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, clip_value, pack, pack_row_lo):
+    """The head losses' sample side: the five leaf views (_sample_side) or, with `pack`, K2's pack; returns ld_smp / the
+    pack's lanes."""
+    if pack is None:
+        return _sample_side(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, clip_value)
+    if lane_idx is not None:
+        _check(lane_idx, torch.int32, "lane_idx")
+        if lane_idx.numel() != n:
+            raise ValueError(f"lane_idx has {lane_idx.numel()} entries, policy side has {n} lanes")
+    return _pack_side(pack, int(pack_row_lo), T, n, lane_idx is not None)
+
+
+def _pack_side(pack, pack_row_lo: int, T: int, n: int, has_idx: bool) -> int:
+    """Validates K2's pack as a loss's sample side (rows [pack_row_lo, pack_row_lo + T)); returns its lanes N."""
+    _check(pack, torch.float32, "pack")
+    if pack.dim() != 4 or pack.shape[2:] != (2, 4) or 2 * pack.shape[0] < pack_row_lo + T or pack_row_lo < 0:
+        raise ValueError(f"pack: expected K2's [ceil(L/2), N, 2, 4] float32 pack holding rows [{pack_row_lo}, "
+                         f"{pack_row_lo + T}), got shape {tuple(pack.shape)}")
+    if not has_idx and pack.shape[1] != n:
+        raise ValueError(f"pack has {pack.shape[1]} lanes but the policy side has {n}")
+    return pack.shape[1]
+
+
 def ppo_loss_fwd_bwd(new_logp, v_pred, entropy, old_logp, old_value, ret, adv, on_reset_next, norm_stats, hyper: LossHyper,
                      local_stats=None, popart_mean_std=None, lane_idx=None, grads=None, out=None, out_f32=None,
                      workspace=None, defer: bool = False):
@@ -556,13 +579,7 @@ def ppo_loss_batched(problems: Sequence[dict], old_logp, old_value, ret, adv, on
                              _ptr(ls), _ptr(q["grads"][0]), _ptr(q["grads"][1]), _ptr(q["grads"][2]), _ptr(out),
                              _ptr(out_f32), _ptr(ws))
     if pack is not None:
-        _check(pack, torch.float32, "pack")
-        if pack.dim() != 4 or pack.shape[2:] != (2, 4) or 2 * pack.shape[0] < pack_row_lo + T or pack_row_lo < 0:
-            raise ValueError(f"pack: expected K2's [ceil(L/2), N, 2, 4] float32 pack holding rows [{pack_row_lo}, "
-                             f"{pack_row_lo + T}), got shape {tuple(pack.shape)}")
-        ld_smp = pack.shape[1]
-        if not has_idx and pack.shape[1] != n:
-            raise ValueError(f"pack has {pack.shape[1]} lanes but the policy side has {n}")
+        ld_smp = _pack_side(pack, pack_row_lo, T, n, has_idx)
         old_logp = old_value = ret = adv = on_reset_next = None
     else:
         ld_smp = _sample_side(old_logp, old_value, ret, adv, on_reset_next, problems[0].get("lane_idx"), T, n,
@@ -609,7 +626,8 @@ def _availability(available, logits) -> torch.Tensor:
 
 def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_logp, old_value, ret, adv, on_reset_next,
                          norm_stats, hyper: LossHyper, local_stats=None, popart_mean_std=None, lane_idx=None,
-                         want_logp_entropy: bool = False, available=None, workspace=None, defer: bool = False):
+                         want_logp_entropy: bool = False, available=None, workspace=None, defer: bool = False,
+                         pack: Optional[torch.Tensor] = None, pack_row_lo: int = 0):
     """Loss starting from the actor head's logits `[T, n, sum K]` and int32 actions `[T, n, heads]`
     (actor_critic_policy.py:303-324 fused in).  Returns (g_logits, g_value, out, out_f32, logp, entropy).
 
@@ -620,7 +638,10 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     `available` (SMAC's available_action, the logits' shape): where it is 0 the logit is replaced by -1e10 before the
     Categorical (actor_critic_policy.py:135-136) and its gradient is 0.  torch.uint8 and torch.bool are read in place; a
     floating mask costs one extra pass (`available != 0`).  At most 159 logits per transition with a mask, 199 without.
-    `defer` (needs an explicit `workspace` slot): out / out_f32 are None and loss_finalize folds the slot later."""
+    `defer` (needs an explicit `workspace` slot): out / out_f32 are None and loss_finalize folds the slot later.
+    `pack` (K2's whole `[ceil(L/2), N, 2, 4]` pack, `new_pack`) with `pack_row_lo` = the sample row of loss row 0: the
+    sample side is read from it, one 16-byte item per transition (srl_ppo_loss_from_logits_pack), and the five sample leaves
+    may be None -- the results are those of the leaves the pack was written from, bit for bit."""
     if available is not None:
         available = _availability(available, logits)
     dtype = logits.dtype if isinstance(logits, torch.Tensor) else torch.float32
@@ -643,7 +664,8 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     n = logits[0].numel() // SK
     if _rows_lanes(v_pred) != (T, n) or action.numel() != T * n * heads:
         raise ValueError("logits, action and v_pred disagree on [T, n]")
-    ld_smp = _sample_side(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, hyper.clip_value)
+    ld_smp = _sample_side_or_pack(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, hyper.clip_value, pack,
+                                  pack_row_lo)
     _check(norm_stats, torch.float64, "norm_stats")
     local_stats = norm_stats if local_stats is None else _check(local_stats, torch.float64, "local_stats")
     dev = logits.device
@@ -661,9 +683,14 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     ws = loss_workspace(dev) if workspace is None else _check(workspace, torch.uint8, "workspace")
     hc = hyper.to_c()
     hs = (ctypes.c_int32 * heads)(*[int(k) for k in head_sizes])
-    tail = (hs, heads, _ptr(v_pred), _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp,
-            _ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
+    rest = (_ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
             _ptr(g_logits), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws), ws.numel(), _stream())
+    if pack is not None:
+        _lib.call("srl_ppo_loss_from_logits_pack", _ptr(logits), logits.element_size(), _ptr(available), _ptr(action), hs,
+                  heads, _ptr(v_pred), _ptr(pack), ld_smp, int(pack_row_lo), *rest)
+        return g_logits, g_value, out, out_f32, logp, ent
+    tail = (hs, heads, _ptr(v_pred), _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next),
+            ld_smp) + rest
     suffix = "_bf16" if dtype == torch.bfloat16 else ""
     if available is None:
         _lib.call("srl_ppo_loss_from_logits" + suffix, _ptr(logits), _ptr(action), *tail)
@@ -698,7 +725,8 @@ def gaussian_loss_workspace(device) -> torch.Tensor:
 
 def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, ret, adv, on_reset_next, norm_stats,
                            hyper: LossHyper, local_stats=None, popart_mean_std=None, lane_idx=None,
-                           want_logp_entropy: bool = False, workspace=None, defer: bool = False):
+                           want_logp_entropy: bool = False, workspace=None, defer: bool = False,
+                           pack: Optional[torch.Tensor] = None, pack_row_lo: int = 0):
     """Loss starting from a diagonal-Gaussian actor head: `mean` and float32 `action` `[T, n, D]`, `log_std` either
     `[T, n, D]` (one per transition) or `[D]` (one parameter shared by every transition), D <= 64.  The head's log-prob
     and entropy are torch.distributions.Normal(mean, log_std.exp()).log_prob(action).sum(-1) / .entropy().sum(-1); the
@@ -714,7 +742,8 @@ def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, r
     (an nn.Parameter, which autocast leaves alone) or bfloat16 (a module cast with .bfloat16()) with either mean dtype:
     it is widened (D elements), its gradient is summed in float64 as always, and comes back float32 or rounded to
     bfloat16 once, in log_std's dtype.  `action` is float32 always: the actions the actors sampled, on which old_logp
-    was computed."""
+    was computed.  `pack` / `pack_row_lo`: the sample side from K2's pack, as in ppo_loss_from_logits (the five sample
+    leaves may then be None)."""
     dtype = mean.dtype if isinstance(mean, torch.Tensor) else torch.float32
     if dtype not in (torch.float32, torch.bfloat16):
         raise ValueError(f"mean: expected dtype torch.float32 or torch.bfloat16, got {dtype}")
@@ -758,7 +787,8 @@ def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, r
     ls_dtype = log_std.dtype
     if shared and ls_dtype == torch.bfloat16:
         log_std = log_std.float()
-    ld_smp = _sample_side(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, hyper.clip_value)
+    ld_smp = _sample_side_or_pack(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, hyper.clip_value, pack,
+                                  pack_row_lo)
     _check(norm_stats, torch.float64, "norm_stats")
     local_stats = norm_stats if local_stats is None else _check(local_stats, torch.float64, "local_stats")
     if popart_mean_std is not None:
@@ -778,12 +808,16 @@ def ppo_loss_from_gaussian(mean, log_std, action, v_pred, old_logp, old_value, r
         out_f32 = torch.empty(4, dtype=torch.float32, device=dev)
     ws = gaussian_loss_workspace(dev) if workspace is None else _check(workspace, torch.uint8, "workspace")
     hc = hyper.to_c()
-    suffix = "_bf16" if dtype == torch.bfloat16 else ""
-    _lib.call("srl_ppo_loss_from_gaussian" + suffix, _ptr(mean), _ptr(log_std), int(shared), _ptr(action), D,
-              _ptr(v_pred), _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp,
-              _ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
-              _ptr(g_mean), _ptr(g_log_std), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws),
-              ws.numel(), _stream())
+    tail = (_ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
+            _ptr(g_mean), _ptr(g_log_std), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws),
+            ws.numel(), _stream())
+    if pack is not None:
+        _lib.call("srl_ppo_loss_from_gaussian_pack", _ptr(mean), _ptr(log_std), int(shared), _ptr(action), D,
+                  mean.element_size(), _ptr(v_pred), _ptr(pack), ld_smp, int(pack_row_lo), *tail)
+    else:
+        suffix = "_bf16" if dtype == torch.bfloat16 else ""
+        _lib.call("srl_ppo_loss_from_gaussian" + suffix, _ptr(mean), _ptr(log_std), int(shared), _ptr(action), D,
+                  _ptr(v_pred), _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp, *tail)
     if g_log_std.dtype != ls_dtype:
         g_log_std = g_log_std.to(ls_dtype)  # what autograd's cast hands a bfloat16 parameter through .float()
     return g_mean, g_log_std, g_value, out, out_f32, logp, ent

@@ -10,7 +10,11 @@ After that an experiment selects it exactly like the stock trainer (legacy/exper
 Nothing else in SRL changes: `api.trainer.make` builds the policy and calls `cls(policy=policy, **cfg.args)`
 (api/trainer.py:238-246); `GPUThread` calls `trainer.distributed(...)` once and `trainer.step(sample)` in a loop
 (distributed/system/trainer_worker.py:94,171).
+
+A policy trained through the fused head losses declares `ppo_head = True` and returns
+`srl_b200.srl_plugin.PPOHeadAnalyzedResult` from `analyze(..., target="ppo_head")` (INTEGRATION.md).
 """
+from srl_b200.api import PPOHeadAnalyzedResult  # noqa: F401  (the record a `ppo_head` policy returns)
 from srl_b200.postprocess import TrajGAEB200
 from srl_b200.trainer import MultiAgentPPOB200
 

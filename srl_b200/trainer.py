@@ -21,7 +21,7 @@ The policy network, its optimizer, gradient clipping and DDP stay PyTorch (cuBLA
 from __future__ import annotations
 
 from collections import defaultdict
-from typing import Dict, Optional
+from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 import torch
@@ -29,7 +29,7 @@ import torch.distributed as dist
 import torch.nn as nn
 
 from srl_b200 import ops
-from srl_b200.api import PytorchTrainer, TrainerStepResult, register
+from srl_b200.api import PPOHeadAnalyzedResult, PytorchTrainer, TrainerStepResult, register
 from srl_b200.hotpath import HotPath
 from srl_b200.namedarray import flatten, from_flattened, record_class, recursive_apply
 
@@ -146,6 +146,12 @@ class MultiAgentPPOB200(PytorchTrainer):
         self.copy_threads = int(kwargs.get("copy_threads", 8))  # host threads filling the pinned staging blocks
         if self.vtrace and (self.num_minibatches > 1 or self.recompute_adv_among_epochs):
             raise ValueError("vtrace supports num_minibatches == 1 without recompute_adv_among_epochs")
+        # A policy that declares `ppo_head = True` hands over its actor head (api.PPOHeadAnalyzedResult) and trains through
+        # the fused head losses K4b / K4c; every other policy takes the `target="ppo"` path.
+        self.ppo_head = getattr(policy, "ppo_head", False) is True
+        if self.ppo_head and self.vtrace:
+            raise ValueError("vtrace=True needs the policy's new log-probabilities before the GAE scan, and a `ppo_head` "
+                             "policy returns its actor head instead; train V-trace with target='ppo' (no ppo_head)")
         self.frames = 0
         self._hp: Optional[HotPath] = None
         self._pending = None  # (host sample, device float sample) staged by the previous step() call
@@ -286,7 +292,8 @@ class MultiAgentPPOB200(PytorchTrainer):
                 mb = whole if idx is None else self._float_view(self._gather_minibatch(tensor_sample, idx, hp))
                 # mappo.py:243-246
                 tail_len = 1 if (self.vtrace and not cached_adv and not have_adv) else self.bootstrap_steps
-                res = self.policy.analyze(mb[:L - tail_len], target="ppo", burn_in_steps=self.burn_in_steps)
+                res = self.policy.analyze(mb[:L - tail_len], target="ppo_head" if self.ppo_head else "ppo",
+                                          burn_in_steps=self.burn_in_steps)
                 if not have_adv:  # mappo.py:249-257
                     vt = None
                     if self.vtrace and not cached_adv:
@@ -299,11 +306,14 @@ class MultiAgentPPOB200(PytorchTrainer):
                 if self._popart and j == 0:  # once per epoch, before the loss (mappo.py:263-264)
                     hp.update_popart()
                     self._popart.push(hp)
-                nl, vp, en = (x[:T].reshape(T, -1) for x in (res.new_action_log_probs, res.state_values, res.entropy))
-                g_lp, g_v, g_en, _, _ = hp.loss(e, j, nl.detach().contiguous(), vp.detach().contiguous(),
-                                                en.detach().contiguous())
+                if self.ppo_head:
+                    outs = self._head_loss(hp, e, j, res)
+                else:
+                    nl, vp, en = (x[:T].reshape(T, -1) for x in (res.new_action_log_probs, res.state_values, res.entropy))
+                    g_lp, g_v, g_en, _, _ = hp.loss(e, j, nl.detach().contiguous(), vp.detach().contiguous(),
+                                                    en.detach().contiguous())
+                    outs = [(o, g) for o, g in ((nl, g_lp), (vp, g_v), (en, g_en)) if o.requires_grad]
                 self.optimizer.zero_grad(set_to_none=True)  # mappo.py:273-274: loss.backward()
-                outs = [(o, g) for o, g in ((nl, g_lp), (vp, g_v), (en, g_en)) if o.requires_grad]
                 torch.autograd.backward([o for o, _ in outs], [g for _, g in outs])
                 if self.max_grad_norm is not None:  # mappo.py:280-284
                     gn = nn.utils.clip_grad_norm_(self.policy.parameters(), self.max_grad_norm)
@@ -365,6 +375,28 @@ class MultiAgentPPOB200(PytorchTrainer):
         return TrainerStepResult(stats=stats, step=self.policy.version)
 
     # ----------------------------------------------------------------------------------------------------
+    def _head_loss(self, hp: HotPath, e: int, j: int, res) -> List[Tuple[torch.Tensor, torch.Tensor]]:
+        """K4b / K4c for minibatch (e, j) on the head a `ppo_head` policy returned: [(output, d loss / d output)] for the
+        outputs that require grad (the loss scalars follow at hp.finalize())."""
+        h = _head_fields(res, hp.T, hp.n_mb)
+        T, n = hp.T, hp.n_mb
+        vp = h.state_values[:T].reshape(T, n)
+        if h.logits is not None:
+            lg = h.logits[:T].reshape(T, n, -1)
+            act = h.action[:T].reshape(T, n, -1).to(torch.int32).contiguous()
+            av = None if h.available is None else h.available[:T].reshape(T, n, -1).contiguous()
+            g_lg, g_v = hp.loss_from_logits(e, j, lg.detach().contiguous(), act, [int(k) for k in h.head_sizes],
+                                            vp.detach().contiguous(), av)
+            pairs = ((lg, g_lg), (vp, g_v))
+        else:
+            mu = h.mean[:T].reshape(T, n, -1)
+            ls = h.log_std if h.log_std.dim() == 1 else h.log_std[:T].reshape(T, n, -1)
+            act = h.action[:T].reshape(T, n, -1).contiguous()
+            g_mu, g_ls, g_v = hp.loss_from_gaussian(e, j, mu.detach().contiguous(), ls.detach().contiguous(), act,
+                                                    vp.detach().contiguous())
+            pairs = ((mu, g_mu), (ls, g_ls), (vp, g_v))
+        return [(o, g) for o, g in pairs if o.requires_grad]
+
     def _host_mirror(self, hp: HotPath) -> Dict[str, torch.Tensor]:
         """Pinned host images of what a step reports, allocated once per batch shape."""
         key = (hp.L, hp.N, hp.epochs, hp.minibatches)
@@ -406,6 +438,69 @@ class MultiAgentPPOB200(PytorchTrainer):
             names.append((name, dst))
         ops.batch_gather(pairs, env_idx)
         return from_flattened(names, record_class(tensor_sample))
+
+
+_HEAD_FLOATS = (torch.float32, torch.bfloat16)
+
+
+def _head_fields(res, T: int, n: int) -> PPOHeadAnalyzedResult:
+    """Checks what analyze(target="ppo_head") returned against the contract of api.PPOHeadAnalyzedResult for T loss rows of
+    n lanes; raises TypeError / ValueError naming the field."""
+    if not isinstance(res, PPOHeadAnalyzedResult):
+        raise TypeError(f"analyze(target='ppo_head') must return srl_b200.api.PPOHeadAnalyzedResult, got {type(res).__name__}")
+
+    def tensor(name, required=True):
+        x = getattr(res, name)
+        if x is None and not required:
+            return None
+        if x is None:
+            raise ValueError(f"PPOHeadAnalyzedResult.{name} is required")
+        if not isinstance(x, torch.Tensor):
+            raise TypeError(f"PPOHeadAnalyzedResult.{name}: expected a torch.Tensor, got {type(x).__name__}")
+        return x
+
+    sv, act = tensor("state_values"), tensor("action")
+    if sv.dtype not in _HEAD_FLOATS:
+        raise ValueError(f"PPOHeadAnalyzedResult.state_values: dtype {sv.dtype}, expected torch.float32 or torch.bfloat16")
+    if sv.dim() < 2 or sv.shape[-1] != 1 or sv.shape[0] < T or sv[0].numel() != n:
+        raise ValueError(f"PPOHeadAnalyzedResult.state_values: expected [T', B, (A,) 1] with T' >= {T} rows of {n} lanes, "
+                         f"got shape {tuple(sv.shape)}")
+    lead = tuple(sv.shape[:-1])
+    if (res.logits is None) == (res.mean is None):
+        raise ValueError("PPOHeadAnalyzedResult: set exactly one of `logits` (categorical head) and `mean` (Gaussian head)")
+    if res.logits is not None:
+        lg = tensor("logits")
+        if lg.dtype != sv.dtype:
+            raise ValueError(f"PPOHeadAnalyzedResult.logits: dtype {lg.dtype} differs from state_values' {sv.dtype}")
+        if res.head_sizes is None:
+            raise ValueError("PPOHeadAnalyzedResult.head_sizes is required with logits")
+        hs = [int(k) for k in res.head_sizes]
+        if tuple(lg.shape[:-1]) != lead or lg.shape[-1] != sum(hs):
+            raise ValueError(f"PPOHeadAnalyzedResult.logits: expected {lead + (sum(hs),)} (state_values' rows and lanes, "
+                             f"sum of head_sizes {hs}), got {tuple(lg.shape)}")
+        if act.dtype == torch.bool or act.dtype.is_complex or tuple(act.shape) != lead + (len(hs),):
+            raise ValueError(f"PPOHeadAnalyzedResult.action: expected integer-valued {lead + (len(hs),)}, got "
+                             f"{act.dtype} {tuple(act.shape)}")
+        av = tensor("available", required=False)
+        if av is not None and tuple(av.shape) != tuple(lg.shape):
+            raise ValueError(f"PPOHeadAnalyzedResult.available: shape {tuple(av.shape)} differs from logits' "
+                             f"{tuple(lg.shape)}")
+    else:
+        mu, ls = tensor("mean"), tensor("log_std")
+        if mu.dtype != sv.dtype:
+            raise ValueError(f"PPOHeadAnalyzedResult.mean: dtype {mu.dtype} differs from state_values' {sv.dtype}")
+        if mu.dim() != len(lead) + 1 or tuple(mu.shape[:-1]) != lead:
+            raise ValueError(f"PPOHeadAnalyzedResult.mean: expected {lead + ('D',)}, got {tuple(mu.shape)}")
+        D = mu.shape[-1]
+        if tuple(ls.shape) != (D,) and tuple(ls.shape) != tuple(mu.shape):
+            raise ValueError(f"PPOHeadAnalyzedResult.log_std: expected [{D}] or the mean's {tuple(mu.shape)}, got "
+                             f"{tuple(ls.shape)}")
+        if ls.dim() > 1 and ls.dtype != mu.dtype:
+            raise ValueError(f"PPOHeadAnalyzedResult.log_std: dtype {ls.dtype} differs from mean's {mu.dtype}")
+        if act.dtype != torch.float32 or tuple(act.shape) != tuple(mu.shape):
+            raise ValueError(f"PPOHeadAnalyzedResult.action: expected float32 {tuple(mu.shape)}, got {act.dtype} "
+                             f"{tuple(act.shape)}")
+    return res
 
 
 register("mappo_b200", MultiAgentPPOB200)
