@@ -71,7 +71,8 @@ int srl_device_info(int* sm_count, int* cc_major, int* cc_minor);
  *
  * pack (optional, may be NULL; needs old_logp): the sample side of the loss as ONE 16-byte item per transition,
  * {old_logp[t], value[t] (as stored in the sample), ret[t], mask[t] ? adv[t] : NaN} with mask[t] = 1 - on_reset[t+1]
- * (row L-1: NaN), the two rows of a row pair next to each other: item (t, lane) is float4 number
+ * (row L-1: NaN).  With V-trace the first column is vtrace_old_logp[t] for rows 0..L-2 and 0 in row L-1, and old_logp is
+ * not read (it must still be non-NULL).  The two rows of a row pair sit next to each other: item (t, lane) is float4 number
  * ((t / 2) * N + lane) * 2 + t % 2, i.e. float32 [ceil(L / 2), N, 2, 4] (so the buffer holds L + L % 2 rows), 32-byte
  * aligned.  A minibatch that gathers lanes through a permutation (srl_ppo_loss_fwd_bwd_batched, `pack`) then issues one
  * 256-bit load per lane and ROW PAIR -- every 32-byte sector it touches is used whole -- instead of five narrow loads per

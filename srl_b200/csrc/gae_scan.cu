@@ -22,11 +22,13 @@ namespace {
 constexpr int kThreads = 256;
 constexpr size_t kSmemBudget = 200 * 1024;
 
+// (delta, m) (2 x f64, interleaved) + adv (f32) + v' (f32) + flags (u8) per cell; with the loss pack also old_logp and
+// the raw value (2 x f32)
+__host__ __device__ constexpr size_t gae_cell_bytes(bool pack) { return 16 + 4 + 4 + 1 + (pack ? 8 : 0); }
+
 __host__ __device__ constexpr size_t gae_smem_bytes(int L, int LW, bool pack) {
-  // (delta, m) (2 x f64, interleaved) + adv (f32) + v' (f32) + flags (u8), each [L][LW]; with the loss pack also
-  // old_logp and the raw value (2 x f32)
-  // (the per-lane reduction scratch [kThreads/LW][7][LW] f64 = 14 KB aliases the same bytes)
-  const size_t tile = static_cast<size_t>(L) * LW * (16 + 4 + 4 + 1 + (pack ? 8 : 0));
+  // the tile is [L][LW] cells (the per-lane reduction scratch [kThreads/LW][7][LW] f64 = 14 KB aliases the same bytes)
+  const size_t tile = static_cast<size_t>(L) * LW * gae_cell_bytes(pack);
   const size_t scratch = static_cast<size_t>(kThreads) * 7 * 8;
   return tile > scratch ? tile : scratch;
 }
@@ -393,8 +395,8 @@ int gae_scan_impl(const float* reward, const float* value, const uint8_t* done, 
   if (const char* e = getenv("SRL_GAE_LW")) lw = atoi(e);  // tuning knob of the instrumented build only
 #endif
   SRL_REQUIRE(gae_smem_bytes(L, lw, with_pack) <= kSmemBudget, SRL_ERR_UNSUPPORTED,
-              "srl_gae_scan: L=%d does not fit the shared-memory tile (max L ~ %d)", L,
-              static_cast<int>(kSmemBudget / (8 * 25)));
+              "srl_gae_scan: L=%d does not fit the shared-memory tile (max L = %d%s)", L,
+              static_cast<int>(kSmemBudget / (8 * gae_cell_bytes(with_pack))), with_pack ? " with the loss pack" : "");
   if (vtrace) {
     if (lw == 32) return launch<32, true>(p, st);
     if (lw == 16) return launch<16, true>(p, st);
