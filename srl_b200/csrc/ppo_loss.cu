@@ -644,7 +644,7 @@ extern "C" int srl_ppo_loss_fwd_bwd_batched(const srl_loss_problem* problems, in
     if (mode == kPack && pair)
       rc = launch_loss_pair(b, nb, st);
     else if (mode == kPack)
-      rc = launch_loss_pack(b, nb, dense_ok, st);
+      rc = launch_loss_pack(b, nb, st);
     else if (mode == kDense)
       rc = launch_loss_dense(b, nb, dense_ok, st);
     else

@@ -639,7 +639,7 @@ int fill_loss_hyper(const srl_ppo_hyper* hyper, const double* popart_mean_std, L
 // defined in ppo_loss_dense.cu / ppo_loss_gather.cu / ppo_loss_pack.cu
 int launch_loss_dense(LossBatch& b, int n_problems, bool lanes4, cudaStream_t st);
 int launch_loss_gather(LossBatch& b, int n_problems, bool lanes4, cudaStream_t st);
-int launch_loss_pack(LossBatch& b, int n_problems, bool lanes4, cudaStream_t st);
+int launch_loss_pack(LossBatch& b, int n_problems, cudaStream_t st);
 // ppo_loss_pair.cu: the pack form for permuted minibatches of even width (two lanes x two rows per thread and step, the
 // loads of the next step in flight under the arithmetic of this one, units dealt evenly over a persistent grid)
 bool loss_pair_eligible(const LossShared& s, bool aligned8);

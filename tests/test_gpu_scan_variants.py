@@ -13,8 +13,6 @@ that reproduces the first bit for bit.
 import ctypes
 import dataclasses
 import re
-import shutil
-import subprocess
 import zlib
 from typing import Callable, Optional, Tuple, Union
 
@@ -23,12 +21,11 @@ import pytest
 import torch
 
 from oracle import ref_math as M
+from tests.kernel_variants import F64_SENTINEL, Guarded, launched, library_kernels
 
 GAMMA, LMBDA = 0.995, 0.9
 RHO, C = 1.0, 0.9  # V-trace clips: rho != c, and the ratios below straddle both
 SMEM_BUDGET = 200 * 1024  # gae_scan.cu kSmemBudget
-F32_SENTINEL = 0x7FA5A5A5  # signalling-NaN bit patterns no kernel writes
-F64_SENTINEL = 0x7FF4A5A5A5A5A5A5
 PACK_MASKED_ADV = 0x7FC00000  # gae_common.cuh kPackMaskedAdv
 
 
@@ -210,15 +207,7 @@ CROSS = ["tma-spec-pack-popart", "tma-general-pack-popart", "tma-vtrace-pack", "
 def test_case_table_names_every_scan_instantiation_in_the_library():
     """The set of gae_scan*_kernel instantiations in libsrl_b200.so (cuobjdump -symbols | cu++filt) is the set CASES names:
     an instantiation with no case, or a case naming one that does not exist, fails here."""
-    if shutil.which("cuobjdump") is None or shutil.which("cu++filt") is None:
-        pytest.skip("cuobjdump / cu++filt not available")
-    from srl_b200 import _lib, build
-    build.build()
-    sym = subprocess.run(["cuobjdump", "-symbols", _lib.lib_path()], capture_output=True, text=True)
-    if sym.returncode != 0:
-        pytest.skip("cuobjdump not available")
-    names = subprocess.run(["cu++filt"], input=sym.stdout, capture_output=True, text=True, check=True).stdout
-    built = {k for k in (kernel_id(line) for line in names.splitlines()) if k is not None}
+    built = library_kernels(kernel_id)
     assert len(built) == 36, sorted(built)
     named = {c.kernel for c in CASES.values()}
     assert built == named, f"in the library only: {sorted(built - named)}; in the table only: {sorted(named - built)}"
@@ -262,24 +251,6 @@ def _place(x: torch.Tensor, aligned: bool) -> torch.Tensor:
     return out
 
 
-class Guarded:
-    """An output as a view into a larger buffer: 256 bytes of sentinel on both sides (the view stays 256-byte aligned, so
-    routing does not change) and the view itself pre-filled with the sentinel."""
-
-    def __init__(self, shape, dtype):
-        self.n = int(np.prod(shape))
-        self.g = 256 // torch.empty((), dtype=dtype).element_size()
-        self.ity = torch.int32 if dtype == torch.float32 else torch.int64
-        self.sentinel = F32_SENTINEL if dtype == torch.float32 else F64_SENTINEL
-        self.buf = torch.empty(self.n + 2 * self.g, dtype=dtype, device="cuda")
-        self.buf.view(self.ity).fill_(self.sentinel)
-        self.t = self.buf[self.g:self.g + self.n].view(shape)
-
-    def guards_intact(self) -> bool:
-        b = self.buf.view(self.ity)
-        return bool((b[:self.g] == self.sentinel).all()) and bool((b[self.g + self.n:] == self.sentinel).all())
-
-
 def _inputs(name: str, case: Case, N: int) -> dict:
     """Seeded CPU inputs of a case; they depend on the name and shape only, not on the alignment."""
     g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
@@ -321,16 +292,6 @@ def _run(ops, case: Case, x: dict, N: int, aligned: bool, perm_job: Optional[dic
     if case.vtrace:  # the importance ratio as torch computes it on the device from the same float32 leaves
         out["ratio"] = (kw["vtrace_new_logp"] - kw["vtrace_old_logp"]).exp().cpu()
     return out
-
-
-def _launched(fn):
-    """fn()'s result and the gae_scan*_kernel instantiations it launched (kernel_id strings, from the CUDA profiler)."""
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        res = fn()
-        torch.cuda.synchronize()
-    return res, [k for k in (kernel_id(e.name) for e in prof.events()) if k is not None]
 
 
 def _oracle(case: Case, x: dict, ratio: Optional[torch.Tensor]):
@@ -411,8 +372,8 @@ def test_scan_variant_matches_oracle(ops, sms, name):
     want = expected_kernel(case.L, N, case.aligned, case.vtrace, case.popart, case.pack, sms)
     assert want == case.kernel, f"{name}: at {sms} SMs these inputs route to {want}, not {case.kernel}"
     x = _inputs(name, case, N)
-    out, launched = _launched(lambda: _run(ops, case, x, N, case.aligned))
-    assert launched and set(launched) == {case.kernel}, f"{name}: launched {launched}, expected {case.kernel}"
+    out, ran = launched(lambda: _run(ops, case, x, N, case.aligned), kernel_id)
+    assert ran and set(ran) == {case.kernel}, f"{name}: launched {ran}, expected {case.kernel}"
     _check_case(ops, case, x, out, name)
     again = _run(ops, case, x, N, case.aligned)
     torch.cuda.synchronize()
