@@ -491,6 +491,70 @@ int srl_ppo_loss_from_gaussian_pack(
     double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * K4d  Same loss, but starting from a Beta actor head (actions bounded to an interval, D = 1 .. 64 dimensions).
+ * NEW capability: no reference line pins this head; the definition is torch.distributions.Beta(c1, c0) with
+ * c1 = concentration1 (alpha) and c0 = concentration0 (beta), summed over the action dimensions, as any PyTorch Beta
+ * policy computes it (x in (0, 1), psi = digamma):
+ *   logp = sum_d [ (c1-1) log x + (c0-1) log(1-x) + lgamma(c1+c0) - lgamma(c1) - lgamma(c0) ]      (.log_prob(x).sum(-1))
+ *   H    = sum_d [ lgamma(c1) + lgamma(c0) - lgamma(c1+c0) - (c1-1) psi(c1) - (c0-1) psi(c0)
+ *                  + (c1+c0-2) psi(c1+c0) ]                                                          (.entropy().sum(-1))
+ * The loss, the ten outputs and the masking are K4's.  Writes
+ *   g_concentration1[i, d] = g_lp (log x - psi(c1) + psi(c1+c0)) + g_en ((c1+c0-2) psi'(c1+c0) - (c1-1) psi'(c1))
+ *   g_concentration0[i, d] = g_lp (log(1-x) - psi(c0) + psi(c1+c0)) + g_en ((c1+c0-2) psi'(c1+c0) - (c0-1) psi'(c0))
+ * with (g_lp, g_en) = d loss / d (logp, H) of transition i, and d loss / d v_pred.  The per-dimension terms and their
+ * sums over d are float64 (lgamma(c1+c0) - lgamma(c1) - lgamma(c0) cancels for large concentrations); logp and H are
+ * rounded to float32 once, each gradient once.  The actions are the float32 samples in the open interval (0, 1) (a
+ * policy maps them to its action bounds itself) and the concentrations are positive; neither is checked on the device.
+ * An action outside (0, 1) gives what torch's formula gives; a concentration that is not positive (or NaN) gives NaN
+ * psi / psi' terms, so that transition's entropy and gradients are NaN (torch's digamma would evaluate a negative
+ * argument) -- the launch ends either way, and a NaN transition makes the statistics NaN.  The workspace (zero before first use, left zero) is one
+ * K4 slot of srl_ppo_loss_workspace_bytes(T, n) bytes, so out == NULL followed by srl_ppo_loss_finalize works as for
+ * srl_ppo_loss_fwd_bwd.  D outside [1, 64] is an invalid argument.
+ * ------------------------------------------------------------------------------------------ */
+int srl_ppo_loss_from_beta(
+    const float* concentration1, const float* concentration0, /* [T,n,D] */
+    const float* action, int D,                                 /* [T,n,D] float32, in (0, 1) */
+    const float* v_pred,                                        /* [T,n]   */
+    const float* old_logp, const float* old_value, const float* ret, const float* adv,
+    const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper,
+    float* g_concentration1, float* g_concentration0, float* g_value, /* [T,n,D], [T,n,D], [T,n] */
+    float* logp_out, float* entropy_out,                                /* [T,n] or NULL          */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+/* The entry above with a bfloat16 policy side (a Beta policy under torch.autocast(dtype=torch.bfloat16)): same arguments
+ * in the same order; concentration1, concentration0, v_pred and their gradients are bfloat16 bit patterns (uint16_t).
+ * action, logp_out / entropy_out, the sample side and the ten outputs stay float32.  Each bfloat16 input is widened to
+ * float32 where it is read and all arithmetic is the entry above's, so logp and entropy are bit-identical to
+ * srl_ppo_loss_from_beta's on the widened values and each gradient is that entry's float32 result rounded to bfloat16
+ * once (round to nearest even); out and out_f32 are too whenever both entries launch the same grid (as for
+ * srl_ppo_loss_from_gaussian_bf16). */
+int srl_ppo_loss_from_beta_bf16(
+    const uint16_t* concentration1, const uint16_t* concentration0, /* [T,n,D] bfloat16 */
+    const float* action, int D,                                       /* [T,n,D] float32  */
+    const uint16_t* v_pred,                                           /* [T,n] bfloat16   */
+    const float* old_logp, const float* old_value, const float* ret, const float* adv,
+    const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper,
+    uint16_t* g_concentration1, uint16_t* g_concentration0, uint16_t* g_value, /* bfloat16 out */
+    float* logp_out, float* entropy_out,                                        /* [T,n] float32 or NULL */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+/* srl_ppo_loss_from_beta(_bf16) with the sample side read from K2's loss pack, as srl_ppo_loss_from_gaussian_pack reads
+ * it; elem_bytes = 4 or 2 selects the float32 or bfloat16 policy side.  Bit-identical to the leaf entry with the same
+ * lane_idx on the leaves the pack was written from; the same argument checks as srl_ppo_loss_from_gaussian_pack. */
+int srl_ppo_loss_from_beta_pack(
+    const void* concentration1, const void* concentration0, /* [T,n,D], float32 or bfloat16 */
+    const float* action, int D,                               /* [T,n,D] float32              */
+    int elem_bytes, const void* v_pred,                       /* [T,n], the concentrations' type */
+    const float* pack, int64_t pack_lanes, int pack_row_lo, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper,
+    void* g_concentration1, void* g_concentration0, void* g_value,
+    float* logp_out, float* entropy_out,                      /* [T,n] float32 or NULL        */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * K5a  Philox-keyed permutation of the environment axis (NEW capability: the reference has no
  * minibatching, SURVEY.md F2; nearest relative SimpleReplayBuffer.get, base/buffer.py:262-277).
  * out is [n_epochs][n_env * group]; row r holds epoch (epoch + r):

@@ -147,6 +147,22 @@ SIGNATURES = {
                                                 c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
                                                 c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                                 c_void_p, c_size_t, c_void_p]),
+    "srl_ppo_loss_from_beta": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                       c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                       c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                       c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                       c_void_p, c_size_t, c_void_p]),
+    # concentration1, concentration0, v_pred and their gradients: bfloat16 device pointers
+    "srl_ppo_loss_from_beta_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                            c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                            c_void_p, c_size_t, c_void_p]),
+    "srl_ppo_loss_from_beta_pack": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p,
+                                            c_void_p, c_int64, c_int, c_void_p,
+                                            c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                            c_void_p, c_size_t, c_void_p]),
     "srl_philox_perm": (c_int, [c_uint64, c_uint32, c_int, c_int, c_int, c_void_p, c_void_p]),
     "srl_philox4x32_10": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "srl_batch_gather": (c_int, [POINTER(LeafDesc), c_int, c_void_p, c_int, c_int, c_void_p]),

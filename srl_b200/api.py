@@ -54,7 +54,7 @@ class PPOHeadAnalyzedResult:
 
     A policy opts in by declaring the class attribute `ppo_head = True`; `MultiAgentPPOB200` then calls
     `policy.analyze(sample, target="ppo_head", burn_in_steps=...)` instead of `target="ppo"` and trains through the fused
-    head losses (K4b / K4c): the policy builds no torch.distributions object, and the trainer hands the gradients of the
+    head losses (K4b / K4c / K4d): the policy builds no torch.distributions object, and the trainer hands the gradients of the
     loss with respect to the fields below to autograd.  Return them as the network produced them (still attached to the
     graph).  Shapes lead with the analyzed rows and lanes `[T', B, (A,)]` of the sample, burn-in rows already dropped, as
     `target="ppo"` returns its tensors; float32 or bfloat16 (torch.autocast) on the policy's device.
@@ -68,6 +68,9 @@ class PPOHeadAnalyzedResult:
         to int32 once.
       diagonal Gaussian: `mean [T', B, (A,) D]`, `log_std` either one `[D]` parameter shared by every transition or the
         mean's shape, D <= 64; `action` the float32 actions the actors sampled, the mean's shape.
+      Beta (bounded actions): `concentration1` (alpha) and `concentration0` (beta), both `[T', B, (A,) D]`, positive, in
+        the dtype of `state_values`, D <= 64 -- torch.distributions.Beta(concentration1, concentration0); `action` the
+        float32 samples in (0, 1) the actors drew, the concentrations' shape (the policy maps them to its action bounds).
     `state_values [T', B, (A,) 1]` in the head's dtype (a scalar critic; with PopArt, the normalised value).
     """
     state_values: Any
@@ -77,6 +80,8 @@ class PPOHeadAnalyzedResult:
     available: Any = None
     mean: Any = None
     log_std: Any = None
+    concentration1: Any = None
+    concentration0: Any = None
 
 
 @dataclasses.dataclass

@@ -385,6 +385,16 @@ class HotPath:
             **self._head_common(e, j))
         return g_mean, g_log_std, g_value
 
+    def loss_from_beta(self, e: int, j: int, concentration1: torch.Tensor, concentration0: torch.Tensor,
+                       action: torch.Tensor, v_pred: torch.Tensor):
+        """K4d for minibatch (e, j) in deferred mode, the head twin of loss(): concentration1, concentration0 and float32
+        actions in (0, 1) `[T, n_mb, D]`, v_pred `[T, n_mb]`.  Gradients now, loss scalars + stats at finalize().
+        Returns (g_concentration1, g_concentration0, g_value) in the inputs' dtype."""
+        g_c1, g_c0, g_value, _, _, _, _ = ops.ppo_loss_from_beta(
+            concentration1, concentration0, action, v_pred, hyper=self.hyper, defer=True,
+            workspace=self.workspace[e * self.minibatches + j], **self._head_common(e, j))
+        return g_c1, g_c0, g_value
+
     def _head_common(self, e: int, j: int) -> dict:
         """Statistics rows and sample side of a head loss for minibatch (e, j): K2's pack where this step's scan wrote it
         and the minibatch is permuted, the leaves through lane_idx otherwise (one minibatch, cached advantages,

@@ -853,6 +853,120 @@ class PPOGaussianLossFunction(torch.autograd.Function):
         return (g_mean * grad_loss, g_ls * grad_loss, None, g_v * grad_loss) + (None,) * 10
 
 
+BETA_MAX_D = 64
+
+
+def ppo_loss_from_beta(concentration1, concentration0, action, v_pred, old_logp, old_value, ret, adv, on_reset_next,
+                       norm_stats, hyper: LossHyper, local_stats=None, popart_mean_std=None, lane_idx=None,
+                       want_logp_entropy: bool = False, workspace=None, defer: bool = False,
+                       pack: Optional[torch.Tensor] = None, pack_row_lo: int = 0):
+    """Loss starting from a Beta actor head (actions bounded to an interval): `concentration1` (alpha), `concentration0`
+    (beta) and float32 `action` `[T, n, D]`, D <= 64, with the action in the open interval (0, 1) -- a policy maps it to
+    its bounds itself -- and positive concentrations (neither is checked; a concentration that is not positive gives NaN
+    entropy and gradients for its transition).  The head's log-prob and entropy are
+    torch.distributions.Beta(concentration1, concentration0).log_prob(action).sum(-1) / .entropy().sum(-1); the loss is
+    ppo_loss_fwd_bwd's.  Returns (g_concentration1, g_concentration0, g_value, out, out_f32, logp, entropy): logp /
+    entropy `[T, n]` only with want_logp_entropy.  `defer` (needs an explicit `workspace`, a loss slot): out / out_f32
+    are None and loss_finalize folds the slot later; the gradients are complete either way.
+
+    The concentrations and `v_pred` are torch.float32 or torch.bfloat16, the same for all three (a Beta policy under
+    torch.autocast passes its bfloat16 outputs as they are); their gradients come back in that dtype, logp / entropy and
+    the statistics are float32.  bfloat16 inputs are widened exactly and the arithmetic is the float32 entry's; each
+    bfloat16 gradient is the float32 one rounded once (nearest even).  `action` is float32 always: the actions the actors
+    sampled, on which old_logp was computed.  `pack` / `pack_row_lo`: the sample side from K2's pack, as in
+    ppo_loss_from_logits (the five sample leaves may then be None)."""
+    dtype = concentration1.dtype if isinstance(concentration1, torch.Tensor) else torch.float32
+    if dtype not in (torch.float32, torch.bfloat16):
+        raise ValueError(f"concentration1: expected dtype torch.float32 or torch.bfloat16, got {dtype}")
+    if isinstance(v_pred, torch.Tensor) and v_pred.dtype != dtype:
+        raise ValueError(f"v_pred has dtype {v_pred.dtype} but concentration1 has {dtype}; both must have the same dtype, "
+                         f"cast one of them")
+    if isinstance(concentration0, torch.Tensor) and concentration0.dtype != dtype:
+        raise ValueError(f"concentration0 has dtype {concentration0.dtype} but concentration1 has {dtype}; both must have "
+                         f"the same dtype, cast one of them")
+    if isinstance(action, torch.Tensor) and action.dtype != torch.float32:
+        raise ValueError(f"action: expected dtype torch.float32, got {action.dtype}; pass the float32 actions the actors "
+                         f"sampled (old_logp was computed on them, and a rounded action would bias every ratio)")
+    _check(v_pred, dtype, "v_pred")
+    T, n = _rows_lanes(v_pred)
+    _check(concentration1, dtype, "concentration1")
+    _check(concentration0, dtype, "concentration0")
+    _check(action, torch.float32, "action")
+    c1, c0 = concentration1, concentration0
+    D = c1.shape[-1] if c1.dim() >= 2 else 0
+    if c1.dim() < 2 or c1.shape[0] != T or c1.numel() != T * n * D:
+        raise ValueError(f"concentration1: expected [T, n, D] with [T, n] = [{T}, {n}] (v_pred), got shape "
+                         f"{tuple(c1.shape)}")
+    if not 1 <= D <= BETA_MAX_D:
+        raise ValueError(f"concentration1: D = {D} action dimensions, supported are 1 .. {BETA_MAX_D}")
+    if tuple(c0.shape) != tuple(c1.shape):
+        raise ValueError(f"concentration0: shape {tuple(c0.shape)} does not match concentration1 {tuple(c1.shape)}")
+    if tuple(action.shape) != tuple(c1.shape):
+        raise ValueError(f"action: shape {tuple(action.shape)} does not match concentration1 {tuple(c1.shape)}")
+    ld_smp = _sample_side_or_pack(old_logp, old_value, ret, adv, on_reset_next, lane_idx, T, n, hyper.clip_value, pack,
+                                  pack_row_lo)
+    _check(norm_stats, torch.float64, "norm_stats")
+    local_stats = norm_stats if local_stats is None else _check(local_stats, torch.float64, "local_stats")
+    if popart_mean_std is not None:
+        _check(popart_mean_std, torch.float64, "popart_mean_std")
+    dev = c1.device
+    g_c1 = torch.empty_like(c1)
+    g_c0 = torch.empty_like(c0)
+    g_value = torch.empty_like(v_pred)
+    logp = torch.empty_like(v_pred, dtype=torch.float32) if want_logp_entropy else None
+    ent = torch.empty_like(v_pred, dtype=torch.float32) if want_logp_entropy else None
+    if defer:
+        if workspace is None:
+            raise ValueError("deferred finalisation needs an explicit workspace")
+        out = out_f32 = None
+    else:
+        out = torch.empty(SRL_LOSS_OUT_LEN, dtype=torch.float64, device=dev)
+        out_f32 = torch.empty(4, dtype=torch.float32, device=dev)
+    ws = loss_workspace(dev) if workspace is None else _check(workspace, torch.uint8, "workspace")
+    hc = hyper.to_c()
+    tail = (_ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
+            _ptr(g_c1), _ptr(g_c0), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws),
+            ws.numel(), _stream())
+    if pack is not None:
+        _lib.call("srl_ppo_loss_from_beta_pack", _ptr(c1), _ptr(c0), _ptr(action), D, c1.element_size(), _ptr(v_pred),
+                  _ptr(pack), ld_smp, int(pack_row_lo), *tail)
+    else:
+        suffix = "_bf16" if dtype == torch.bfloat16 else ""
+        _lib.call("srl_ppo_loss_from_beta" + suffix, _ptr(c1), _ptr(c0), _ptr(action), D, _ptr(v_pred), _ptr(old_logp),
+                  _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next), ld_smp, *tail)
+    return g_c1, g_c0, g_value, out, out_f32, logp, ent
+
+
+class PPOBetaLossFunction(torch.autograd.Function):
+    """Autograd node for a Beta policy (bounded actions): forward returns the scalar loss (float32) and the float64 stats
+    vector of ppo_loss_from_beta; backward hands the gradients the same launch produced to concentration1,
+    concentration0 and v_pred.  A policy under torch.autocast("cuda", dtype=torch.bfloat16) passes its bfloat16
+    concentrations and value as they are, with no casts, and gets bfloat16 gradients (the float32 ones rounded once); the
+    action stays float32.
+
+        loss, out = PPOBetaLossFunction.apply(concentration1, concentration0, action, v_pred, old_logp, old_value, ret,
+                                              adv, on_reset_next, norm_stats, local_stats, popart_mean_std, lane_idx,
+                                              hyper)
+        loss.backward()
+    """
+
+    @staticmethod
+    def forward(ctx, concentration1, concentration0, action, v_pred, old_logp, old_value, ret, adv, on_reset_next,
+                norm_stats, local_stats, popart_mean_std, lane_idx, hyper):
+        g_c1, g_c0, g_v, out, out_f32, _, _ = ppo_loss_from_beta(
+            concentration1.detach(), concentration0.detach(), action, v_pred.detach(), old_logp, old_value, ret, adv,
+            on_reset_next, norm_stats, hyper, local_stats=local_stats, popart_mean_std=popart_mean_std,
+            lane_idx=lane_idx)
+        ctx.save_for_backward(g_c1, g_c0, g_v.view(v_pred.shape))
+        ctx.mark_non_differentiable(out)
+        return out_f32[0], out
+
+    @staticmethod
+    def backward(ctx, grad_loss, _grad_out):
+        g_c1, g_c0, g_v = ctx.saved_tensors
+        return (g_c1 * grad_loss, g_c0 * grad_loss, None, g_v * grad_loss) + (None,) * 10
+
+
 class PPOCategoricalLossFunction(torch.autograd.Function):
     """Autograd node for a categorical policy (K4b): forward returns the scalar loss (float32) and the float64 stats
     vector of ppo_loss_from_logits; backward hands the gradients the same launch produced to the logits (exactly 0 where

@@ -147,7 +147,7 @@ class MultiAgentPPOB200(PytorchTrainer):
         if self.vtrace and (self.num_minibatches > 1 or self.recompute_adv_among_epochs):
             raise ValueError("vtrace supports num_minibatches == 1 without recompute_adv_among_epochs")
         # A policy that declares `ppo_head = True` hands over its actor head (api.PPOHeadAnalyzedResult) and trains through
-        # the fused head losses K4b / K4c; every other policy takes the `target="ppo"` path.
+        # the fused head losses K4b / K4c / K4d; every other policy takes the `target="ppo"` path.
         self.ppo_head = getattr(policy, "ppo_head", False) is True
         if self.ppo_head and self.vtrace:
             raise ValueError("vtrace=True needs the policy's new log-probabilities before the GAE scan, and a `ppo_head` "
@@ -376,7 +376,7 @@ class MultiAgentPPOB200(PytorchTrainer):
 
     # ----------------------------------------------------------------------------------------------------
     def _head_loss(self, hp: HotPath, e: int, j: int, res) -> List[Tuple[torch.Tensor, torch.Tensor]]:
-        """K4b / K4c for minibatch (e, j) on the head a `ppo_head` policy returned: [(output, d loss / d output)] for the
+        """K4b / K4c / K4d for minibatch (e, j) on the head a `ppo_head` policy returned: [(output, d loss / d output)] for the
         outputs that require grad (the loss scalars follow at hp.finalize())."""
         h = _head_fields(res, hp.T, hp.n_mb)
         T, n = hp.T, hp.n_mb
@@ -388,6 +388,12 @@ class MultiAgentPPOB200(PytorchTrainer):
             g_lg, g_v = hp.loss_from_logits(e, j, lg.detach().contiguous(), act, [int(k) for k in h.head_sizes],
                                             vp.detach().contiguous(), av)
             pairs = ((lg, g_lg), (vp, g_v))
+        elif h.concentration1 is not None:
+            c1, c0 = (c[:T].reshape(T, n, -1) for c in (h.concentration1, h.concentration0))
+            act = h.action[:T].reshape(T, n, -1).contiguous()
+            g_c1, g_c0, g_v = hp.loss_from_beta(e, j, c1.detach().contiguous(), c0.detach().contiguous(), act,
+                                                vp.detach().contiguous())
+            pairs = ((c1, g_c1), (c0, g_c0), (vp, g_v))
         else:
             mu = h.mean[:T].reshape(T, n, -1)
             ls = h.log_std if h.log_std.dim() == 1 else h.log_std[:T].reshape(T, n, -1)
@@ -466,8 +472,10 @@ def _head_fields(res, T: int, n: int) -> PPOHeadAnalyzedResult:
         raise ValueError(f"PPOHeadAnalyzedResult.state_values: expected [T', B, (A,) 1] with T' >= {T} rows of {n} lanes, "
                          f"got shape {tuple(sv.shape)}")
     lead = tuple(sv.shape[:-1])
-    if (res.logits is None) == (res.mean is None):
-        raise ValueError("PPOHeadAnalyzedResult: set exactly one of `logits` (categorical head) and `mean` (Gaussian head)")
+    beta = res.concentration1 is not None or res.concentration0 is not None
+    if (res.logits is not None) + (res.mean is not None) + beta != 1:
+        raise ValueError("PPOHeadAnalyzedResult: set exactly one of `logits` (categorical head), `mean` (Gaussian head) "
+                         "and `concentration1` / `concentration0` (Beta head)")
     if res.logits is not None:
         lg = tensor("logits")
         if lg.dtype != sv.dtype:
@@ -485,6 +493,22 @@ def _head_fields(res, T: int, n: int) -> PPOHeadAnalyzedResult:
         if av is not None and tuple(av.shape) != tuple(lg.shape):
             raise ValueError(f"PPOHeadAnalyzedResult.available: shape {tuple(av.shape)} differs from logits' "
                              f"{tuple(lg.shape)}")
+    elif beta:
+        c1, c0 = tensor("concentration1"), tensor("concentration0")
+        for name, c in (("concentration1", c1), ("concentration0", c0)):
+            if c.dtype != sv.dtype:
+                raise ValueError(f"PPOHeadAnalyzedResult.{name}: dtype {c.dtype} differs from state_values' {sv.dtype}")
+            if c.dim() != len(lead) + 1 or tuple(c.shape[:-1]) != lead:
+                raise ValueError(f"PPOHeadAnalyzedResult.{name}: expected {lead + ('D',)}, got {tuple(c.shape)}")
+        if tuple(c0.shape) != tuple(c1.shape):
+            raise ValueError(f"PPOHeadAnalyzedResult.concentration0: shape {tuple(c0.shape)} differs from "
+                             f"concentration1's {tuple(c1.shape)}")
+        if c1.shape[-1] > ops.BETA_MAX_D:
+            raise ValueError(f"PPOHeadAnalyzedResult.concentration1: D = {c1.shape[-1]} action dimensions, supported are "
+                             f"1 .. {ops.BETA_MAX_D}")
+        if act.dtype != torch.float32 or tuple(act.shape) != tuple(c1.shape):
+            raise ValueError(f"PPOHeadAnalyzedResult.action: expected float32 {tuple(c1.shape)}, got {act.dtype} "
+                             f"{tuple(act.shape)}")
     else:
         mu, ls = tensor("mean"), tensor("log_std")
         if mu.dtype != sv.dtype:
