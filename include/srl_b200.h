@@ -418,7 +418,52 @@ int srl_ppo_loss_from_logits_pack(
     double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
- * K4c  Same loss, but starting from a diagonal-Gaussian actor head (continuous actions, D = 1 .. 64 dimensions).
+ * K4b-wide  K4b for wide rows: 1 .. SRL_MAX_HEADS heads of sum K = 1 .. SRL_K4B_WIDE_MAX_SUM_K logits per transition
+ * (Go's 362 actions, chess's 4672 with a legal-move mask, a language model's vocabulary in bfloat16), where the entries
+ * above stage a [256, sum K] tile in shared memory and stop at SRL_K4B_MAX_SUM_K / SRL_K4B_MAX_SUM_K_MASKED.  A warp walks
+ * one transition's row instead.  Same contract as K4b: per head h with K_h logits z, lp = z - logsumexp(z),
+ * logp = sum_h lp[a_h], H = sum_h -sum_k softmax(z)_k lp_k; K4's loss, its ten outputs, masking and statistics; writes
+ * d loss / d logits (g_lp ([k == a] - p_k) - g_en p_k (lp_k + H_h)) and d loss / d v_pred.  Correct at every width from 1
+ * up, the narrow ones included, though ops.ppo_loss_from_logits only routes rows the entries above refuse here.
+ *  - elem_bytes = 4 (float32) or 2 (bfloat16) selects the policy side's element type (logits, v_pred, g_logits, g_value),
+ *    with the rules of the _bf16 entries: each input widened where it is read, float32 arithmetic, each gradient rounded
+ *    once.  Every logit goes to the same lane in the same order for both types, so the bfloat16 launch returns exactly the
+ *    float32 launch's logp and entropy on the widened values and its gradients rounded, and the same `out` / `out_f32`.
+ *  - available: NULL or the mask of srl_ppo_loss_from_logits_masked.  An unavailable logit is float32(-1e10) and gets
+ *    exactly 0 gradient, also where it is the chosen action.  A head with no available action adds exactly 0 to logp and
+ *    to the entropy, as in torch: its entropy is computed as (l - m) - w / s with l = fl(m + log s) already rounded (m the
+ *    head's max, s = sum e^{z-m}, w = sum e^{z-m} (z - m)), not as log s - w / s, which would give log K.
+ *  - -inf logits of an unmasked policy (dead agents) give finite entropies and gradients (lp is clamped at -FLT_MAX as
+ *    torch's Categorical.entropy clamps it); a chosen -inf action gives logp -inf and ratio 0.
+ *  - The grid has at most as many CTAs as one workspace slot has partial rows, so srl_ppo_loss_workspace_bytes and the
+ *    deferred mode (out == NULL, then srl_ppo_loss_finalize) work as for the entries above.
+ * srl_ppo_loss_from_logits_wide takes the leaves of srl_ppo_loss_from_logits; srl_ppo_loss_from_logits_wide_pack takes
+ * srl_ppo_loss_from_logits_pack's arguments in its order and makes its checks.  Argument checks and error texts are the K4b
+ * entries'; elem_bytes other than 2 or 4 is SRL_ERR_INVALID_ARG, sum K above SRL_K4B_WIDE_MAX_SUM_K SRL_ERR_UNSUPPORTED.
+ * ------------------------------------------------------------------------------------------ */
+#define SRL_K4B_WIDE_MAX_SUM_K 262144
+int srl_ppo_loss_from_logits_wide(
+    const void* logits, int elem_bytes, /* [T, n, sumK] dense, float32 or bfloat16 */
+    const uint8_t* available,           /* [T, n, sumK] dense or NULL               */
+    const int32_t* action,              /* [T, n, heads]                            */
+    const int32_t* head_sizes_host, int heads, const void* v_pred, /* [T, n] dense, the logits' type */
+    const float* old_logp, const float* old_value, const float* ret, const float* adv,
+    const uint8_t* on_reset_next, int64_t ld_smp, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper, void* g_logits, /* [T, n, sumK] out, the logits' type */
+    void* g_value,                               /* [T, n] out, the logits' type */
+    float* logp_out, float* entropy_out,         /* [T, n] float32 out or NULL */
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+int srl_ppo_loss_from_logits_wide_pack(
+    const void* logits, int elem_bytes, const uint8_t* available, const int32_t* action,
+    const int32_t* head_sizes_host, int heads, const void* v_pred,
+    const float* pack, int64_t pack_lanes, int pack_row_lo, const int32_t* lane_idx, int T, int n,
+    const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+    const srl_ppo_hyper* hyper, void* g_logits, void* g_value, float* logp_out, float* entropy_out,
+    double* out, float* out_f32, void* workspace, size_t workspace_bytes, srl_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
+ * K4c Same loss, but starting from a diagonal-Gaussian actor head (continuous actions, D = 1 .. 64 dimensions).
  * NEW capability: the reference's policies are categorical, so no reference line pins this head; the definition is
  * torch.distributions.Normal(mean, exp(log_std)), summed over the action dimensions, as any PyTorch Gaussian policy
  * computes it (sigma = exp(s)):

@@ -21,6 +21,7 @@ SRL_MAX_LEAVES = 32
 SRL_MAX_HEADS = 8
 SRL_K4B_MAX_SUM_K = 199
 SRL_K4B_MAX_SUM_K_MASKED = 159
+SRL_K4B_WIDE_MAX_SUM_K = 262144
 SRL_MAX_LOSS_BATCH = 32
 ABI_VERSION = 12
 
@@ -142,6 +143,17 @@ SIGNATURES = {
                                               c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
                                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                               c_size_t, c_void_p]),
+    # K4b-wide: srl_ppo_loss_from_logits's leaves with the _pack entry's (logits, elem_bytes, available) in front
+    "srl_ppo_loss_from_logits_wide": (c_int, [c_void_p, c_int, c_void_p, c_void_p, POINTER(c_int32), c_int, c_void_p,
+                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                              c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                              c_size_t, c_void_p]),
+    "srl_ppo_loss_from_logits_wide_pack": (c_int, [c_void_p, c_int, c_void_p, c_void_p, POINTER(c_int32), c_int, c_void_p,
+                                                   c_void_p, c_int64, c_int, c_void_p,
+                                                   c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),
+                                                   c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                   c_size_t, c_void_p]),
     "srl_ppo_loss_from_gaussian_pack": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p,
                                                 c_void_p, c_int64, c_int, c_void_p,
                                                 c_int, c_int, c_void_p, c_void_p, c_void_p, POINTER(PpoHyper),

@@ -61,8 +61,8 @@ class PPOHeadAnalyzedResult:
 
     Exactly one head kind:
       categorical (actor_critic_policy.py:303-324): `logits [T', B, (A,) sum K]` -- what the policy would hand to
-        `Categorical(logits=...)`, the heads side by side -- `head_sizes` (the K of each head, at most 8 heads, sum K <= 199,
-        <= 159 with a mask) and optionally `available` (SMAC's available_action, the logits' shape, non-zero = available;
+        `Categorical(logits=...)`, the heads side by side -- `head_sizes` (the K of each head, at most 8 heads, sum K <= 262144;
+        rows wider than 199, or 159 with a mask, run the wide kernel K4b-wide) and optionally `available` (SMAC's available_action, the logits' shape, non-zero = available;
         an unavailable logit is treated as masked_fill(-1e10), actor_critic_policy.py:135-136).  `action [T', B, (A,)
         heads]` of any integer dtype or integer-valued floats (SRL stores `action.x` as float32); the trainer converts it
         to int32 once.

@@ -52,20 +52,8 @@ __global__ void __launch_bounds__(256) loss_finalize_kernel(unsigned char* __res
 // A CTA takes 256 consecutive transitions; their [256, sumK] logits block is contiguous in memory, so
 // it is staged through shared memory with coalesced loads (row stride sumK+1 words: conflict-free
 // per-thread row walks), turned into d loss / d logits in place, and streamed back out coalesced.
-// The policy side (logits, v_pred, g_logits, g_value) is float or bfloat16, the kernel's element type T; pr.v_pred and
-// pr.g_value point at T as well (Problem is K4's struct, typed float).  Everything else, the arithmetic included, is float.
-struct LogitsParams {
-  LossShared s;
-  Problem pr;             // new_logp / entropy / g_logp / g_entropy are unused here
-  const void* logits;     // [T*n, SK] of T
-  const int32_t* action;  // [T*n, heads]
-  void* g_logits;         // [T*n, SK] of T
-  float* logp_out;        // [T*n] or null
-  float* entropy_out;     // [T*n] or null
-  int heads, SK;
-  int head_size[SRL_MAX_HEADS];
-  const uint8_t* available;  // [T*n, SK], 0 = unavailable (MASKED instantiations only)
-};
+// The policy side (logits, v_pred, g_logits, g_value) is float or bfloat16, the kernel's element type T (LogitsParams,
+// ppo_loss.cuh).  Everything else, the arithmetic included, is float.
 
 // How the kernel got here (ncu, T=128 N=4096 K=18: profiles/r2_notes.md).  First version: 2180 instructions per transition --
 // the staged [256, SK + 1] block was walked once per pass (max, exp / sum, entropy, gradient) with a run-time trip count,
@@ -81,15 +69,6 @@ struct LogitsParams {
 #define SRL_K4B_MIN_BLOCKS 2
 #endif
 constexpr int kStage = 9;  // manual staging batch per thread (last, partial tile only)
-
-// actor_critic_policy.py:135-136: logits.masked_fill(available_action == 0, -1e10) before the Categorical
-constexpr float kUnavailableLogit = -1e10f;
-
-// logit k of a row as the Categorical sees it
-template <bool MASKED, typename T>
-__device__ __forceinline__ float logit_at(const T* z, const uint8_t* m, int k) {
-  return (MASKED && m[k] == 0) ? kUnavailableLogit : to_float(z[k]);
-}
 
 // forward passes of one head held in registers: log-sum-exp, 1 / sum, entropy; e_k to `ez` when CACHE_E.  With MASKED,
 // `m` is the head's availability bytes and an unavailable logit reads as kUnavailableLogit (its e_k is 0 unless the whole
@@ -385,17 +364,44 @@ int launch_logits(const LogitsParams& q, bool cache_e, size_t smem, cudaStream_t
   return SRL_OK;
 }
 
+// the staged-tile kernel for the rows of q: caches e_k in shared memory when the [256, sum K] blocks fit
+int launch_logits_tile(const LogitsParams& q, size_t elem_bytes, bool masked, bool pack, cudaStream_t stream) {
+  const size_t sk = static_cast<size_t>(q.SK);
+  const size_t row_bytes = 256 * sk * elem_bytes;                            // dense [256, sum K] block of the element type
+  const size_t e_bytes = 256 * sk * sizeof(float);                           // the cached exponentials, float either way
+  const size_t mask_bytes = masked ? 256 * sk : 0;                           // + its [256, sum K] availability bytes
+  const bool cache_e = row_bytes + e_bytes + mask_bytes + 16 <= 200 * 1024;  // all fit: one exponential per logit
+  const size_t smem = row_bytes + (cache_e ? e_bytes : 0) + mask_bytes + 16;  // + the mbarrier of the bulk copies
+  const bool bf16 = elem_bytes == sizeof(__nv_bfloat16);
+  if (pack) {
+    if (bf16)
+      return masked ? launch_logits<true, __nv_bfloat16, true>(q, cache_e, smem, stream)
+                    : launch_logits<false, __nv_bfloat16, true>(q, cache_e, smem, stream);
+    return masked ? launch_logits<true, float, true>(q, cache_e, smem, stream)
+                  : launch_logits<false, float, true>(q, cache_e, smem, stream);
+  }
+  if (bf16)
+    return masked ? launch_logits<true, __nv_bfloat16, false>(q, cache_e, smem, stream)
+                  : launch_logits<false, __nv_bfloat16, false>(q, cache_e, smem, stream);
+  return masked ? launch_logits<true, float, false>(q, cache_e, smem, stream)
+                : launch_logits<false, float, false>(q, cache_e, smem, stream);
+}
+
+}  // namespace
+
 // srl_ppo_loss_from_logits (available == NULL) and srl_ppo_loss_from_logits_masked (elem_bytes = 4), their _bf16 twins
 // (elem_bytes = 2: logits, v_pred, g_logits and g_value are bfloat16) and srl_ppo_loss_from_logits_pack (pack != NULL: the
-// sample side is K2's pack, ld_smp its lanes, pack_row_lo the absolute row of loss row 0; the five leaves are not read)
-int ppo_loss_from_logits(const char* fn, size_t elem_bytes, const void* logits, const uint8_t* available,
-                         const int32_t* action, const int32_t* head_sizes_host, int heads, const void* v_pred,
-                         const float* old_logp, const float* old_value, const float* ret, const float* adv,
-                         const uint8_t* on_reset_next, int64_t ld_smp, const float* pack, int pack_row_lo,
-                         const int32_t* lane_idx, int T, int n, const double* norm_stats, const double* local_stats,
-                         const double* popart_mean_std, const srl_ppo_hyper* hyper, void* g_logits, void* g_value,
-                         float* logp_out, float* entropy_out, double* out, float* out_f32, void* workspace,
-                         size_t workspace_bytes, cudaStream_t stream) {
+// sample side is K2's pack, ld_smp its lanes, pack_row_lo the absolute row of loss row 0; the five leaves are not read),
+// with launch = launch_logits_tile and the limits SRL_K4B_MAX_SUM_K(_MASKED); the _wide entries (ppo_loss_wide.cu) pass
+// their own kernel and limit
+int ppo_loss_from_logits(const char* fn, int max_sum_k, int max_sum_k_masked, LogitsLauncher launch, size_t elem_bytes,
+                         const void* logits, const uint8_t* available, const int32_t* action,
+                         const int32_t* head_sizes_host, int heads, const void* v_pred, const float* old_logp,
+                         const float* old_value, const float* ret, const float* adv, const uint8_t* on_reset_next,
+                         int64_t ld_smp, const float* pack, int pack_row_lo, const int32_t* lane_idx, int T, int n,
+                         const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+                         const srl_ppo_hyper* hyper, void* g_logits, void* g_value, float* logp_out, float* entropy_out,
+                         double* out, float* out_f32, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   SRL_REQUIRE(T >= 1 && n >= 1, SRL_ERR_INVALID_ARG, "%s: need T >= 1 and n >= 1", fn);
   SRL_REQUIRE(heads >= 1 && heads <= SRL_MAX_HEADS && head_sizes_host, SRL_ERR_INVALID_ARG,
               "%s: heads=%d outside [1, %d]", fn, heads, SRL_MAX_HEADS);
@@ -418,13 +424,8 @@ int ppo_loss_from_logits(const char* fn, size_t elem_bytes, const void* logits, 
     sk += q.head_size[i];
   }
   const bool masked = available != nullptr;
-  const int max_sk = masked ? SRL_K4B_MAX_SUM_K_MASKED : SRL_K4B_MAX_SUM_K;
+  const int max_sk = masked ? max_sum_k_masked : max_sum_k;
   SRL_REQUIRE(sk <= max_sk, SRL_ERR_UNSUPPORTED, "%s: sum K = %lld too wide (max %d)", fn, sk, max_sk);
-  const size_t row_bytes = static_cast<size_t>(256) * sk * elem_bytes;     // dense [256, sum K] block of the element type
-  const size_t e_bytes = static_cast<size_t>(256) * sk * sizeof(float);    // the cached exponentials, float either way
-  const size_t mask_bytes = masked ? static_cast<size_t>(256) * sk : 0;    // + its [256, sum K] availability bytes
-  const bool cache_e = row_bytes + e_bytes + mask_bytes + 16 <= 200 * 1024;  // all fit: one exponential per logit
-  const size_t smem = row_bytes + (cache_e ? e_bytes : 0) + mask_bytes + 16;  // + the mbarrier of the bulk copies
   q.heads = heads;
   q.SK = static_cast<int>(sk);
   q.logits = logits;
@@ -463,22 +464,19 @@ int ppo_loss_from_logits(const char* fn, size_t elem_bytes, const void* logits, 
   pr.out = out;
   pr.out_f32 = out_f32;
   pr.slot = reinterpret_cast<SlotHeader*>(workspace);
-  const bool bf16 = elem_bytes == sizeof(__nv_bfloat16);
-  if (pack) {
-    if (bf16)
-      return masked ? launch_logits<true, __nv_bfloat16, true>(q, cache_e, smem, stream)
-                    : launch_logits<false, __nv_bfloat16, true>(q, cache_e, smem, stream);
-    return masked ? launch_logits<true, float, true>(q, cache_e, smem, stream)
-                  : launch_logits<false, float, true>(q, cache_e, smem, stream);
-  }
-  if (bf16)
-    return masked ? launch_logits<true, __nv_bfloat16, false>(q, cache_e, smem, stream)
-                  : launch_logits<false, __nv_bfloat16, false>(q, cache_e, smem, stream);
-  return masked ? launch_logits<true, float, false>(q, cache_e, smem, stream)
-                : launch_logits<false, float, false>(q, cache_e, smem, stream);
+  return launch(q, elem_bytes, masked, pack != nullptr, stream);
 }
 
-}  // namespace
+int check_logits_pack(const char* fn, int elem_bytes, const float* pack, int64_t pack_lanes, int pack_row_lo,
+                      const int32_t* lane_idx, int n) {
+  SRL_REQUIRE(elem_bytes == 4 || elem_bytes == 2, SRL_ERR_INVALID_ARG, "%s: elem_bytes=%d, need 4 (float32) or 2 (bfloat16)",
+              fn, elem_bytes);
+  SRL_REQUIRE(pack != nullptr && aligned(pack, 16), SRL_ERR_INVALID_ARG, "%s: pack is null or not 16-byte aligned", fn);
+  SRL_REQUIRE(pack_row_lo >= 0, SRL_ERR_INVALID_ARG, "%s: pack_row_lo=%d < 0", fn, pack_row_lo);
+  SRL_REQUIRE(lane_idx != nullptr || pack_lanes >= n, SRL_ERR_INVALID_ARG,
+              "%s: pack_lanes=%lld < n=%d without lane_idx", fn, static_cast<long long>(pack_lanes), n);
+  return SRL_OK;
+}
 
 int fill_loss_hyper(const srl_ppo_hyper* hyper, const double* popart_mean_std, LossHyperDev& h) {
   SRL_REQUIRE(hyper != nullptr, SRL_ERR_INVALID_ARG, "ppo loss: null hyper pointer");
@@ -689,7 +687,7 @@ extern "C" int srl_ppo_loss_from_logits(const float* logits, const int32_t* acti
                                         float* g_value, float* logp_out, float* entropy_out, double* out,
                                         float* out_f32, void* workspace, size_t workspace_bytes,
                                         srl_stream_t stream) {
-  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits", sizeof(float), logits, nullptr, action, head_sizes_host,
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits", SRL_K4B_MAX_SUM_K, SRL_K4B_MAX_SUM_K_MASKED, srl::loss::launch_logits_tile, sizeof(float), logits, nullptr, action, head_sizes_host,
                                          heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp, nullptr, 0, lane_idx, T, n,
                                          norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value, logp_out,
                                          entropy_out, out, out_f32, workspace, workspace_bytes,
@@ -707,7 +705,7 @@ extern "C" int srl_ppo_loss_from_logits_masked(const float* logits, const uint8_
                                                void* workspace, size_t workspace_bytes, srl_stream_t stream) {
   SRL_REQUIRE(available != nullptr, SRL_ERR_INVALID_ARG,
               "srl_ppo_loss_from_logits_masked: null pointer available (use srl_ppo_loss_from_logits without a mask)");
-  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked", sizeof(float), logits, available, action,
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked", SRL_K4B_MAX_SUM_K, SRL_K4B_MAX_SUM_K_MASKED, srl::loss::launch_logits_tile, sizeof(float), logits, available, action,
                                          head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp,
                                          nullptr, 0, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value,
                                          logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
@@ -723,7 +721,7 @@ extern "C" int srl_ppo_loss_from_logits_bf16(const uint16_t* logits, const int32
                                              uint16_t* g_value, float* logp_out, float* entropy_out, double* out,
                                              float* out_f32, void* workspace, size_t workspace_bytes,
                                              srl_stream_t stream) {
-  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_bf16", sizeof(__nv_bfloat16), logits, nullptr, action,
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_bf16", SRL_K4B_MAX_SUM_K, SRL_K4B_MAX_SUM_K_MASKED, srl::loss::launch_logits_tile, sizeof(__nv_bfloat16), logits, nullptr, action,
                                          head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next, ld_smp,
                                          nullptr, 0, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits, g_value,
                                          logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
@@ -742,7 +740,7 @@ extern "C" int srl_ppo_loss_from_logits_masked_bf16(const uint16_t* logits, cons
   SRL_REQUIRE(available != nullptr, SRL_ERR_INVALID_ARG,
               "srl_ppo_loss_from_logits_masked_bf16: null pointer available (use srl_ppo_loss_from_logits_bf16 without a "
               "mask)");
-  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked_bf16", sizeof(__nv_bfloat16), logits, available,
+  return srl::loss::ppo_loss_from_logits("srl_ppo_loss_from_logits_masked_bf16", SRL_K4B_MAX_SUM_K, SRL_K4B_MAX_SUM_K_MASKED, srl::loss::launch_logits_tile, sizeof(__nv_bfloat16), logits, available,
                                          action, head_sizes_host, heads, v_pred, old_logp, old_value, ret, adv, on_reset_next,
                                          ld_smp, nullptr, 0, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper, g_logits,
                                          g_value, logp_out, entropy_out, out, out_f32, workspace, workspace_bytes,
@@ -759,13 +757,9 @@ extern "C" int srl_ppo_loss_from_logits_pack(const void* logits, int elem_bytes,
                                              size_t workspace_bytes, srl_stream_t stream) {
   using namespace srl;
   constexpr const char* fn = "srl_ppo_loss_from_logits_pack";
-  SRL_REQUIRE(elem_bytes == 4 || elem_bytes == 2, SRL_ERR_INVALID_ARG, "%s: elem_bytes=%d, need 4 (float32) or 2 (bfloat16)",
-              fn, elem_bytes);
-  SRL_REQUIRE(pack != nullptr && aligned(pack, 16), SRL_ERR_INVALID_ARG, "%s: pack is null or not 16-byte aligned", fn);
-  SRL_REQUIRE(pack_row_lo >= 0, SRL_ERR_INVALID_ARG, "%s: pack_row_lo=%d < 0", fn, pack_row_lo);
-  SRL_REQUIRE(lane_idx != nullptr || pack_lanes >= n, SRL_ERR_INVALID_ARG,
-              "%s: pack_lanes=%lld < n=%d without lane_idx", fn, static_cast<long long>(pack_lanes), n);
-  return srl::loss::ppo_loss_from_logits(fn, static_cast<size_t>(elem_bytes), logits, available, action, head_sizes_host,
+  const int rc = srl::loss::check_logits_pack(fn, elem_bytes, pack, pack_lanes, pack_row_lo, lane_idx, n);
+  if (rc != SRL_OK) return rc;
+  return srl::loss::ppo_loss_from_logits(fn, SRL_K4B_MAX_SUM_K, SRL_K4B_MAX_SUM_K_MASKED, srl::loss::launch_logits_tile, static_cast<size_t>(elem_bytes), logits, available, action, head_sizes_host,
                                          heads, v_pred, nullptr, nullptr, nullptr, nullptr, nullptr, pack_lanes, pack,
                                          pack_row_lo, lane_idx, T, n, norm_stats, local_stats, popart_mean_std, hyper,
                                          g_logits, g_value, logp_out, entropy_out, out, out_f32, workspace,

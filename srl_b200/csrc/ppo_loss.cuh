@@ -403,6 +403,47 @@ __device__ __forceinline__ void load_pack_item(const LossShared& p, int t, int c
   ad = valid ? k.w : 0.f;
 }
 
+// ---- K4b (ppo_loss.cu: the staged-tile kernel; ppo_loss_wide.cu: a warp per row for wide rows) ------------------------
+// actor_critic_policy.py:135-136: logits.masked_fill(available_action == 0, -1e10) before the Categorical
+constexpr float kUnavailableLogit = -1e10f;
+
+// logit k of a row as the Categorical sees it
+template <bool MASKED, typename T>
+__device__ __forceinline__ float logit_at(const T* z, const uint8_t* m, int k) {
+  return (MASKED && m[k] == 0) ? kUnavailableLogit : to_float(z[k]);
+}
+
+// One K4b launch.  The policy side (logits, v_pred, g_logits, g_value) is float or bfloat16, the kernel's element type T;
+// pr.v_pred and pr.g_value point at T as well (Problem is K4's struct, typed float).
+struct LogitsParams {
+  LossShared s;
+  Problem pr;             // new_logp / entropy / g_logp / g_entropy are unused here
+  const void* logits;     // [T*n, SK] of T
+  const int32_t* action;  // [T*n, heads]
+  void* g_logits;         // [T*n, SK] of T
+  float* logp_out;        // [T*n] or null
+  float* entropy_out;     // [T*n] or null
+  int heads, SK;
+  int head_size[SRL_MAX_HEADS];
+  const uint8_t* available;  // [T*n, SK], 0 = unavailable (MASKED instantiations only)
+};
+
+// Launches one K4b kernel on the filled q (elem_bytes 4 or 2, masked: q.available is set, pack: q.s.pack is the sample side).
+using LogitsLauncher = int (*)(const LogitsParams& q, size_t elem_bytes, bool masked, bool pack, cudaStream_t stream);
+// ppo_loss.cu: the K4b entries' argument checks and LogitsParams filling, shared by the staged-tile entries and the _wide
+// ones; rows wider than max_sum_k (max_sum_k_masked with a mask) are SRL_ERR_UNSUPPORTED, the rest goes to `launch`
+int ppo_loss_from_logits(const char* fn, int max_sum_k, int max_sum_k_masked, LogitsLauncher launch, size_t elem_bytes,
+                         const void* logits, const uint8_t* available, const int32_t* action,
+                         const int32_t* head_sizes_host, int heads, const void* v_pred, const float* old_logp,
+                         const float* old_value, const float* ret, const float* adv, const uint8_t* on_reset_next,
+                         int64_t ld_smp, const float* pack, int pack_row_lo, const int32_t* lane_idx, int T, int n,
+                         const double* norm_stats, const double* local_stats, const double* popart_mean_std,
+                         const srl_ppo_hyper* hyper, void* g_logits, void* g_value, float* logp_out, float* entropy_out,
+                         double* out, float* out_f32, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+// ppo_loss.cu: the checks the _pack entries add (elem_bytes, the pack's pointer and alignment, pack_row_lo, pack_lanes)
+int check_logits_pack(const char* fn, int elem_bytes, const float* pack, int64_t pack_lanes, int pack_row_lo,
+                      const int32_t* lane_idx, int n);
+
 __device__ __forceinline__ void unpack4(const float4 v, float (&a)[4]) { a[0] = v.x, a[1] = v.y, a[2] = v.z, a[3] = v.w; }
 
 // Work decomposition of the row-tile kernel (dense leaves, leaves through lane_idx, odd shapes of the pack form): grid =

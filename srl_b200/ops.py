@@ -13,7 +13,8 @@ from typing import List, Optional, Sequence, Tuple
 import torch
 
 from srl_b200 import _lib
-from srl_b200._lib import (SRL_LANE_PART, SRL_LOSS_OUT_LEN, SRL_MAX_HEADS, SRL_MAX_LEAVES, SRL_MAX_LOSS_BATCH, LeafDesc, LossProblem,
+from srl_b200._lib import (SRL_K4B_MAX_SUM_K, SRL_K4B_MAX_SUM_K_MASKED, SRL_LANE_PART, SRL_LOSS_OUT_LEN, SRL_MAX_HEADS,
+                           SRL_MAX_LEAVES, SRL_MAX_LOSS_BATCH, LeafDesc, LossProblem,
                            PpoHyper, VALUE_LOSS_CODES)
 
 
@@ -637,7 +638,10 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     to bfloat16 once (nearest even).
     `available` (SMAC's available_action, the logits' shape): where it is 0 the logit is replaced by -1e10 before the
     Categorical (actor_critic_policy.py:135-136) and its gradient is 0.  torch.uint8 and torch.bool are read in place; a
-    floating mask costs one extra pass (`available != 0`).  At most 159 logits per transition with a mask, 199 without.
+    floating mask costs one extra pass (`available != 0`).
+    Up to 8 heads of up to 262144 logits per transition (SRL_K4B_WIDE_MAX_SUM_K) in all.  Rows of up to 199 logits (159 with
+    a mask) run K4b, which stages 256 rows at a time in shared memory; wider rows run K4b-wide
+    (srl_ppo_loss_from_logits_wide / _wide_pack), where a warp walks each row -- the same results to float32 rounding.
     `defer` (needs an explicit `workspace` slot): out / out_f32 are None and loss_finalize folds the slot later.
     `pack` (K2's whole `[ceil(L/2), N, 2, 4]` pack, `new_pack`) with `pack_row_lo` = the sample row of loss row 0: the
     sample side is read from it, one 16-byte item per transition (srl_ppo_loss_from_logits_pack), and the five sample leaves
@@ -685,12 +689,17 @@ def ppo_loss_from_logits(logits, action, head_sizes: Sequence[int], v_pred, old_
     hs = (ctypes.c_int32 * heads)(*[int(k) for k in head_sizes])
     rest = (_ptr(lane_idx), T, n, _ptr(norm_stats), _ptr(local_stats), _ptr(popart_mean_std), ctypes.byref(hc),
             _ptr(g_logits), _ptr(g_value), _ptr(logp), _ptr(ent), _ptr(out), _ptr(out_f32), _ptr(ws), ws.numel(), _stream())
+    wide = SK > (SRL_K4B_MAX_SUM_K if available is None else SRL_K4B_MAX_SUM_K_MASKED)
     if pack is not None:
-        _lib.call("srl_ppo_loss_from_logits_pack", _ptr(logits), logits.element_size(), _ptr(available), _ptr(action), hs,
-                  heads, _ptr(v_pred), _ptr(pack), ld_smp, int(pack_row_lo), *rest)
+        _lib.call("srl_ppo_loss_from_logits_wide_pack" if wide else "srl_ppo_loss_from_logits_pack", _ptr(logits),
+                  logits.element_size(), _ptr(available), _ptr(action), hs, heads, _ptr(v_pred), _ptr(pack), ld_smp,
+                  int(pack_row_lo), *rest)
         return g_logits, g_value, out, out_f32, logp, ent
     tail = (hs, heads, _ptr(v_pred), _ptr(old_logp), _ptr(old_value), _ptr(ret), _ptr(adv), _ptr(on_reset_next),
             ld_smp) + rest
+    if wide:
+        _lib.call("srl_ppo_loss_from_logits_wide", _ptr(logits), logits.element_size(), _ptr(available), _ptr(action), *tail)
+        return g_logits, g_value, out, out_f32, logp, ent
     suffix = "_bf16" if dtype == torch.bfloat16 else ""
     if available is None:
         _lib.call("srl_ppo_loss_from_logits" + suffix, _ptr(logits), _ptr(action), *tail)
